@@ -29,6 +29,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 import numpy as np
 
@@ -326,6 +327,29 @@ class DevBatch:
                 f"c+{accel}+{block}": one(cms, "compress_kernel*"), f"d+{block}": one(dms, "decompress_kernel*")}
 
 
+DUMP_SAMPLE_BLOCKS = 8
+
+
+def dump_outputs(out_dir, d_out, d_ooff, d_olen):
+    """Write what the last timed step hands its caller, so that two builds can be compared output for output: every
+    block's offset in the compacted stream, its compressed length and the CRC-32 of its framed bytes (float64), and the
+    framed bytes (header included) of a fixed, seeded sample of blocks, one byte per float32 element.  The whole stream
+    (~0.6 GB at the default size) is not written; the sample stays under 21 MB at any size, as the blocks are 640000
+    bytes."""
+    os.makedirs(out_dir, exist_ok=True)
+    ooff = d_ooff.cpu().numpy()
+    n = ooff.size - 1
+    out = d_out[:int(ooff[-1])].cpu().numpy()
+    blocks = [out[int(ooff[i]):int(ooff[i + 1])] for i in range(n)]
+    pick = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_SAMPLE_BLOCKS), replace=False))
+    np.save(os.path.join(out_dir, "block_offsets.npy"), ooff.astype(np.float64))
+    np.save(os.path.join(out_dir, "block_lengths.npy"), d_olen.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "block_crc32.npy"), np.array([zlib.crc32(b) for b in blocks], dtype=np.float64))
+    np.save(os.path.join(out_dir, "sample_block_index.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "sample_block_bytes.npy"), np.concatenate([blocks[i] for i in pick]).astype(np.float32))
+    log(f"outputs of the last timed step written to {out_dir}")
+
+
 def copy_ceiling(ctx, pin_src, total, pin_dst, comp_total, reps, barrier):
     """Plain cudaMemcpyAsync of one step's H2D and D2H bytes on two streams at once (b200lz4_copy_probe: no kernels),
     all ranks together; wall-clock per repetition."""
@@ -415,6 +439,8 @@ def run_gpu(args):
     kern_ms = [ev[2 * k].elapsed_time(ev[2 * k + 1]) for k in range(args.steps)]
     compact_ms = [ev[2 * k + 1].elapsed_time(ev[2 * k + 2]) for k in range(args.steps)]
     gpu_launches = args.steps * 3
+    if args.dump_outputs and rank == 0:                    # before the probes below reuse B's buffers
+        dump_outputs(args.dump_outputs, B.d_out, L["d_ooff"], L["d_olen"])
 
     # ---- e2e: the C-ABI host call with pinned host buffers (H2D + kernels + D2H + sync inside)
     ctx = lz.Context(local)
@@ -750,7 +776,11 @@ def main():
     ap.add_argument("--no-check", action="store_true", help="skip the in-bench parity spot check")
     ap.add_argument("--config3", action="store_true", help="run config 3 (8 GiB pre-compressed stream) at N = 1 as well")
     ap.add_argument("--config3-gib", type=int, default=8)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's stripe) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     import __graft_entry__ as ge
     if int(os.environ.get("LOCAL_RANK", "0")) == 0:
         ge.build_cpu_side()

@@ -29,20 +29,40 @@ def port(built):
     return Oracle("port")
 
 
+def _golden():
+    """tests/golden/make_golden.py: the stored outputs of the reference's codec and the inputs they belong to."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(ROOT, "tests", "golden", "make_golden.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def pytest_report_header(config):
+    from oracle.oracle import available
+    if available("reference"):
+        return "parity oracle: reference build (oracle/_ref/libreflz4.so)"
+    return "parity oracle: restatement (oracle/lz4_oracle.c), checked first against the stored reference outputs in tests/golden"
+
+
 @pytest.fixture(scope="session")
 def ref(built):
-    """The reference's own lz4.c, compiled by oracle/Makefile into oracle/_ref (prebuilt here, it travels to the GPU
-    box).  There is NO silent downgrade: without it the parity tests fail, unless B200LZ4_ALLOW_PORT_ORACLE=1
-    explicitly selects the restatement (which test_oracle.py pins against the reference wherever both exist)."""
+    """The reference's codec where oracle/Makefile could build it into oracle/_ref (it needs the reference's source tree,
+    which the repository does not contain).  Otherwise the restatement (oracle/lz4_oracle.c), and only after it has
+    reproduced, byte for byte, every stored output of the reference's codec in tests/golden/golden.json and decoded it
+    back (the report header says which one a run uses)."""
     from oracle.oracle import Oracle, available
     if available("reference"):
         return Oracle("reference")
-    if os.environ.get("B200LZ4_ALLOW_PORT_ORACLE") == "1":
-        import warnings
-        warnings.warn("oracle/_ref is missing: parity is checked against the RESTATEMENT (oracle/lz4_oracle.c), not the reference")
-        return Oracle("port")
-    pytest.fail("oracle/_ref/libreflz4.so is missing (build it here with `make -C oracle`; it is git-ignored but travels "
-                "with the snapshot).  Set B200LZ4_ALLOW_PORT_ORACLE=1 to run against the restatement instead.")
+    golden = _golden()
+    port = Oracle("port")
+    for case in golden.load("golden.json")["cases"]:
+        try:
+            golden.check_golden_case(port, case)
+        except AssertionError as e:
+            pytest.fail(f"the restatement no longer reproduces the reference's stored output ({e}): it cannot stand in "
+                        "for the reference")
+    return port
 
 
 @pytest.fixture(scope="session")

@@ -1,21 +1,30 @@
 #!/usr/bin/env python
-"""Generate tests/golden/golden.json from the REFERENCE's own codec.
+"""Stored outputs of the reference's codec, and the one definition of the inputs they were computed on.
 
-Run in the build container only (needs /root/reference):  python tests/golden/make_golden.py
-It compiles /root/reference/cbits/lz4.c unmodified (oracle/Makefile -> oracle/_ref/libreflz4.so),
-drives it with the Haskell shim's call sequence (oracle/ref_driver.c) on seeded inputs
-(streamly_lz4_b200/datagen, deterministic) and records, per case, the generator parameters,
-every block's compressed length, the SHA-256 of the framed stream and -- for the small cases --
-the framed bytes themselves (hex).  The reference ships no golden vectors of its own
-(SURVEY.md section 8c), so these outputs of the reference run here are the pin.
+  python tests/golden/make_golden.py           -> golden.json: per case the generator parameters, every block's
+                                                  compressed length, the SHA-256 of the framed stream and, for the small
+                                                  cases, the framed bytes themselves (hex)
+  python tests/golden/make_golden.py checks    -> reference_checks.json: what tests/test_oracle.py compares the
+                                                  restatement with (compress digests on every generator and
+                                                  configuration, random edge sizes, the decoder's accept/reject verdict
+                                                  and output digest on truncated and bit-flipped blocks)
+
+Both need the reference build, oracle/_ref/libreflz4.so: oracle/ref_driver.c compiled with -DDRV_USE_REFERENCE against
+an LZ4 (oracle/Makefile builds it from the reference's own cbits/lz4.c when REF points at its tree).  The reference
+ships no golden vectors of its own (SURVEY.md section 8c), so these outputs are the pin; each file records the LZ4
+version that made it.  The tests import this module for the inputs, so generator and tests cannot drift apart.
 """
 import hashlib
 import json
 import os
 import sys
 
-ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-sys.path.insert(0, ROOT)
+import numpy as np
+
+HERE = os.path.dirname(os.path.abspath(__file__))
+ROOT = os.path.dirname(os.path.dirname(HERE))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
 
 from oracle.oracle import Oracle, available  # noqa: E402
 from streamly_lz4_b200 import datagen  # noqa: E402
@@ -41,38 +50,140 @@ CASES = [
 ]
 TINY_SIZES = [0, 1, 4, 12, 13, 14, 0, 3, 64, 2, 500, 0, 15, 31]
 
+# inputs of the restatement-vs-reference checks (tests/test_oracle.py)
+KINDS = ["text", "random", "sparse01", "records", "mixed", "bits01", "biased01", "zero"]
+CONFIGS = [(65536, 1, True), (65536, 1, False), (640000, 400, False), (100000, 5, True), (4096, 1, True),
+           (1000, 12, True), (333, 0, True), (3 << 20, 1, False), (50000, 65537, True)]     # block, accel, linked
 
-def arrays_of(case):
-    name, kind, seed, total, bs, accel, linked, cfg = case
-    if name == "tiny_sizes":
-        d = datagen.make(kind, seed, 4096)
+
+def sha(chunks) -> str:
+    return hashlib.sha256(b"".join(chunks)).hexdigest()
+
+
+def load(name: str) -> dict:
+    with open(os.path.join(HERE, name)) as f:
+        return json.load(f)
+
+
+def arrays_of(case: dict):
+    if case["name"] == "tiny_sizes":
+        d = datagen.make(case["kind"], case["seed"], 4096)
         out, at = [], 0
         for n in TINY_SIZES:
             out.append(d[at:at + n].tobytes()); at += n
         return out
-    d = datagen.make(kind, seed, total)
-    return [d[i:i + bs].tobytes() for i in range(0, total, bs)]
+    d = datagen.make(case["kind"], case["seed"], case["total"])
+    return [d[i:i + case["block"]].tobytes() for i in range(0, case["total"], case["block"])]
 
 
-def main():
-    assert available("reference") or os.path.exists("/root/reference/cbits/lz4.c"), "needs the reference tree"
-    ref = Oracle("reference")
-    out = {"generator": "tests/golden/make_golden.py", "codec": "reference cbits/lz4.c (LZ4 1.9.3), oracle/ref_driver.c call sequence",
-           "cases": []}
-    for case in CASES:
-        name, kind, seed, total, bs, accel, linked, cfg = case
+def check_golden_case(ora, case: dict) -> None:
+    """`ora` reproduces the stored framed stream of `case` and decodes it back to the input."""
+    arrays = arrays_of(case)
+    assert sha(arrays) == case["input_sha256"], "data generator drifted"
+    framed = ora.compress_chunks(arrays, case["accel"], block_size=case["block_size"], linked=case["linked"])
+    assert [len(f) for f in framed] == case["framed_lens"], case["name"]
+    assert sha(framed) == case["framed_sha256"], case["name"]
+    if "framed_hex" in case:
+        assert b"".join(framed).hex() == case["framed_hex"], case["name"]
+    assert ora.decompress_chunks_raw(framed, block_size=case["block_size"], linked=case["linked"]) == arrays, case["name"]
+
+
+def config_arrays(kind: str, block: int):
+    d = datagen.make(kind, 4242, 3 << 20)
+    return [d[i:i + block].tobytes() for i in range(0, min(d.size, 200 * block), block)]
+
+
+def edge_size_trials():
+    """30 linked streams of 12 arrays with sizes around the format's thresholds, each with its acceleration."""
+    rng = np.random.default_rng(1)
+    d = datagen.make("text", 1, 400000)
+    trials = []
+    for _ in range(30):
+        sizes = [int(x) for x in rng.choice([0, 1, 2, 3, 4, 5, 11, 12, 13, 14, 15, 16, 17, 100, 255, 270, 4096, 65535, 65536, 65547],
+                                            size=12)]
+        arrays, at = [], 0
+        for n in sizes:
+            at = (at + 997) % (d.size - n - 1)
+            arrays.append(d[at:at + n].tobytes())
+        trials.append((arrays, int(rng.integers(-1, 13))))
+    return trials
+
+
+def decoder_input():
+    return datagen.make("text", 13, 100000).tobytes()
+
+
+def corrupted_blocks(payload: bytes, n_plain: int):
+    """Framed single blocks (8-byte header) whose payload is truncated or has one bit flipped."""
+    rng = np.random.default_rng(7)
+    cases = [payload[:k] for k in (1, 2, 10, len(payload) // 2, len(payload) - 1)]
+    for _ in range(300):
+        b = bytearray(payload)
+        at = int(rng.integers(0, len(b)))
+        b[at] ^= 1 << int(rng.integers(0, 8))
+        cases.append(bytes(b))
+    return [len(c).to_bytes(4, "little") + n_plain.to_bytes(4, "little") + c for c in cases]
+
+
+def decode_verdict(ora, framed: bytes):
+    """The decoder's decision on one independent framed block: None when rejected, else the output's SHA-256."""
+    try:
+        return sha(ora.decompress_chunks_raw([framed], linked=False))
+    except RuntimeError:
+        return None
+
+
+def codec_name(ora) -> str:
+    v = ora.lib.LZ4_versionNumber()
+    return f"LZ4 {v // 10000}.{v // 100 % 100}.{v % 100} through oracle/ref_driver.c"
+
+
+def make_golden(ref):
+    out = {"generator": "tests/golden/make_golden.py", "codec": codec_name(ref), "cases": []}
+    for name, kind, seed, total, bs, accel, linked, cfg in CASES:
+        case = {"name": name, "kind": kind, "seed": seed, "total": total, "block": bs}
         arrays = arrays_of(case)
         framed = ref.compress_chunks(arrays, accel, block_size=cfg, linked=linked)
         blob = b"".join(framed)
-        entry = {"name": name, "kind": kind, "seed": seed, "total": total, "block": bs, "accel": accel,
-                 "linked": linked, "block_size": cfg, "input_sha256": hashlib.sha256(b"".join(arrays)).hexdigest(),
-                 "framed_lens": [len(f) for f in framed], "framed_sha256": hashlib.sha256(blob).hexdigest()}
+        entry = dict(case, accel=accel, linked=linked, block_size=cfg, input_sha256=sha(arrays),
+                     framed_lens=[len(f) for f in framed], framed_sha256=sha(framed))
         if len(blob) <= 4096:
             entry["framed_hex"] = blob.hex()
             entry["input_hex"] = b"".join(arrays).hex()
         out["cases"].append(entry)
         print(name, len(arrays), "blocks", len(blob), "bytes")
-    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden.json"), "w") as f:
+    return out
+
+
+def make_checks(ref):
+    configs = {}
+    for kind in KINDS:
+        configs[kind] = []
+        for block, accel, linked in CONFIGS:
+            arrays = config_arrays(kind, block)
+            framed = ref.compress_chunks(arrays, accel, linked=linked)
+            assert ref.decompress_chunks_raw(framed, linked=linked) == arrays
+            configs[kind].append({"block": block, "accel": accel, "linked": linked, "input_sha256": sha(arrays),
+                                  "framed_sha256": sha(framed)})
+    edges = [sha(ref.compress_chunks(arrays, accel, linked=True)) for arrays, accel in edge_size_trials()]
+    d = decoder_input()
+    payload = ref.compress_chunks([d], 1, linked=False)[0][8:]
+    verdicts = [decode_verdict(ref, c) for c in corrupted_blocks(payload, len(d))]
+    print("configs", sum(map(len, configs.values())), "edge trials", len(edges), "corrupted blocks", len(verdicts),
+          "rejected", verdicts.count(None))
+    return {"generator": "tests/golden/make_golden.py checks", "codec": codec_name(ref),
+            "configs": configs, "edge_size_trials": edges,
+            "decoder": {"payload_sha256": hashlib.sha256(payload).hexdigest(), "verdicts": verdicts}}
+
+
+def main():
+    assert available("reference"), "needs the reference build oracle/_ref/libreflz4.so"
+    ref = Oracle("reference")
+    if sys.argv[1:] == ["checks"]:
+        name, out = "reference_checks.json", make_checks(ref)
+    else:
+        name, out = "golden.json", make_golden(ref)
+    with open(os.path.join(HERE, name), "w") as f:
         json.dump(out, f, indent=1)
 
 

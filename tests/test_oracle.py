@@ -1,101 +1,76 @@
 """CPU tests: pin the oracle.
 
 1. The restatement (oracle/lz4_oracle.c) must reproduce the committed golden vectors, which
-   are outputs of the reference's own cbits/lz4.c (tests/golden/make_golden.py).
-2. Where the reference build is present (oracle/_ref/libreflz4.so), the restatement must equal
-   it byte for byte on fresh seeded inputs, including the hash-table-dependent linked mode.
+   are outputs of the reference's codec (tests/golden/make_golden.py).
+2. On fresh seeded inputs, including the hash-table-dependent linked mode and the decoder's
+   accept/reject decisions on corrupted blocks, the restatement must equal the reference's codec:
+   its stored digests (tests/golden/reference_checks.json), and byte for byte a live reference
+   build wherever one is present (oracle/_ref/libreflz4.so).
 3. The Haskell-level logic restated in Python (resize, headers) must satisfy the properties
    of test/Main.hs:189-245.
 """
 import hashlib
-import json
+import importlib.util
 import os
 
 import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-GOLDEN = json.load(open(os.path.join(HERE, "golden", "golden.json")))
+_spec = importlib.util.spec_from_file_location("make_golden", os.path.join(HERE, "golden", "make_golden.py"))
+golden = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(golden)
+GOLDEN = golden.load("golden.json")
+CHECKS = golden.load("reference_checks.json")
 
 
-def arrays_of(case):
-    from streamly_lz4_b200 import datagen
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(HERE, "golden", "make_golden.py"))
-    if case["name"] == "tiny_sizes":
-        mg = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mg)
-        d = datagen.make(case["kind"], case["seed"], 4096)
-        out, at = [], 0
-        for n in mg.TINY_SIZES:
-            out.append(d[at:at + n].tobytes()); at += n
-        return out
-    d = datagen.make(case["kind"], case["seed"], case["total"])
-    return [d[i:i + case["block"]].tobytes() for i in range(0, case["total"], case["block"])]
+def live_reference():
+    from oracle.oracle import Oracle, available
+    return Oracle("reference") if available("reference") else None
 
 
 @pytest.mark.parametrize("case", GOLDEN["cases"], ids=[c["name"] for c in GOLDEN["cases"]])
 def test_port_matches_golden(port, case):
-    arrays = arrays_of(case)
-    assert hashlib.sha256(b"".join(arrays)).hexdigest() == case["input_sha256"], "data generator drifted"
-    framed = port.compress_chunks(arrays, case["accel"], block_size=case["block_size"], linked=case["linked"])
-    assert [len(f) for f in framed] == case["framed_lens"]
-    blob = b"".join(framed)
-    assert hashlib.sha256(blob).hexdigest() == case["framed_sha256"]
-    if "framed_hex" in case:
-        assert blob.hex() == case["framed_hex"]
-    back = port.decompress_chunks_raw(framed, block_size=case["block_size"], linked=case["linked"])
-    assert back == arrays
+    golden.check_golden_case(port, case)
 
 
 def test_reference_matches_golden_when_present(built):
-    from oracle.oracle import Oracle, available
-    if not available("reference"):
+    ref = live_reference()
+    if ref is None:
         pytest.skip("reference build not present on this box")
-    ref = Oracle("reference")
     for case in GOLDEN["cases"]:
-        arrays = arrays_of(case)
-        framed = ref.compress_chunks(arrays, case["accel"], block_size=case["block_size"], linked=case["linked"])
-        assert hashlib.sha256(b"".join(framed)).hexdigest() == case["framed_sha256"], case["name"]
+        framed = ref.compress_chunks(golden.arrays_of(case), case["accel"], block_size=case["block_size"], linked=case["linked"])
+        assert golden.sha(framed) == case["framed_sha256"], case["name"]
 
 
-@pytest.mark.parametrize("kind", ["text", "random", "sparse01", "records", "mixed", "bits01", "biased01", "zero"])
+@pytest.mark.parametrize("kind", golden.KINDS)
 def test_port_equals_reference(built, port, kind):
-    from oracle.oracle import Oracle, available
-    from streamly_lz4_b200 import datagen
-    if not available("reference"):
-        pytest.skip("reference build not present on this box")
-    ref = Oracle("reference")
-    d = datagen.make(kind, 4242, 3 << 20)
-    for bs, accel, linked in [(65536, 1, True), (65536, 1, False), (640000, 400, False), (100000, 5, True),
-                              (4096, 1, True), (1000, 12, True), (333, 0, True), (3 << 20, 1, False), (50000, 65537, True)]:
-        arrays = [d[i:i + bs].tobytes() for i in range(0, min(d.size, 200 * bs), bs)]
-        a = ref.compress_chunks(arrays, accel, linked=linked)
+    ref = live_reference()
+    stored = CHECKS["configs"][kind]
+    assert [(c["block"], c["accel"], c["linked"]) for c in stored] == golden.CONFIGS
+    for want in stored:
+        bs, accel, linked = want["block"], want["accel"], want["linked"]
+        arrays = golden.config_arrays(kind, bs)
+        assert golden.sha(arrays) == want["input_sha256"], "data generator drifted"
         b = port.compress_chunks(arrays, accel, linked=linked)
-        assert a == b, (kind, bs, accel, linked)
-        assert port.decompress_chunks_raw(a, linked=linked) == arrays
-        assert ref.decompress_chunks_raw(b, linked=linked) == arrays
+        assert golden.sha(b) == want["framed_sha256"], (kind, bs, accel, linked)
+        assert port.decompress_chunks_raw(b, linked=linked) == arrays
+        if ref is not None:
+            a = ref.compress_chunks(arrays, accel, linked=linked)
+            assert a == b, (kind, bs, accel, linked)
+            assert ref.decompress_chunks_raw(b, linked=linked) == arrays
 
 
 def test_port_equals_reference_edge_sizes(built, port):
-    from oracle.oracle import Oracle, available
-    from streamly_lz4_b200 import datagen
-    if not available("reference"):
-        pytest.skip("reference build not present on this box")
-    ref = Oracle("reference")
-    rng = np.random.default_rng(1)
-    d = datagen.make("text", 1, 400000)
-    for trial in range(30):
-        sizes = [int(x) for x in rng.choice([0, 1, 2, 3, 4, 5, 11, 12, 13, 14, 15, 16, 17, 100, 255, 270, 4096, 65535, 65536, 65547],
-                                            size=12)]
-        arrays, at = [], 0
-        for n in sizes:
-            at = (at + 997) % (d.size - n - 1)
-            arrays.append(d[at:at + n].tobytes())
-        accel = int(rng.integers(-1, 13))
-        a = ref.compress_chunks(arrays, accel, linked=True)
-        assert a == port.compress_chunks(arrays, accel, linked=True), (sizes, accel)
-        assert port.decompress_chunks_raw(a, linked=True) == arrays
+    ref = live_reference()
+    trials = golden.edge_size_trials()
+    assert len(trials) == len(CHECKS["edge_size_trials"])
+    for (arrays, accel), want in zip(trials, CHECKS["edge_size_trials"]):
+        b = port.compress_chunks(arrays, accel, linked=True)
+        assert golden.sha(b) == want, ([len(a) for a in arrays], accel)
+        if ref is not None:
+            assert ref.compress_chunks(arrays, accel, linked=True) == b, ([len(a) for a in arrays], accel)
+        assert port.decompress_chunks_raw(b, linked=True) == arrays
 
 
 def test_acceleration_clamp(port):
@@ -111,32 +86,18 @@ def test_acceleration_clamp(port):
 
 
 def test_decoder_accept_reject_agrees_with_reference(built, port):
-    from oracle.oracle import Oracle, available
-    from streamly_lz4_b200 import datagen
-    if not available("reference"):
-        pytest.skip("reference build not present on this box")
-    ref = Oracle("reference")
-    d = datagen.make("text", 13, 100000).tobytes()
-    payload = ref.compress_chunks([d], 1, linked=False)[0][8:]
-    rng = np.random.default_rng(7)
-    cases = [payload[:k] for k in (1, 2, 10, len(payload) // 2, len(payload) - 1)]
-    for _ in range(300):
-        b = bytearray(payload)
-        at = int(rng.integers(0, len(b)))
-        b[at] ^= 1 << int(rng.integers(0, 8))
-        cases.append(bytes(b))
-    agree = 0
-    for c in cases:
-        arr = len(c).to_bytes(4, "little") + len(d).to_bytes(4, "little") + c
-        res = []
-        for o in (ref, port):
-            try:
-                res.append(o.decompress_chunks_raw([arr], linked=False))
-            except RuntimeError:
-                res.append(None)
-        assert res[0] == res[1]
-        agree += 1
-    assert agree == len(cases)
+    ref = live_reference()
+    d = golden.decoder_input()
+    payload = port.compress_chunks([d], 1, linked=False)[0][8:]
+    assert hashlib.sha256(payload).hexdigest() == CHECKS["decoder"]["payload_sha256"]
+    blocks = golden.corrupted_blocks(payload, len(d))
+    want = CHECKS["decoder"]["verdicts"]
+    assert len(blocks) == len(want) and want.count(None) > 0
+    for i, (arr, w) in enumerate(zip(blocks, want)):
+        got = golden.decode_verdict(port, arr)
+        assert got == w, f"corrupted block {i}: restatement {'rejects' if got is None else 'accepts'} it, the reference did not"
+        if ref is not None:
+            assert golden.decode_verdict(ref, arr) == got, f"corrupted block {i}"
 
 
 # ---- resizeChunksD restatement (pure Python) --------------------------------------------------
