@@ -11,7 +11,6 @@ NVFLAGS := $(EXTRA) $(ARCH) -O3 -lineinfo -std=c++17 -Xcompiler -fPIC,-Wall,-Wno
 LIB    := $(PKG)/libb200lz4.so
 BOUNDS := $(PKG)/libb200lz4_bounds.so
 GEN    := $(PKG)/datagen/libb200gen.so
-HOSTT  := $(PKG)/csrc/host_mirror_test
 
 CU_SRCS  := $(wildcard $(CSRC)/*.cu)
 CU_HDRS  := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) $(wildcard $(CSRC)/*.hpp) include/b200lz4.h

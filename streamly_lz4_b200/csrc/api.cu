@@ -2,6 +2,7 @@
 // the batched host/device entry points, re-framing and the legacy LZ4_* aliases.
 // There is no CPU codec in this library: every compress/decompress call runs the
 // sm_100a kernels, and fails with B200LZ4_E_CUDA when no such device is usable.
+// What the host batch calls decide before they touch the device is in host_plan.h.
 #include <algorithm>
 #include <climits>
 #include <cstdio>
@@ -15,9 +16,12 @@
 #include <vector>
 
 #include "b200lz4.h"
+#include "host_plan.h"
 #include "kernels.h"
 
 using namespace b200lz4;
+using namespace hostplan;
+static_assert(kMaxInputSize == kMaxInput, "host_plan.h restates LZ4_MAX_INPUT_SIZE");
 
 namespace {
 
@@ -31,47 +35,40 @@ int fail_cuda(cudaError_t e, const char* what)
 }
 #define CU(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return fail_cuda(e__, #call); } while (0)
 
-inline int bound_of(int n) { return ((unsigned)n > (unsigned)kMaxInput) ? 0 : n + n / 255 + 16; }
-inline int64_t align16(int64_t v) { return (v + 15) & ~int64_t(15); }
-
-struct DevBuf {
+// grow-only buffer in device memory, or (kPinned) in page-locked host memory the device can see: kernels mirror sizes into it
+template <bool kPinned>
+struct Buf {
     void* p = nullptr; size_t cap = 0;
     int ensure(size_t bytes)
     {
         if (bytes <= cap) return 0;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
+        release();
         size_t want = bytes + bytes / 8 + 4096;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e != cudaSuccess) { p = nullptr; return fail(B200LZ4_E_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e)); }
+        cudaError_t e = kPinned ? cudaHostAlloc(&p, want, cudaHostAllocMapped | cudaHostAllocPortable) : cudaMalloc(&p, want);
+        if (e != cudaSuccess) { p = nullptr; return fail(B200LZ4_E_NOMEM, std::string(kPinned ? "cudaHostAlloc: " : "cudaMalloc: ") + cudaGetErrorString(e)); }
         cap = want;
         return 0;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    void release() { if (p) { if (kPinned) cudaFreeHost(p); else cudaFree(p); } p = nullptr; cap = 0; }
 };
-struct PinBuf {
-    void* p = nullptr; size_t cap = 0;
-    int ensure(size_t bytes)
+
+// the device timeline of one host batch call
+struct CallEvents {
+    cudaEvent_t start = nullptr, h2d_end = nullptr;         // H2D stream: before the call's first and after its last copy
+    cudaEvent_t k0 = nullptr;                               // before the first kernel
+    cudaEvent_t d0 = nullptr, d1 = nullptr;                 // D2H stream: t_d2h
+    cudaEvent_t h2d[kMaxGroups] = {}, k[kMaxGroups] = {};   // per chunk / group: its kernels may start; its kernels are done
+    template <class F> void each(F f)
     {
-        if (bytes <= cap) return 0;
-        if (p) cudaFreeHost(p);
-        p = nullptr; cap = 0;
-        size_t want = bytes + bytes / 8 + 4096;
-        cudaError_t e = cudaHostAlloc(&p, want, cudaHostAllocMapped | cudaHostAllocPortable);    // device-visible: kernels mirror sizes into it
-        if (e != cudaSuccess) { p = nullptr; return fail(B200LZ4_E_NOMEM, std::string("cudaHostAlloc: ") + cudaGetErrorString(e)); }
-        cap = want;
-        return 0;
+        for (cudaEvent_t* e : {&start, &h2d_end, &k0, &d0, &d1}) f(*e);
+        for (auto& e : h2d) f(e);
+        for (auto& e : k) f(e);
     }
-    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
 };
 
 }  // namespace
 
-constexpr int kMaxChunks = 6;           // pipeline depth of the host batch calls (H2D + D2H + chunk streams must fit the
-                                        // 8 hardware queues of the default CUDA_DEVICE_MAX_CONNECTIONS, else chunks serialize)
 constexpr int kKernelStreams = kMaxChunks;   // one stream per chunk: chunk kernels must be able to overlap
-constexpr int kMaxGroups = 16;          // streamed compress call: block groups (events, work counters, arrival flags)
-constexpr int kMaxSegs = 16;            // ... and segments a block is cut into on its way to / from the device
 constexpr size_t kFlagBytes = 1024 + kMaxGroups * kMaxSegs * sizeof(uint32_t);   // ctx->d_flags: see b200lz4_ctx
 
 struct b200lz4_ctx {
@@ -79,11 +76,10 @@ struct b200lz4_ctx {
     cudaStream_t stream = nullptr;                  // H2D + bookkeeping
     cudaStream_t kstream[kKernelStreams] = {};      // chunk kernels (run concurrently)
     cudaStream_t dstream = nullptr;                 // D2H
-    Scratch* scratch = nullptr;                     // kMaxChunks records: one work counter per in-flight kernel
-    DevBuf d_src, d_slots, d_out, d_desc, d_wide;   // d_wide: descriptor rings of decompress_kernel_wide (one slice per chunk)
-    PinBuf h_desc;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t ev_h2d[kMaxGroups] = {}, ev_k[kMaxGroups] = {}, ev_k0 = nullptr, ev_d0 = nullptr, ev_d1 = nullptr;
+    Scratch* scratch = nullptr;                     // kMaxGroups records: one work counter per in-flight kernel
+    Buf<false> d_src, d_slots, d_out, d_desc, d_wide;   // d_wide: descriptor rings of decompress_kernel_wide (one slice per chunk)
+    Buf<true> h_desc;
+    CallEvents ev;
     // streamed compress call (compress_host_streamed): per-group arrival flags + finder cycle counters in HBM, the
     // constants the copy stream writes into the flags, and what earlier calls measured (the copy schedule is tuned by it)
     uint32_t* d_flags = nullptr;            // [kMaxGroups] u32 flags, then at byte 64: u64 busy cycles, u64 bytes; at byte 1024:
@@ -112,29 +108,7 @@ struct b200lz4_dstream {
 
 namespace {
 
-// carve typed arrays out of one host/device descriptor block
-struct Carver {
-    size_t off = 0;
-    size_t take(size_t bytes) { size_t o = off; off = (off + bytes + 15) & ~size_t(15); return o; }
-};
-
-int check_blocks(const int64_t* off, const int32_t* len, int n, int64_t bytes)
-{
-    for (int i = 0; i < n; i++) {
-        if (len[i] < 0 || off[i] < 0 || off[i] + (int64_t)len[i] > bytes)
-            return fail(B200LZ4_E_ARG, "block " + std::to_string(i) + " lies outside the source buffer");
-    }
-    return 0;
-}
-int check_streams(const int32_t* first, int n_streams, int n_blocks)
-{
-    if (!first) return 0;
-    if (n_streams < 0 || (n_streams == 0 && n_blocks != 0)) return fail(B200LZ4_E_ARG, "n_streams");
-    if (n_streams == 0) return 0;
-    if (first[0] != 0 || first[n_streams] != n_blocks) return fail(B200LZ4_E_ARG, "stream_first must start at 0 and end at n_blocks");
-    for (int s = 0; s < n_streams; s++) if (first[s] > first[s + 1]) return fail(B200LZ4_E_ARG, "stream_first must be non-decreasing");
-    return 0;
-}
+int fail(const Verdict& v) { return fail(v.code, v.msg); }
 
 int set_dict_fields(CState* d_state, uint8_t* buf, uint32_t cap, cudaStream_t st)
 {
@@ -169,48 +143,6 @@ int sync_all(b200lz4_ctx* c)
     CU(cudaStreamSynchronize(c->dstream));
     if (c->fstream) CU(cudaStreamSynchronize(c->fstream));
     return 0;
-}
-
-// ---- pipeline planning ------------------------------------------------------
-// A host batch is cut into up to kMaxChunks chunks of whole streams (independent mode: whole
-// blocks).  Chunk k's H2D copy, its kernels and its D2H copy run on three different CUDA
-// streams, so that transfers in both directions overlap the kernels of neighbouring chunks;
-// the chunk kernels themselves run concurrently on kKernelStreams streams because a codec
-// kernel is bound by per-block latency, not by the number of blocks it is given.
-struct Chunk { int b0, b1, s0, s1; int64_t lo, hi; };
-
-int plan_chunks(const int64_t* off, const int32_t* len, int n, const int32_t* first, int ns, Chunk* out, bool early_start = false)
-{
-    int64_t total = 0;
-    for (int i = 0; i < n; i++) total += len[i];
-    // Chunk k becomes ready when its H2D copy lands and finishes one block latency later, so the end of the
-    // call is "last byte arrives + block latency + D2H of the last chunk": keep the last chunk small.
-    // early_start (mirrored decompress: the output leaves from inside the kernels, so the call ends one PCIe-bound stretch
-    // after the FIRST chunk has landed): a small first chunk instead of a small last one
-    static const double kShareTail[kMaxChunks] = {0.14, 0.20, 0.20, 0.20, 0.18, 0.08};
-    static const double kShareHead[kMaxChunks] = {0.03, 0.09, 0.18, 0.24, 0.24, 0.22};
-    const double* kShare = early_start ? kShareHead : kShareTail;
-    const bool small = total < (int64_t(48) << 20);
-    int k = 0, unit = 0;
-    const int units = first ? ns : n;
-    int64_t done = 0;
-    while (unit < units) {
-        Chunk c; c.s0 = unit; c.b0 = first ? first[unit] : unit;
-        double upto = 0;
-        for (int q = 0; q <= k; q++) upto += kShare[q];
-        const int64_t target = (small || k == kMaxChunks - 1) ? total : (int64_t)(upto * (double)total);
-        while (unit < units && (done < target || k == kMaxChunks - 1 || small)) {
-            const int u0 = first ? first[unit] : unit, u1 = first ? first[unit + 1] : unit + 1;
-            for (int i = u0; i < u1; i++) done += len[i];
-            unit++;
-        }
-        c.s1 = unit; c.b1 = first ? first[unit] : unit;
-        c.lo = INT64_MAX; c.hi = 0;
-        for (int i = c.b0; i < c.b1; i++) { c.lo = std::min(c.lo, off[i]); c.hi = std::max(c.hi, off[i] + (int64_t)len[i]); }
-        if (c.lo > c.hi) c.lo = c.hi = 0;
-        out[k++] = c;
-    }
-    return k;
 }
 
 // ---- hardware-queue aliasing ---------------------------------------------------
@@ -285,14 +217,131 @@ int probe_stream_aliasing(b200lz4_ctx* c)
     return 0;
 }
 
-// One segment of every block of a group: `rows` ranges of `width` bytes at constant pitches, as one pitched copy.  (The copy
-// engine moves a pitched copy row by row: measured 9 % slower than one plain copy of the same bytes on an idle link and
-// 15 % slower while the opposite direction is busy, which is why segments are not made smaller than they have to be.)
-int copy_rows(uint8_t* dst, size_t dpitch, const uint8_t* src, size_t spitch, size_t width, size_t rows, cudaMemcpyKind kind, cudaStream_t st)
+// ---- shared steps of the host pipelines ------------------------------------------------------------------------------
+// A plain host batch is cut into up to kMaxChunks chunks of whole streams (independent mode: whole blocks, host_plan.h:
+// plan_chunks).  Chunk k's H2D copy, its kernels and its D2H copy run on three different CUDA streams, so that transfers
+// in both directions overlap the kernels of neighbouring chunks; the chunk kernels themselves run concurrently on
+// kKernelStreams streams because a codec kernel is bound by per-block latency, not by the number of blocks it is given.
+// The streamed calls cut the batch into groups instead, and blocks into segments.
+
+int ensure_desc(b200lz4_ctx* c, const DescLayout& lay)
 {
-    if (rows == 0 || width == 0) return 0;
-    if (rows == 1 || (width == dpitch && width == spitch)) CU(cudaMemcpyAsync(dst, src, width * rows, kind, st));
-    else CU(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, st));
+    const int rc = c->h_desc.ensure(lay.bytes);
+    return rc ? rc : c->d_desc.ensure(lay.bytes);
+}
+
+// Range k (chunk or group): H2D copy of its source bytes (none for an empty span), then its kernels go to ks behind it
+int start_range(b200lz4_ctx* c, int k, cudaStream_t ks, Span span, uint8_t* d_src, const uint8_t* hsrc)
+{
+    if (span.hi > span.lo) CU(cudaMemcpyAsync(d_src + span.lo, hsrc + span.lo, (size_t)(span.hi - span.lo), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaEventRecord(c->ev.h2d[k], c->stream));
+    CU(cudaStreamWaitEvent(ks, c->ev.h2d[k], 0));
+    if (k == 0) CU(cudaEventRecord(c->ev.k0, ks));
+    return 0;
+}
+
+// the kernel arguments every host pipeline fills alike: the batch's descriptors in d_desc, the launch's units of range r
+template <class Args>
+Args launch_args(const DescLayout& lay, void* dd, const uint8_t* d_src, uint8_t* d_slots, int n, int header, const Range& r,
+                 Scratch* scratch, bool linked, bool states)
+{
+    Args a{};
+    a.src = d_src; a.src_off = lay.src_off_in(dd); a.src_len = lay.src_len_in(dd); a.n_blocks = n;
+    a.first_block = r.b0; a.n_streams = r.u1 - r.u0;
+    a.stream_first = linked ? lay.first_in(dd) + r.u0 : nullptr;
+    a.states = states ? lay.states_in(dd) + r.u0 : nullptr;
+    a.dst = d_slots; a.dst_off = lay.slot_off_in(dd); a.out_len = lay.out_len_in(dd);
+    a.header = header; a.scratch = scratch;
+    return a;
+}
+
+// Compress range k, then pack its blocks behind each other in d_out: the scan kernel mirrors sizes and offsets into the
+// pinned descriptor block (device-visible host memory), range k's n_k + 1 offsets from entry b0 + k of out_off.
+int compress_range(b200lz4_ctx* c, const CompressArgs& a, const DescLayout& lay, const Range& r, int k, uint8_t* d_out, cudaStream_t ks)
+{
+    void* hd = c->h_desc.p;
+    CU(launch_compress(a, ks));
+    CompactArgs g{a.dst, a.dst_off + r.b0, a.out_len + r.b0, r.b1 - r.b0, a.header, d_out + lay.slot_off_in(hd)[r.b0],
+                  lay.out_off_in(c->d_desc.p) + r.b0 + k, lay.out_off_in(hd) + r.b0 + k, lay.out_len_in(hd) + r.b0};
+    CU(launch_compact(g, ks));
+    c->launches += kernel_launches_per_compress() + kernel_launches_per_compact();
+    CU(cudaEventRecord(c->ev.k[k], ks));
+    return 0;
+}
+
+// As each range's kernels finish, its compacted bytes go home behind those of the ranges before it
+int drain_compacted(b200lz4_ctx* c, const Range* r, int nr, const DescLayout& lay, const uint8_t* d_out,
+                    void* dst, int64_t dst_cap, int64_t* dst_off, int n, bool log)
+{
+    const int64_t* h_out_off = lay.out_off_in(c->h_desc.p);
+    const int64_t* h_slot_off = lay.slot_off_in(c->h_desc.p);
+    int64_t base = 0;
+    int rc = 0;
+    for (int k = 0; k < nr; k++) {
+        CU(cudaEventSynchronize(c->ev.k[k]));
+        if (log) { fprintf(stderr, "[b200lz4] streamed: group %d done\n", k); fflush(stderr); }
+        const int nk = r[k].b1 - r[k].b0;
+        const int64_t* off_k = h_out_off + r[k].b0 + k;
+        const int64_t total_k = off_k[nk];
+        for (int i = 0; i < nk; i++) dst_off[r[k].b0 + i] = base + off_k[i];
+        if (base + total_k > dst_cap) { rc = fail(B200LZ4_E_NOMEM, "dst_cap too small"); break; }
+        if (total_k) CU(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + base, d_out + h_slot_off[r[k].b0], (size_t)total_k,
+                                        cudaMemcpyDeviceToHost, c->dstream));
+        base += total_k;
+    }
+    dst_off[n] = base;
+    return rc;
+}
+
+// Segment s of every block of group grp as one pitched copy (block i at dst + i * dpitch and src + i * spitch), queued
+// after a copy of its own of the share of a short last block (last_len < L).  The copy engine moves a pitched copy row by
+// row: measured 9 % slower than one plain copy of the same bytes on an idle link and 15 % slower while the opposite
+// direction is busy, which is why segments are not made smaller than they have to be.
+int copy_piece(uint8_t* dst, size_t dpitch, const uint8_t* src, size_t spitch, const Geometry& geo, const Range& grp,
+               int n, int L, int last_len, int s, cudaMemcpyKind kind, cudaStream_t st)
+{
+    const int lo = s * geo.seg, width = std::min(geo.seg, L - lo);
+    int rows = grp.b1 - grp.b0;
+    if (grp.b1 == n && last_len < L) {
+        rows--;
+        const int wl = std::min(width, last_len - lo);
+        if (wl > 0) CU(cudaMemcpyAsync(dst + dpitch * (n - 1) + lo, src + spitch * (n - 1) + lo, (size_t)wl, kind, st));
+    }
+    if (rows <= 0) return 0;
+    dst += dpitch * grp.b0 + lo;
+    src += spitch * grp.b0 + lo;
+    if (rows == 1 || ((size_t)width == dpitch && (size_t)width == spitch)) CU(cudaMemcpyAsync(dst, src, (size_t)width * rows, kind, st));
+    else CU(cudaMemcpy2DAsync(dst, dpitch, src, spitch, (size_t)width, (size_t)rows, kind, st));
+    return 0;
+}
+
+// Every host pipeline ends here once it has queued work, failed (rc) or not, so that nothing it queued is left running on
+// the ctx's streams.  Then the timing split, the block sizes, the device timeline of its ranges (B200LZ4_DEBUG; label
+// NULL: none) and the per-block check: a compressed block failed with a size <= 0, a decompressed one with a size < 0.
+int finish_call(b200lz4_ctx* c, int rc, const Range* r, int nr, const char* label, const char* landed,
+                const int32_t* h_out_len, int32_t* out_len, int n, bool decode)
+{
+    const cudaError_t e = cudaEventRecord(c->ev.d1, c->dstream);
+    if (e != cudaSuccess && !rc) rc = fail_cuda(e, "cudaEventRecord(ev.d1)");
+    if (const int s = sync_all(c)) return s;
+    if (rc) return rc;
+    cudaEventElapsedTime(&c->t_h2d, c->ev.start, c->ev.h2d_end);
+    cudaEventElapsedTime(&c->t_kernel, c->ev.k0, c->ev.k[nr - 1]);
+    cudaEventElapsedTime(&c->t_d2h, c->ev.d0, c->ev.d1);
+    memcpy(out_len, h_out_len, sizeof(int32_t) * n);
+    if (label && getenv("B200LZ4_DEBUG")) {         // ms since the call's first event
+        float t = 0;
+        for (int k = 0; k < nr; k++) {
+            float a = 0, b = 0;
+            cudaEventElapsedTime(&a, c->ev.start, c->ev.h2d[k]); cudaEventElapsedTime(&b, c->ev.start, c->ev.k[k]);
+            fprintf(stderr, "[b200lz4] %s %d: blocks %d..%d  %s %.2f  kernels done %.2f\n", label, k, r[k].b0, r[k].b1, landed, a, b);
+        }
+        cudaEventElapsedTime(&t, c->ev.start, c->ev.h2d_end); fprintf(stderr, "[b200lz4] h2d done %.2f\n", t);
+        cudaEventElapsedTime(&t, c->ev.start, c->ev.d1); fprintf(stderr, "[b200lz4] d2h done %.2f\n", t);
+    }
+    for (int i = 0; i < n; i++)
+        if (decode ? out_len[i] < 0 : out_len[i] <= 0)
+            return fail(B200LZ4_E_BLOCK, "block " + std::to_string(i) + (decode ? " failed to decompress" : " failed to compress"));
     return 0;
 }
 
@@ -303,32 +352,11 @@ int copy_rows(uint8_t* dst, size_t dpitch, const uint8_t* src, size_t spitch, si
 // segments and block groups into 2-D copies (one segment of every block of a group per copy), each followed by a 4-byte
 // copy that bumps the group's arrival flag; the group's kernel is launched as soon as its FIRST segment has landed and
 // its finders wait for later segments only if they get there before the data (compress.cu: kStreamed).  Pieces are sent
-// in deadline order, key(g, s) = g + s * w: w = 0 is the plain block order, a large w sends segment 0 of every block
-// first.  w is chosen so that a group's segments arrive at the pace its finders consume them, from what the previous
-// streamed call on this ctx measured (finder cycles per byte, H2D rate); then the end of the call is "last byte lands +
-// one SEGMENT latency + the last group's D2H".  The device layout is private to the call (128-byte aligned block starts,
-// 128 bytes of gap), so no L1 sector is read before it is complete.
-struct StreamShape { int L; int64_t P; bool ok; };
-constexpr double kStreamSpread = 1.5;    // measured: a little later is better than a little early (the D2H copies of finished groups
-                                        // share the link, and a starved finder only waits while an early piece delays everyone else's)
+// in deadline order (host_plan.h: piece_order), with w chosen so that a group's segments arrive at the pace its finders
+// consume them, from what the previous streamed call on this ctx measured (finder cycles per byte, H2D rate); then the
+// end of the call is "last byte lands + one SEGMENT latency + the last group's D2H".  The device layout is private to the
+// call (128-byte aligned block starts, 128 bytes of gap), so no L1 sector is read before it is complete.
 constexpr int kStreamedGaveUp = -1000;  // internal: compress_host retries through the plain pipeline
-
-StreamShape streamed_shape(const int64_t* off, const int32_t* len, int n, const int32_t* stream_first, const int32_t* block_cap)
-{
-    StreamShape r{0, 0, false};
-    const bool off_env = getenv("B200LZ4_NO_STREAMED") != nullptr;      // (read per call: bench.py times both pipelines in one process)
-    if (off_env || stream_first || block_cap || n < 96) return r;
-    const int L = len[0];
-    if (L < 65536 || (int64_t)L * n < (int64_t(96) << 20)) return r;
-    const int64_t P = off[1] - off[0];
-    if (P < L) return r;
-    for (int i = 0; i < n; i++) {
-        if (off[i] != off[0] + P * i) return r;
-        if (i < n - 1 ? len[i] != L : (len[i] <= 0 || len[i] > L)) return r;
-    }
-    r.L = L; r.P = P; r.ok = true;
-    return r;
-}
 
 int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_off, const int32_t* src_len, int n,
                            const StreamShape& shp, int accel, int header,
@@ -338,61 +366,28 @@ int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_o
     const int L = shp.L;
     const int nks = c->n_kgood;             // kernel streams that cannot block the copy stream (>= 2, checked by the caller)
     const int64_t DP = ((int64_t)L + 127) / 128 * 128 + 128;       // device pitch
-    int64_t total = 0;
-    for (int i = 0; i < n; i++) total += src_len[i];
-
-    // ---- schedule parameters
-    const char* env_w = getenv("B200LZ4_STREAM_W");      // measurement overrides (read per call)
-    const char* env_g = getenv("B200LZ4_STREAM_G");
-    const char* env_s = getenv("B200LZ4_STREAM_S");
-    const char* env_f = getenv("B200LZ4_STREAM_FLAG");
+    const int64_t total = total_bytes(src_len, n);
+    const char* env_f = getenv("B200LZ4_STREAM_FLAG");      // measurement overrides (read per call)
     const bool flag_by_kernel = env_f && env_f[0] == 'k';
     const bool flag_inline_copy = env_f && env_f[0] == 'c';
     const bool flag_separate = !flag_by_kernel && !flag_inline_copy && c->fstream != nullptr;
-    const double ns_per_byte = c->est_ns_per_byte > 0 ? c->est_ns_per_byte : 12.0;       // first call: ~85 MB/s per finder
-    const double h2d_gbs = c->est_h2d_gbs > 0 ? c->est_h2d_gbs : 50.0;
-    const double t_block_ms = ns_per_byte * 1.1 * L * 1e-6, t_h2d_ms = (double)total / (h2d_gbs * 1e6);
-    const double rho = t_block_ms / t_h2d_ms;
-    int G = env_g ? atoi(env_g) : (rho <= 0.45 ? 2 * nks : nks);        // a group runs behind group g - nks on its stream
-    if (G < 1) G = 1;
-    if (G > kMaxGroups) G = kMaxGroups;
-    // segments of ~160 000 bytes (rows of a pitched copy: smaller ones cost copy-engine efficiency while the D2H direction is
-    // busy, larger ones lengthen the tail, which is one segment's worth of finder time): 4 for 640 000-byte blocks, 16 from 2.5 MB
-    int S = env_s ? atoi(env_s) : (int)std::min<int64_t>(kMaxSegs, std::max<int64_t>(4, ((int64_t)L + 80000) / 160000));
-    if (S < 1) S = 1;
-    if (S > kMaxSegs) S = kMaxSegs;
-    const int seg = (int)((((int64_t)L + S - 1) / S + 127) / 128 * 128);
-    S = (L + seg - 1) / seg;
-    const int per_group = (n + G - 1) / G;
-    G = (n + per_group - 1) / per_group;
-    // a group's S pieces are (S - 1) * w key units apart, the whole schedule spans (G - 1) + (S - 1) * w units in t_h2d:
-    // the last piece of a group should land when its finders get there, (S - 1) / S of a block time after the first
-    double w = (double)G;
-    if (S - rho * (S - 1) > 0.01) w = kStreamSpread * rho * (G - 1) / (S - rho * (S - 1));
-    if (env_w) w = atof(env_w);
-    if (w > G) w = G;
+    const Geometry geo = compress_geometry(n, L, total, nks, c->est_ns_per_byte, c->est_h2d_gbs, getenv("B200LZ4_STREAM_G"),
+                                           getenv("B200LZ4_STREAM_S"), getenv("B200LZ4_STREAM_W"));
+    Range groups[kMaxGroups];
+    plan_groups(geo, n, groups);
 
-    // ---- descriptor block (device offsets are the private layout)
-    Carver cv;
-    const size_t o_src_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_slot_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_src_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_upload_end = cv.off;
-    const size_t o_out_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_out_off = cv.take(sizeof(int64_t) * (n + G));
-    const size_t desc_bytes = cv.off;
-    if ((rc = c->h_desc.ensure(desc_bytes))) return rc;
-    if ((rc = c->d_desc.ensure(desc_bytes))) return rc;
-    uint8_t* hd = static_cast<uint8_t*>(c->h_desc.p);
-    uint8_t* dd = static_cast<uint8_t*>(c->d_desc.p);
-    int64_t* h_src_off = reinterpret_cast<int64_t*>(hd + o_src_off);
-    int64_t* h_slot_off = reinterpret_cast<int64_t*>(hd + o_slot_off);
-    memcpy(hd + o_src_len, src_len, sizeof(int32_t) * n);
+    const DescLayout lay(n, n, 0, 0, 0, n + geo.G, 0);
+    if ((rc = ensure_desc(c, lay))) return rc;
+    void* hd = c->h_desc.p;
+    void* dd = c->d_desc.p;
+    int64_t* h_src_off = lay.src_off_in(hd);
+    int64_t* h_slot_off = lay.slot_off_in(hd);
+    memcpy(lay.src_len_in(hd), src_len, sizeof(int32_t) * n);
     int64_t slots_total = 0;
     for (int i = 0; i < n; i++) {
         h_src_off[i] = DP * i;
         h_slot_off[i] = slots_total;
-        slots_total += align16((int64_t)bound_of(src_len[i]) + header + 16);
+        slots_total += compress_slot(compress_cap(src_len[i], header));
     }
     if ((rc = c->d_src.ensure((size_t)(DP * n) + 256))) return rc;
     if ((rc = c->d_slots.ensure((size_t)slots_total + 64))) return rc;
@@ -401,99 +396,43 @@ int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_o
     uint8_t* d_src = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(c->d_src.p) + 127) & ~uintptr_t(127));
     uint8_t* d_slots = static_cast<uint8_t*>(c->d_slots.p);
     uint8_t* d_out = static_cast<uint8_t*>(c->d_out.p);
-    int64_t* d_out_off = reinterpret_cast<int64_t*>(dd + o_out_off);
-    int32_t* d_out_len = reinterpret_cast<int32_t*>(dd + o_out_len);
     unsigned long long* d_busy = reinterpret_cast<unsigned long long*>(reinterpret_cast<uint8_t*>(c->d_flags) + 64);
-
-    // ---- pieces in deadline order
-    struct Piece { int g, s; double key; };
-    std::vector<Piece> pieces;
-    pieces.reserve((size_t)G * S);
-    for (int g = 0; g < G; g++) for (int s2 = 0; s2 < S; s2++) pieces.push_back({g, s2, g + s2 * w});
-    std::stable_sort(pieces.begin(), pieces.end(), [](const Piece& x, const Piece& y) { return x.key < y.key; });
+    const std::vector<Piece> pieces = piece_order(geo);
+    const bool dbg = getenv("B200LZ4_DEBUG") != nullptr;
 
     cudaStream_t st = c->stream;
-    CU(cudaEventRecord(c->ev[0], st));
-    CU(cudaMemsetAsync(c->d_flags, 0, 256, st));
-    CU(cudaMemcpyAsync(dd, hd, o_upload_end, cudaMemcpyHostToDevice, st));
-    bool first_kernel = true;
-    for (const Piece& pc : pieces) {
-        const int b0 = pc.g * per_group, b1 = std::min(n, b0 + per_group);
-        const int lo = pc.s * seg, width = std::min(seg, L - lo);
-        int rows = b1 - b0;
-        if (b1 == n && src_len[n - 1] < L) {        // the batch's last block may be shorter: its share of the segment goes separately
-            rows--;
-            const int wl = std::min(width, src_len[n - 1] - lo);
-            if (wl > 0) CU(cudaMemcpyAsync(d_src + DP * (n - 1) + lo, hsrc + src_off[n - 1] + lo, (size_t)wl, cudaMemcpyHostToDevice, st));
+    auto enqueue = [&]() -> int {
+        CU(cudaEventRecord(c->ev.start, st));
+        CU(cudaMemsetAsync(c->d_flags, 0, 256, st));
+        CU(cudaMemcpyAsync(dd, hd, lay.upload, cudaMemcpyHostToDevice, st));
+        for (size_t pi = 0; pi < pieces.size(); pi++) {
+            const Piece pc = pieces[pi];
+            if ((rc = copy_piece(d_src, (size_t)DP, hsrc + src_off[0], (size_t)shp.P, geo, groups[pc.g], n, L, src_len[n - 1], pc.s,
+                                 cudaMemcpyHostToDevice, st))) return rc;
+            if (flag_separate) {                // the flag is raised from another stream: the next piece starts right behind this one
+                while (c->ev_piece.size() <= pi) { cudaEvent_t e; CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); c->ev_piece.push_back(e); }
+                CU(cudaEventRecord(c->ev_piece[pi], st));
+                CU(cudaStreamWaitEvent(c->fstream, c->ev_piece[pi], 0));
+                CU(launch_set_flag(c->d_flags + pc.g, (uint32_t)(pc.s + 1), c->fstream));
+                c->launches++;
+            }
+            else if (flag_by_kernel) CU(launch_set_flag(c->d_flags + pc.g, (uint32_t)(pc.s + 1), st));
+            else CU(cudaMemcpyAsync(c->d_flags + pc.g, c->h_const + (pc.s + 1), sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+            if (pc.s != 0) continue;
+            // first segment of the group is on its way: queue the group's kernels behind it
+            cudaStream_t ks = c->kstream[pc.g % nks];
+            if ((rc = start_range(c, pc.g, ks, Span{0, 0}, d_src, hsrc))) return rc;
+            CompressArgs a = launch_args<CompressArgs>(lay, dd, d_src, d_slots, n, header, groups[pc.g], c->scratch + pc.g, false, false);
+            a.accel = accel; a.arrived = c->d_flags + pc.g; a.seg_bytes = geo.seg; a.busy_cycles = d_busy;
+            if ((rc = compress_range(c, a, lay, groups[pc.g], pc.g, d_out, ks))) return rc;
         }
-        if (rows > 0 && (rc = copy_rows(d_src + DP * b0 + lo, (size_t)DP, hsrc + src_off[b0] + lo, (size_t)shp.P, (size_t)width, (size_t)rows,
-                                        cudaMemcpyHostToDevice, st))) return rc;
-        if (flag_separate) {                // the flag is raised from another stream: the next piece starts right behind this one
-            const size_t pi = (size_t)(&pc - pieces.data());
-            while (c->ev_piece.size() <= pi) { cudaEvent_t e; CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); c->ev_piece.push_back(e); }
-            CU(cudaEventRecord(c->ev_piece[pi], st));
-            CU(cudaStreamWaitEvent(c->fstream, c->ev_piece[pi], 0));
-            CU(launch_set_flag(c->d_flags + pc.g, (uint32_t)(pc.s + 1), c->fstream));
-            c->launches++;
-        }
-        else if (flag_by_kernel) CU(launch_set_flag(c->d_flags + pc.g, (uint32_t)(pc.s + 1), st));
-        else CU(cudaMemcpyAsync(c->d_flags + pc.g, c->h_const + (pc.s + 1), sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-        if (pc.s != 0) continue;
-        // first segment of the group is on its way: queue the group's kernels behind it
-        CU(cudaEventRecord(c->ev_h2d[pc.g], st));
-        cudaStream_t ks = c->kstream[pc.g % nks];
-        CU(cudaStreamWaitEvent(ks, c->ev_h2d[pc.g], 0));
-        if (first_kernel) { CU(cudaEventRecord(c->ev_k0, ks)); first_kernel = false; }
-        CompressArgs a{};
-        a.src = d_src;
-        a.src_off = reinterpret_cast<const int64_t*>(dd + o_src_off);
-        a.src_len = reinterpret_cast<const int32_t*>(dd + o_src_len);
-        a.n_blocks = n;
-        a.first_block = b0;
-        a.n_streams = b1 - b0;
-        a.dst = d_slots;
-        a.dst_off = reinterpret_cast<const int64_t*>(dd + o_slot_off);
-        a.out_len = d_out_len;
-        a.accel = accel; a.header = header; a.scratch = c->scratch + pc.g;
-        a.arrived = c->d_flags + pc.g; a.seg_bytes = seg; a.busy_cycles = d_busy;
-        CU(launch_compress(a, ks));
-        CompactArgs cg{d_slots, a.dst_off + b0, d_out_len + b0, b1 - b0, header, d_out + h_slot_off[b0], d_out_off + b0 + pc.g,
-                       reinterpret_cast<int64_t*>(hd + o_out_off) + b0 + pc.g, reinterpret_cast<int32_t*>(hd + o_out_len) + b0};
-        CU(launch_compact(cg, ks));
-        c->launches += kernel_launches_per_compress() + kernel_launches_per_compact();
-        CU(cudaEventRecord(c->ev_k[pc.g], ks));
-    }
-    CU(cudaEventRecord(c->ev[1], st));
-    const bool dbg = getenv("B200LZ4_DEBUG") != nullptr;
-    if (dbg) { fprintf(stderr, "[b200lz4] streamed: %zu pieces queued (G %d S %d seg %d w %.3f)\n", pieces.size(), G, S, seg, w); fflush(stderr); }
-
-    // drain: as each group's sizes arrive, send its compacted bytes home
-    const int32_t* h_out_len = reinterpret_cast<const int32_t*>(hd + o_out_len);
-    const int64_t* h_out_off = reinterpret_cast<const int64_t*>(hd + o_out_off);
-    int64_t base = 0;
-    int result = 0;
-    CU(cudaEventRecord(c->ev_d0, c->dstream));
-    for (int g = 0; g < G; g++) {
-        const int b0 = g * per_group, b1 = std::min(n, b0 + per_group);
-        CU(cudaEventSynchronize(c->ev_k[g]));
-        if (dbg) { fprintf(stderr, "[b200lz4] streamed: group %d done\n", g); fflush(stderr); }
-        const int nk = b1 - b0;
-        const int64_t* off_k = h_out_off + b0 + g;
-        const int64_t total_k = off_k[nk];
-        for (int i = 0; i < nk; i++) dst_off[b0 + i] = base + off_k[i];
-        if (base + total_k > dst_cap) { result = fail(B200LZ4_E_NOMEM, "dst_cap too small"); break; }
-        if (total_k) CU(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + base, d_out + h_slot_off[b0], (size_t)total_k,
-                                        cudaMemcpyDeviceToHost, c->dstream));
-        base += total_k;
-    }
-    dst_off[n] = base;
-    CU(cudaEventRecord(c->ev_d1, c->dstream));
-    if ((rc = sync_all(c))) return rc;
-    if (result) return result;
-    memcpy(out_len, h_out_len, sizeof(int32_t) * n);
-    cudaEventElapsedTime(&c->t_h2d, c->ev[0], c->ev[1]);
-    cudaEventElapsedTime(&c->t_kernel, c->ev_k0, c->ev_k[G - 1]);
-    cudaEventElapsedTime(&c->t_d2h, c->ev_d0, c->ev_d1);
+        CU(cudaEventRecord(c->ev.h2d_end, st));
+        if (dbg) { fprintf(stderr, "[b200lz4] streamed: %zu pieces queued (G %d S %d seg %d w %.3f)\n", pieces.size(), geo.G, geo.S, geo.seg, geo.w); fflush(stderr); }
+        CU(cudaEventRecord(c->ev.d0, c->dstream));
+        return drain_compacted(c, groups, geo.G, lay, d_out, dst, dst_cap, dst_off, n, dbg);
+    };
+    rc = finish_call(c, enqueue(), groups, geo.G, "group", "first segment landed", lay.out_len_in(hd), out_len, n, false);
+    if (rc && rc != B200LZ4_E_BLOCK) return rc;
     // what this call measured tunes the next one's schedule
     unsigned long long busy[3] = {0, 0, 0};
     CU(cudaMemcpy(busy, d_busy, sizeof busy, cudaMemcpyDeviceToHost));
@@ -507,19 +446,8 @@ int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_o
         c->est_h2d_gbs = c->est_h2d_gbs > 0 ? 0.5 * c->est_h2d_gbs + 0.5 * gbs : gbs;
     }
     c->streamed_calls++;
-    if (getenv("B200LZ4_DEBUG")) {
-        fprintf(stderr, "[b200lz4] streamed: G %d S %d seg %d w %.3f rho %.3f  est %.2f ns/B  h2d %.1f GB/s\n", G, S, seg, w, rho, c->est_ns_per_byte, c->est_h2d_gbs);
-        float t = 0;
-        for (int g = 0; g < G; g++) {
-            float x = 0, y = 0;
-            cudaEventElapsedTime(&x, c->ev[0], c->ev_h2d[g]); cudaEventElapsedTime(&y, c->ev[0], c->ev_k[g]);
-            fprintf(stderr, "[b200lz4] group %d: first segment landed %.2f  kernels done %.2f\n", g, x, y);
-        }
-        cudaEventElapsedTime(&t, c->ev[0], c->ev[1]); fprintf(stderr, "[b200lz4] h2d done %.2f\n", t);
-        cudaEventElapsedTime(&t, c->ev[0], c->ev_d1); fprintf(stderr, "[b200lz4] d2h done %.2f\n", t);
-    }
-    for (int i = 0; i < n; i++) if (out_len[i] <= 0) return fail(B200LZ4_E_BLOCK, "block " + std::to_string(i) + " failed to compress");
-    return 0;
+    if (dbg) fprintf(stderr, "[b200lz4] streamed: G %d S %d seg %d w %.3f rho %.3f  est %.2f ns/B  h2d %.1f GB/s\n", geo.G, geo.S, geo.seg, geo.w, geo.rho, c->est_ns_per_byte, c->est_h2d_gbs);
+    return rc;
 }
 
 int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
@@ -528,29 +456,25 @@ int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                   int accel, int header, const int32_t* block_cap,
                   void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
-    if (!c) return fail(B200LZ4_E_ARG, "ctx is NULL");
-    if (n < 0 || (n > 0 && (!src_off || !src_len || !dst_off || !out_len))) return fail(B200LZ4_E_ARG, "NULL descriptor array");
-    if (header != 0 && header != 4 && header != 8) return fail(B200LZ4_E_ARG, "header_mode must be 0, 4 or 8");
-    if (streams && !stream_first) return fail(B200LZ4_E_ARG, "streams given without stream_first");
+    const Verdict v = check_batch(Entry::Ctx, false, c, n, header, 0, src, src_bytes, src_off, src_len, dst, dst_off, out_len,
+                                  stream_first, n_streams, streams != nullptr);
+    if (v.code) return fail(v);
     if (n == 0) { if (dst_off) dst_off[0] = 0; return 0; }
-    if (!src || !dst) return fail(B200LZ4_E_ARG, "NULL data buffer");
     int rc;
-    if ((rc = check_blocks(src_off, src_len, n, src_bytes))) return rc;
-    if ((rc = check_streams(stream_first, n_streams, n))) return rc;
     CU(cudaSetDevice(c->device));
     const int ns = stream_first ? n_streams : n;
-    if (!streams) {
-        const StreamShape shp = streamed_shape(src_off, src_len, n, stream_first, block_cap);
-        if (shp.ok) {
-            if ((rc = probe_stream_aliasing(c))) return rc;
-            if (c->n_kgood >= 2) {
-                rc = compress_host_streamed(c, src, src_off, src_len, n, shp, accel, header, dst, dst_cap, dst_off, out_len);
-                if (rc != kStreamedGaveUp) return rc;
-                // finders gave up waiting for their input (should not happen on verified streams): never again on this
-                // ctx, and this batch goes through the plain pipeline
-                c->n_kgood = 0;
-                if (getenv("B200LZ4_DEBUG")) fprintf(stderr, "[b200lz4] streamed call gave up (%s): plain pipeline from now on\n", g_err.c_str());
-            }
+    // (B200LZ4_NO_STREAMED is read per call: bench.py times both pipelines in one process)
+    const StreamShape shp = streamed_shape(src_off, src_len, n, stream_first != nullptr, block_cap != nullptr,
+                                           getenv("B200LZ4_NO_STREAMED") != nullptr);
+    if (shp.ok) {
+        if ((rc = probe_stream_aliasing(c))) return rc;
+        if (c->n_kgood >= 2) {
+            rc = compress_host_streamed(c, src, src_off, src_len, n, shp, accel, header, dst, dst_cap, dst_off, out_len);
+            if (rc != kStreamedGaveUp) return rc;
+            // finders gave up waiting for their input (should not happen on verified streams): never again on this
+            // ctx, and this batch goes through the plain pipeline
+            c->n_kgood = 0;
+            if (getenv("B200LZ4_DEBUG")) fprintf(stderr, "[b200lz4] streamed call gave up (%s): plain pipeline from now on\n", g_err.c_str());
         }
     }
 
@@ -564,131 +488,56 @@ int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
             }
         }
     }
-    Chunk chunks[kMaxChunks];
-    const int nchunks = plan_chunks(src_off, src_len, n, stream_first, ns, chunks);
+    Range chunks[kMaxChunks];
+    const int nchunks = plan_chunks(src_len, n, stream_first, ns, false, chunks);
 
-    // descriptor block
-    Carver cv;
-    const size_t o_src_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_slot_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_src_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_cap = cv.take(sizeof(int32_t) * n);
-    const size_t o_first = cv.take(sizeof(int32_t) * (ns + 1));
-    const size_t o_states = cv.take(sizeof(void*) * ns);
-    const size_t o_upload_end = cv.off;
-    const size_t o_out_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_out_off = cv.take(sizeof(int64_t) * (n + nchunks));
-    const size_t desc_bytes = cv.off;
-    if ((rc = c->h_desc.ensure(desc_bytes))) return rc;
-    if ((rc = c->d_desc.ensure(desc_bytes))) return rc;
-    uint8_t* hd = static_cast<uint8_t*>(c->h_desc.p);
-    uint8_t* dd = static_cast<uint8_t*>(c->d_desc.p);
-    int64_t* h_slot_off = reinterpret_cast<int64_t*>(hd + o_slot_off);
-    int32_t* h_cap = reinterpret_cast<int32_t*>(hd + o_cap);
-    memcpy(hd + o_src_off, src_off, sizeof(int64_t) * n);
-    memcpy(hd + o_src_len, src_len, sizeof(int32_t) * n);
+    const DescLayout lay(n, n, n, ns + 1, ns, n + nchunks, 0);
+    if ((rc = ensure_desc(c, lay))) return rc;
+    void* hd = c->h_desc.p;
+    void* dd = c->d_desc.p;
+    int64_t* h_slot_off = lay.slot_off_in(hd);
+    int32_t* h_cap = lay.cap_in(hd);
+    memcpy(lay.src_off_in(hd), src_off, sizeof(int64_t) * n);
+    memcpy(lay.src_len_in(hd), src_len, sizeof(int32_t) * n);
     int64_t slots_total = 0;
     for (int i = 0; i < n; i++) {
-        int cap = block_cap ? block_cap[i] : bound_of(src_len[i]);
-        if (cap < 0) cap = 0;
-        h_cap[i] = cap + header;
+        h_cap[i] = block_cap ? std::max(block_cap[i], 0) + header : (int)compress_cap(src_len[i], header);
         h_slot_off[i] = slots_total;
-        slots_total += align16((int64_t)cap + header + 16);
+        slots_total += compress_slot(h_cap[i]);
     }
-    if (stream_first) memcpy(hd + o_first, stream_first, sizeof(int32_t) * (ns + 1));
-    if (streams) { void** hs = reinterpret_cast<void**>(hd + o_states); for (int s = 0; s < ns; s++) hs[s] = streams[s]->d_state; }
+    if (stream_first) memcpy(lay.first_in(hd), stream_first, sizeof(int32_t) * (ns + 1));
+    if (streams) for (int s = 0; s < ns; s++) lay.states_in(hd)[s] = streams[s]->d_state;
 
     if ((rc = c->d_src.ensure((size_t)src_bytes + 64))) return rc;
     if ((rc = c->d_slots.ensure((size_t)slots_total + 64))) return rc;
     if ((rc = c->d_out.ensure((size_t)slots_total + 64))) return rc;
-
     const uint8_t* hsrc = static_cast<const uint8_t*>(src);
     uint8_t* d_src = static_cast<uint8_t*>(c->d_src.p);
     uint8_t* d_slots = static_cast<uint8_t*>(c->d_slots.p);
     uint8_t* d_out = static_cast<uint8_t*>(c->d_out.p);
-    int64_t* d_out_off = reinterpret_cast<int64_t*>(dd + o_out_off);
-    int32_t* d_out_len = reinterpret_cast<int32_t*>(dd + o_out_len);
 
     cudaStream_t st = c->stream;
-    CU(cudaEventRecord(c->ev[0], st));
-    CU(cudaMemcpyAsync(dd, hd, o_upload_end, cudaMemcpyHostToDevice, st));
-    for (int k = 0; k < nchunks; k++) {
-        const Chunk& ch = chunks[k];
-        if (ch.hi > ch.lo) CU(cudaMemcpyAsync(d_src + ch.lo, hsrc + ch.lo, (size_t)(ch.hi - ch.lo), cudaMemcpyHostToDevice, st));
-        CU(cudaEventRecord(c->ev_h2d[k], st));
-        cudaStream_t ks = c->kstream[k % kKernelStreams];
-        CU(cudaStreamWaitEvent(ks, c->ev_h2d[k], 0));
-        if (k == 0) CU(cudaEventRecord(c->ev_k0, ks));
-        CompressArgs a{};
-        a.src = d_src;
-        a.src_off = reinterpret_cast<const int64_t*>(dd + o_src_off);
-        a.src_len = reinterpret_cast<const int32_t*>(dd + o_src_len);
-        a.n_blocks = n;
-        a.first_block = ch.b0;
-        a.stream_first = stream_first ? reinterpret_cast<const int32_t*>(dd + o_first) + ch.s0 : nullptr;
-        a.n_streams = ch.s1 - ch.s0;
-        a.states = streams ? reinterpret_cast<void* const*>(dd + o_states) + ch.s0 : nullptr;
-        a.dst = d_slots;
-        a.dst_off = reinterpret_cast<const int64_t*>(dd + o_slot_off);
-        a.dst_cap = block_cap ? reinterpret_cast<const int32_t*>(dd + o_cap) : nullptr;
-        a.out_len = d_out_len;
-        a.accel = accel; a.header = header; a.scratch = c->scratch + k;
-        CU(launch_compress(a, ks));
-        const int nk = ch.b1 - ch.b0;
-        // the scan kernel mirrors sizes and offsets into the pinned descriptor block (device-visible host memory)
-        CompactArgs g{d_slots, a.dst_off + ch.b0, d_out_len + ch.b0, nk, header, d_out + h_slot_off[ch.b0], d_out_off + ch.b0 + k,
-                      reinterpret_cast<int64_t*>(hd + o_out_off) + ch.b0 + k, reinterpret_cast<int32_t*>(hd + o_out_len) + ch.b0};
-        CU(launch_compact(g, ks));
-        c->launches += kernel_launches_per_compress() + kernel_launches_per_compact();
-        if (k == nchunks - 1) CU(cudaEventRecord(c->ev[2], ks));
-        CU(cudaEventRecord(c->ev_k[k], ks));
-    }
-    CU(cudaEventRecord(c->ev[1], st));
-
-    // drain: as each chunk's sizes arrive, send its compacted bytes home
-    const int32_t* h_out_len = reinterpret_cast<const int32_t*>(hd + o_out_len);
-    const int64_t* h_out_off = reinterpret_cast<const int64_t*>(hd + o_out_off);
-    int64_t base = 0;
-    int result = 0;
-    CU(cudaEventRecord(c->ev_d0, c->dstream));
-    for (int k = 0; k < nchunks; k++) {
-        const Chunk& ch = chunks[k];
-        CU(cudaEventSynchronize(c->ev_k[k]));
-        const int nk = ch.b1 - ch.b0;
-        const int64_t* off_k = h_out_off + ch.b0 + k;
-        const int64_t total_k = off_k[nk];
-        for (int i = 0; i < nk; i++) dst_off[ch.b0 + i] = base + off_k[i];
-        if (base + total_k > dst_cap) { result = fail(B200LZ4_E_NOMEM, "dst_cap too small"); break; }
-        if (total_k) CU(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + base, d_out + h_slot_off[ch.b0], (size_t)total_k,
-                                        cudaMemcpyDeviceToHost, c->dstream));
-        base += total_k;
-    }
-    dst_off[n] = base;
-    CU(cudaEventRecord(c->ev_d1, c->dstream));
-    if ((rc = sync_all(c))) return rc;
-    if (result) return result;
-    memcpy(out_len, h_out_len, sizeof(int32_t) * n);
-    cudaEventElapsedTime(&c->t_h2d, c->ev[0], c->ev[1]);
-    cudaEventElapsedTime(&c->t_kernel, c->ev_k0, c->ev[2]);
-    cudaEventElapsedTime(&c->t_d2h, c->ev_d0, c->ev_d1);
-    if (getenv("B200LZ4_DEBUG")) {          // device timeline of the pipeline, ms since the call's first event
-        float t = 0;
+    auto enqueue = [&]() -> int {
+        CU(cudaEventRecord(c->ev.start, st));
+        CU(cudaMemcpyAsync(dd, hd, lay.upload, cudaMemcpyHostToDevice, st));
         for (int k = 0; k < nchunks; k++) {
-            float a = 0, b = 0;
-            cudaEventElapsedTime(&a, c->ev[0], c->ev_h2d[k]); cudaEventElapsedTime(&b, c->ev[0], c->ev_k[k]);
-            fprintf(stderr, "[b200lz4] chunk %d: blocks %d..%d  h2d done %.2f  kernels done %.2f\n", k, chunks[k].b0, chunks[k].b1, a, b);
+            cudaStream_t ks = c->kstream[k % kKernelStreams];
+            if ((rc = start_range(c, k, ks, byte_span(src_off, src_len, chunks[k].b0, chunks[k].b1), d_src, hsrc))) return rc;
+            CompressArgs a = launch_args<CompressArgs>(lay, dd, d_src, d_slots, n, header, chunks[k], c->scratch + k,
+                                                       stream_first != nullptr, streams != nullptr);
+            a.dst_cap = block_cap ? lay.cap_in(dd) : nullptr;
+            a.accel = accel;
+            if ((rc = compress_range(c, a, lay, chunks[k], k, d_out, ks))) return rc;
         }
-        cudaEventElapsedTime(&t, c->ev[0], c->ev_d1);
-        fprintf(stderr, "[b200lz4] d2h done %.2f\n", t);
-    }
-    if (streams) for (int s = 0; s < n_streams; s++)
+        CU(cudaEventRecord(c->ev.h2d_end, st));
+        CU(cudaEventRecord(c->ev.d0, c->dstream));
+        return drain_compacted(c, chunks, nchunks, lay, d_out, dst, dst_cap, dst_off, n, false);
+    };
+    rc = finish_call(c, enqueue(), chunks, nchunks, "chunk", "h2d done", lay.out_len_in(hd), out_len, n, false);
+    if (streams && (rc == 0 || rc == B200LZ4_E_BLOCK)) for (int s = 0; s < n_streams; s++)
         if (stream_first[s + 1] > stream_first[s]) streams[s]->last_len = (uint32_t)src_len[stream_first[s + 1] - 1];
-    for (int i = 0; i < n; i++) if (out_len[i] <= 0) return fail(B200LZ4_E_BLOCK, "block " + std::to_string(i) + " failed to compress");
-    return 0;
+    return rc;
 }
-
-inline int32_t le32(const uint8_t* p)
-{ return (int32_t)((uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24)); }
 
 int decompress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_off, const int32_t* src_len, int n,
                              int L, int cap_last, void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len);
@@ -699,181 +548,110 @@ int decompress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                     int header, int max_block,
                     void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
-    if (!c) return fail(B200LZ4_E_ARG, "ctx is NULL");
-    if (n < 0 || (n > 0 && (!src_off || !src_len || !dst_off || !out_len))) return fail(B200LZ4_E_ARG, "NULL descriptor array");
-    if (header != 0 && header != 4 && header != 8) return fail(B200LZ4_E_ARG, "header_mode must be 0, 4 or 8");
-    if (header != 8 && max_block < 0) return fail(B200LZ4_E_ARG, "max_block");
-    if (streams && !stream_first) return fail(B200LZ4_E_ARG, "streams given without stream_first");
+    const Verdict v = check_batch(Entry::Ctx, true, c, n, header, max_block, src, src_bytes, src_off, src_len, dst, dst_off, out_len,
+                                  stream_first, n_streams, streams != nullptr);
+    if (v.code) return fail(v);
     if (n == 0) { if (dst_off) dst_off[0] = 0; return 0; }
-    if (!src || !dst) return fail(B200LZ4_E_ARG, "NULL data buffer");
     int rc;
-    if ((rc = check_blocks(src_off, src_len, n, src_bytes))) return rc;
-    if ((rc = check_streams(stream_first, n_streams, n))) return rc;
     CU(cudaSetDevice(c->device));
     const int ns = stream_first ? n_streams : n;
     if (streams) for (int s = 0; s < n_streams; s++)
         if (!streams[s] || streams[s]->ctx != c) return fail(B200LZ4_E_ARG, "stream handle belongs to another ctx");
     const uint8_t* hsrc = static_cast<const uint8_t*>(src);
-    // How the output goes home (B200LZ4_DECODE_OUT): "copy" = D2H copies behind each chunk's kernel; "pieces" = segment by
-    // segment while the blocks are being decoded (decompress_host_streamed; equally large independent blocks; the default
-    // where it applies); "mirror" = independent blocks with their sizes in the headers, page-locked destination: the copier
-    // warps store every output byte to the host buffer as well as to HBM (decompress.cu: kMirror) and no D2H copy follows.
-    // Measured on config 2 (1.07 GB out, 0.77 GB in): copy 27.7 ms, mirror 27.0 ms (the posted writes of 1 678 CTAs reach
-    // 40 GB/s and slow the H2D copy from 15 to 18.5 ms), pieces 26.4 ms -- so mirror stays opt-in.
-    const bool no_streamed = getenv("B200LZ4_NO_STREAMED") != nullptr;
+    // How the output goes home (B200LZ4_DECODE_OUT, host_plan.h: decode_route).  Measured on config 2 (1.07 GB out,
+    // 0.77 GB in): copy 27.7 ms, mirror 27.0 ms (the posted writes of 1 678 CTAs reach 40 GB/s and slow the H2D copy from
+    // 15 to 18.5 ms), pieces 26.4 ms -- so mirror stays opt-in.
     const char* out_env = getenv("B200LZ4_DECODE_OUT");
-    uint8_t* mirror_dst = nullptr;
     const char* dwide_env = getenv("B200LZ4_DWIDE");            // (tests force the wide kernel with it: that one has no mirror)
-    if (out_env && out_env[0] == 'm' && header == 8 && !stream_first && !streams && !(dwide_env && dwide_env[0] == '1')) {
+    uint8_t* mirror_dst = nullptr;
+    if (out_env && out_env[0] == 'm') {
         cudaPointerAttributes pa{};
         if (cudaPointerGetAttributes(&pa, dst) == cudaSuccess && pa.type == cudaMemoryTypeHost && pa.devicePointer)
             mirror_dst = static_cast<uint8_t*>(pa.devicePointer);
         else cudaGetLastError();
     }
-    // equally large independent blocks with their size in the header: the output leaves segment by segment
-    if (!mirror_dst && !no_streamed && !(out_env && out_env[0] == 'c') && header == 8 && !stream_first && !streams && n >= 96 && src_len[0] >= 8) {
-        const int L = le32(hsrc + src_off[0] + 4);
-        bool ok = L >= 65536 && (int64_t)L * n >= (int64_t(96) << 20);
-        int cap_last = 0;
-        for (int i = 0; i < n && ok; i++) {
-            const int cap = src_len[i] >= 8 ? le32(hsrc + src_off[i] + 4) : -1;
-            if (i < n - 1) ok = (cap == L); else { ok = (cap > 0 && cap <= L); cap_last = cap; }
-        }
-        if (ok) return decompress_host_streamed(c, src, src_off, src_len, n, L, cap_last, dst, dst_cap, dst_off, out_len);
-    }
-    Chunk chunks[kMaxChunks];
-    const int nchunks = plan_chunks(src_off, src_len, n, stream_first, ns, chunks, mirror_dst != nullptr);
+    const DecodeRoute route = decode_route(hsrc, src_off, src_len, n, header, stream_first != nullptr, out_env ? out_env[0] : 0,
+                                           getenv("B200LZ4_NO_STREAMED") != nullptr, dwide_env && dwide_env[0] == '1',
+                                           mirror_dst != nullptr);
+    if (route.out == DecodeOut::Pieces)
+        return decompress_host_streamed(c, src, src_off, src_len, n, route.L, route.cap_last, dst, dst_cap, dst_off, out_len);
+    if (route.out != DecodeOut::Mirror) mirror_dst = nullptr;
+    Range chunks[kMaxChunks];
+    const int nchunks = plan_chunks(src_len, n, stream_first, ns, mirror_dst != nullptr, chunks);
 
-    Carver cv;
-    const size_t o_src_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_slot_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_src_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_cap = cv.take(sizeof(int32_t) * n);
-    const size_t o_first = cv.take(sizeof(int32_t) * (ns + 1));
-    const size_t o_states = cv.take(sizeof(void*) * ns);
-    const size_t o_upload_end = cv.off;
-    const size_t o_out_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_out_off = cv.take(sizeof(int64_t) * (n + nchunks));
-    const size_t desc_bytes = cv.off;
-    if ((rc = c->h_desc.ensure(desc_bytes))) return rc;
-    if ((rc = c->d_desc.ensure(desc_bytes))) return rc;
-    uint8_t* hd = static_cast<uint8_t*>(c->h_desc.p);
-    uint8_t* dd = static_cast<uint8_t*>(c->d_desc.p);
-    int64_t* h_slot_off = reinterpret_cast<int64_t*>(hd + o_slot_off);
-    int32_t* h_cap = reinterpret_cast<int32_t*>(hd + o_cap);
-    memcpy(hd + o_src_off, src_off, sizeof(int64_t) * n);
-    memcpy(hd + o_src_len, src_len, sizeof(int32_t) * n);
-    // capacities: the header's uncompLen (BlockHasSize) or the configured maximum (LZ4.hs:189-198)
+    const DescLayout lay(n, n, n, ns + 1, ns, n + nchunks, 0);
+    if ((rc = ensure_desc(c, lay))) return rc;
+    void* hd = c->h_desc.p;
+    void* dd = c->d_desc.p;
+    int64_t* h_slot_off = lay.slot_off_in(hd);
+    int32_t* h_cap = lay.cap_in(hd);
+    memcpy(lay.src_off_in(hd), src_off, sizeof(int64_t) * n);
+    memcpy(lay.src_len_in(hd), src_len, sizeof(int32_t) * n);
     int64_t slots_total = 0;
     for (int i = 0; i < n; i++) {
-        int cap = max_block;
-        if (header == 8) cap = src_len[i] >= 8 ? le32(hsrc + src_off[i] + 4) : 0;
-        if (cap < 0) cap = 0;
-        h_cap[i] = cap;
+        h_cap[i] = decode_cap(hsrc, src_off, src_len, i, header, max_block);
         h_slot_off[i] = slots_total;
-        slots_total += (header == 8) ? (int64_t)cap : align16((int64_t)cap);
+        slots_total += decode_slot(h_cap[i], header);
     }
     const bool contiguous = (header == 8);     // slots are already exactly the output layout
     if (contiguous && slots_total > dst_cap) return fail(B200LZ4_E_NOMEM, "dst_cap too small: need " + std::to_string(slots_total));
-    if (stream_first) memcpy(hd + o_first, stream_first, sizeof(int32_t) * (ns + 1));
-    if (streams) { void** hs = reinterpret_cast<void**>(hd + o_states); for (int s = 0; s < ns; s++) hs[s] = streams[s]->d_state; }
+    if (stream_first) memcpy(lay.first_in(hd), stream_first, sizeof(int32_t) * (ns + 1));
+    if (streams) for (int s = 0; s < ns; s++) lay.states_in(hd)[s] = streams[s]->d_state;
 
     if ((rc = c->d_src.ensure((size_t)src_bytes + 64))) return rc;
     if ((rc = c->d_slots.ensure((size_t)slots_total + 64 + 16))) return rc;
     if (!contiguous && (rc = c->d_out.ensure((size_t)slots_total + 64))) return rc;
     // descriptor rings for chunks the wide kernel may take (few streams): one slice of one CTA-arena per stream, per chunk
     int wide_first[kMaxChunks + 1] = {0};
-    for (int k = 0; k < nchunks; k++) {
-        const int nsk = chunks[k].s1 - chunks[k].s0;
-        wide_first[k + 1] = wide_first[k] + (nsk < kWideMaxCtas ? nsk : kWideMaxCtas);
-    }
+    for (int k = 0; k < nchunks; k++) wide_first[k + 1] = wide_first[k] + std::min(chunks[k].u1 - chunks[k].u0, kWideMaxCtas);
     if ((rc = c->d_wide.ensure((size_t)wide_first[nchunks] * kWideArenaPerCta))) return rc;
     uint8_t* d_src = static_cast<uint8_t*>(c->d_src.p);
     uint8_t* d_slots = static_cast<uint8_t*>(c->d_slots.p);
     if (mirror_dst) d_slots += reinterpret_cast<uintptr_t>(mirror_dst) & 15;      // same address modulo 16 on both sides: 128-bit stores line up
     uint8_t* d_out = static_cast<uint8_t*>(c->d_out.p);
-    int64_t* d_out_off = reinterpret_cast<int64_t*>(dd + o_out_off);
-    int32_t* d_out_len = reinterpret_cast<int32_t*>(dd + o_out_len);
 
     cudaStream_t st = c->stream;
-    CU(cudaEventRecord(c->ev[0], st));
-    CU(cudaMemcpyAsync(dd, hd, o_upload_end, cudaMemcpyHostToDevice, st));
-    CU(cudaEventRecord(c->ev_d0, c->dstream));
-    for (int k = 0; k < nchunks; k++) {
-        const Chunk& ch = chunks[k];
-        if (ch.hi > ch.lo) CU(cudaMemcpyAsync(d_src + ch.lo, hsrc + ch.lo, (size_t)(ch.hi - ch.lo), cudaMemcpyHostToDevice, st));
-        CU(cudaEventRecord(c->ev_h2d[k], st));
-        cudaStream_t ks = c->kstream[k % kKernelStreams];
-        CU(cudaStreamWaitEvent(ks, c->ev_h2d[k], 0));
-        if (k == 0) CU(cudaEventRecord(c->ev_k0, ks));
-        DecompressArgs a{};
-        a.src = d_src;
-        a.src_off = reinterpret_cast<const int64_t*>(dd + o_src_off);
-        a.src_len = reinterpret_cast<const int32_t*>(dd + o_src_len);
-        a.n_blocks = n;
-        a.first_block = ch.b0;
-        a.stream_first = stream_first ? reinterpret_cast<const int32_t*>(dd + o_first) + ch.s0 : nullptr;
-        a.n_streams = ch.s1 - ch.s0;
-        a.states = streams ? reinterpret_cast<void* const*>(dd + o_states) + ch.s0 : nullptr;
-        a.dst = d_slots;
-        a.dst_off = reinterpret_cast<const int64_t*>(dd + o_slot_off);
-        a.dst_cap = reinterpret_cast<const int32_t*>(dd + o_cap);
-        a.out_len = d_out_len;
-        a.header = header; a.max_block = max_block; a.scratch = c->scratch + k;
-        a.wide_arena = reinterpret_cast<uint4*>(static_cast<uint8_t*>(c->d_wide.p) + (size_t)wide_first[k] * kWideArenaPerCta);
-        a.wide_ctas = wide_first[k + 1] - wide_first[k];
-        a.host_dst = mirror_dst;
-        CU(launch_decompress(a, ks));
-        c->launches += kernel_launches_per_decompress();
-        const int nk = ch.b1 - ch.b0;
-        if (!contiguous) {
-            CompactArgs g{d_slots, a.dst_off + ch.b0, d_out_len + ch.b0, nk, 0, d_out + h_slot_off[ch.b0], d_out_off + ch.b0 + k, nullptr, nullptr};
-            CU(launch_compact(g, ks));
-            c->launches += kernel_launches_per_compact();
-            CU(cudaMemcpyAsync(hd + o_out_off + sizeof(int64_t) * (ch.b0 + k), dd + o_out_off + sizeof(int64_t) * (ch.b0 + k),
-                               sizeof(int64_t) * (nk + 1), cudaMemcpyDeviceToHost, ks));
-        }
-        CU(cudaMemcpyAsync(hd + o_out_len + sizeof(int32_t) * ch.b0, dd + o_out_len + sizeof(int32_t) * ch.b0,
-                           sizeof(int32_t) * nk, cudaMemcpyDeviceToHost, ks));
-        if (k == nchunks - 1) CU(cudaEventRecord(c->ev[2], ks));
-        CU(cudaEventRecord(c->ev_k[k], ks));
-        if (contiguous && !mirror_dst) {   // sizes are known from the headers: the D2H copy can be queued right away
-            const int64_t lo = h_slot_off[ch.b0];
-            const int64_t hi = (ch.b1 < n) ? h_slot_off[ch.b1] : slots_total;
-            CU(cudaStreamWaitEvent(c->dstream, c->ev_k[k], 0));
-            if (hi > lo) CU(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + lo, d_slots + lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, c->dstream));
-        }
-    }
-    CU(cudaEventRecord(c->ev[1], st));
-    int result = 0;
-    if (contiguous) {
-        memcpy(dst_off, h_slot_off, sizeof(int64_t) * n); dst_off[n] = slots_total;
-    } else {
-        const int64_t* h_out_off = reinterpret_cast<const int64_t*>(hd + o_out_off);
-        int64_t base = 0;
+    auto enqueue = [&]() -> int {
+        CU(cudaEventRecord(c->ev.start, st));
+        CU(cudaMemcpyAsync(dd, hd, lay.upload, cudaMemcpyHostToDevice, st));
+        CU(cudaEventRecord(c->ev.d0, c->dstream));
         for (int k = 0; k < nchunks; k++) {
-            const Chunk& ch = chunks[k];
-            CU(cudaEventSynchronize(c->ev_k[k]));
+            const Range& ch = chunks[k];
+            cudaStream_t ks = c->kstream[k % kKernelStreams];
+            if ((rc = start_range(c, k, ks, byte_span(src_off, src_len, ch.b0, ch.b1), d_src, hsrc))) return rc;
+            DecompressArgs a = launch_args<DecompressArgs>(lay, dd, d_src, d_slots, n, header, ch, c->scratch + k,
+                                                           stream_first != nullptr, streams != nullptr);
+            a.dst_cap = lay.cap_in(dd);
+            a.max_block = max_block;
+            a.wide_arena = reinterpret_cast<uint4*>(static_cast<uint8_t*>(c->d_wide.p) + (size_t)wide_first[k] * kWideArenaPerCta);
+            a.wide_ctas = wide_first[k + 1] - wide_first[k];
+            a.host_dst = mirror_dst;
+            CU(launch_decompress(a, ks));
+            c->launches += kernel_launches_per_decompress();
             const int nk = ch.b1 - ch.b0;
-            const int64_t* off_k = h_out_off + ch.b0 + k;
-            const int64_t total_k = off_k[nk];
-            for (int i = 0; i < nk; i++) dst_off[ch.b0 + i] = base + off_k[i];
-            if (base + total_k > dst_cap) { result = fail(B200LZ4_E_NOMEM, "dst_cap too small"); break; }
-            if (total_k) CU(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + base, d_out + h_slot_off[ch.b0], (size_t)total_k,
-                                            cudaMemcpyDeviceToHost, c->dstream));
-            base += total_k;
+            if (!contiguous) {
+                CompactArgs g{d_slots, a.dst_off + ch.b0, a.out_len + ch.b0, nk, 0, d_out + h_slot_off[ch.b0],
+                              lay.out_off_in(dd) + ch.b0 + k, nullptr, nullptr};
+                CU(launch_compact(g, ks));
+                c->launches += kernel_launches_per_compact();
+                CU(cudaMemcpyAsync(lay.out_off_in(hd) + ch.b0 + k, lay.out_off_in(dd) + ch.b0 + k, sizeof(int64_t) * (nk + 1), cudaMemcpyDeviceToHost, ks));
+            }
+            CU(cudaMemcpyAsync(lay.out_len_in(hd) + ch.b0, lay.out_len_in(dd) + ch.b0, sizeof(int32_t) * nk, cudaMemcpyDeviceToHost, ks));
+            CU(cudaEventRecord(c->ev.k[k], ks));
+            if (contiguous && !mirror_dst) {   // sizes are known from the headers: the D2H copy can be queued right away
+                const int64_t lo = h_slot_off[ch.b0];
+                const int64_t hi = (ch.b1 < n) ? h_slot_off[ch.b1] : slots_total;
+                CU(cudaStreamWaitEvent(c->dstream, c->ev.k[k], 0));
+                if (hi > lo) CU(cudaMemcpyAsync(static_cast<uint8_t*>(dst) + lo, d_slots + lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, c->dstream));
+            }
         }
-        dst_off[n] = base;
-    }
-    CU(cudaEventRecord(c->ev_d1, c->dstream));
-    if ((rc = sync_all(c))) return rc;
-    if (result) return result;
-    cudaEventElapsedTime(&c->t_h2d, c->ev[0], c->ev[1]);
-    cudaEventElapsedTime(&c->t_kernel, c->ev_k0, c->ev[2]);
-    cudaEventElapsedTime(&c->t_d2h, c->ev_d0, c->ev_d1);
-    memcpy(out_len, hd + o_out_len, sizeof(int32_t) * n);
-    for (int i = 0; i < n; i++) if (out_len[i] < 0) return fail(B200LZ4_E_BLOCK, "block " + std::to_string(i) + " failed to decompress");
-    return 0;
+        CU(cudaEventRecord(c->ev.h2d_end, st));
+        if (!contiguous) return drain_compacted(c, chunks, nchunks, lay, d_out, dst, dst_cap, dst_off, n, false);
+        memcpy(dst_off, h_slot_off, sizeof(int64_t) * n);
+        dst_off[n] = slots_total;
+        return 0;
+    };
+    return finish_call(c, enqueue(), chunks, nchunks, nullptr, nullptr, lay.out_len_in(hd), out_len, n, true);
 }
 
 // ---- streamed decompress call --------------------------------------------------
@@ -890,39 +668,21 @@ int decompress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src
     const int header = 8;
     const int64_t out_total = (int64_t)L * (n - 1) + cap_last;
     if (out_total > dst_cap) return fail(B200LZ4_E_NOMEM, "dst_cap too small: need " + std::to_string(out_total));
-    const char* env_g = getenv("B200LZ4_STREAM_G");
-    const char* env_s = getenv("B200LZ4_STREAM_S");
-    int G = env_g ? atoi(env_g) : 12;
-    if (G < 1) G = 1;
-    if (G > kMaxGroups) G = kMaxGroups;
-    int S = env_s ? atoi(env_s) : 8;
-    if (S < 1) S = 1;
-    if (S > kMaxSegs) S = kMaxSegs;
-    const int seg = (int)((((int64_t)L + S - 1) / S + 127) / 128 * 128);
-    S = (L + seg - 1) / seg;
-    const int per_group = (n + G - 1) / G;
-    G = (n + per_group - 1) / per_group;
+    const Geometry geo = decompress_geometry(n, L, getenv("B200LZ4_STREAM_G"), getenv("B200LZ4_STREAM_S"));
+    Range groups[kMaxGroups];
+    plan_groups(geo, n, groups);
     if ((rc = probe_stream_aliasing(c))) return rc;     // nothing can deadlock here, but kernels queued behind another group's would start late
     const int nks = c->n_kgood >= 2 ? c->n_kgood : kKernelStreams;
 
-    Carver cv;
-    const size_t o_src_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_slot_off = cv.take(sizeof(int64_t) * n);
-    const size_t o_src_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_cap = cv.take(sizeof(int32_t) * n);
-    const size_t o_upload_end = cv.off;
-    const size_t o_out_len = cv.take(sizeof(int32_t) * n);
-    const size_t o_ready = cv.take(sizeof(uint32_t) * kMaxGroups * kMaxSegs);
-    const size_t desc_bytes = cv.off;
-    if ((rc = c->h_desc.ensure(desc_bytes))) return rc;
-    if ((rc = c->d_desc.ensure(desc_bytes))) return rc;
-    uint8_t* hd = static_cast<uint8_t*>(c->h_desc.p);
-    uint8_t* dd = static_cast<uint8_t*>(c->d_desc.p);
-    int64_t* h_slot_off = reinterpret_cast<int64_t*>(hd + o_slot_off);
-    int32_t* h_cap = reinterpret_cast<int32_t*>(hd + o_cap);
-    volatile uint32_t* ready = reinterpret_cast<volatile uint32_t*>(hd + o_ready);
-    memcpy(hd + o_src_off, src_off, sizeof(int64_t) * n);
-    memcpy(hd + o_src_len, src_len, sizeof(int32_t) * n);
+    const DescLayout lay(n, n, n, 0, 0, 0, kMaxGroups * kMaxSegs);
+    if ((rc = ensure_desc(c, lay))) return rc;
+    void* hd = c->h_desc.p;
+    void* dd = c->d_desc.p;
+    int64_t* h_slot_off = lay.slot_off_in(hd);
+    int32_t* h_cap = lay.cap_in(hd);
+    volatile uint32_t* ready = lay.ready_in(hd);
+    memcpy(lay.src_off_in(hd), src_off, sizeof(int64_t) * n);
+    memcpy(lay.src_len_in(hd), src_len, sizeof(int32_t) * n);
     int64_t src_hi = 0;
     for (int i = 0; i < n; i++) {
         h_cap[i] = i < n - 1 ? L : cap_last;
@@ -938,118 +698,79 @@ int decompress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src
     uint8_t* d_src = static_cast<uint8_t*>(c->d_src.p);
     uint8_t* d_slots = static_cast<uint8_t*>(c->d_slots.p);
     uint32_t* d_counts = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(c->d_flags) + 1024);
-
-    cudaStream_t st = c->stream;
-    CU(cudaEventRecord(c->ev[0], st));
-    CU(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * kMaxGroups * kMaxSegs, st));
-    CU(cudaMemcpyAsync(dd, hd, o_upload_end, cudaMemcpyHostToDevice, st));
-    CU(cudaEventRecord(c->ev_d0, c->dstream));
-    for (int g = 0; g < G; g++) {
-        const int b0 = g * per_group, b1 = std::min(n, b0 + per_group);
-        int64_t lo = INT64_MAX, hi = 0;
-        for (int i = b0; i < b1; i++) { lo = std::min(lo, src_off[i]); hi = std::max(hi, src_off[i] + (int64_t)src_len[i]); }
-        if (hi > lo) CU(cudaMemcpyAsync(d_src + lo, hsrc + lo, (size_t)(hi - lo), cudaMemcpyHostToDevice, st));
-        CU(cudaEventRecord(c->ev_h2d[g], st));
-        cudaStream_t ks = c->kstream[g % nks];
-        CU(cudaStreamWaitEvent(ks, c->ev_h2d[g], 0));
-        if (g == 0) CU(cudaEventRecord(c->ev_k0, ks));
-        DecompressArgs a{};
-        a.src = d_src;
-        a.src_off = reinterpret_cast<const int64_t*>(dd + o_src_off);
-        a.src_len = reinterpret_cast<const int32_t*>(dd + o_src_len);
-        a.n_blocks = n;
-        a.first_block = b0;
-        a.n_streams = b1 - b0;
-        a.dst = d_slots;
-        a.dst_off = reinterpret_cast<const int64_t*>(dd + o_slot_off);
-        a.dst_cap = reinterpret_cast<const int32_t*>(dd + o_cap);
-        a.out_len = reinterpret_cast<int32_t*>(hd + o_out_len);     // page-locked, device-visible: no small D2H copies that would queue behind the pieces
-        a.header = header; a.max_block = 0; a.scratch = c->scratch + g;
-        a.seg_count = d_counts + g * kMaxSegs;
-        a.host_ready = reinterpret_cast<uint32_t*>(hd + o_ready) + g * kMaxSegs;
-        a.seg_bytes = seg; a.n_segs = S;
-        CU(launch_decompress(a, ks));
-        c->launches += kernel_launches_per_decompress();
-        CU(cudaEventRecord(c->ev_k[g], ks));
-    }
-    CU(cudaEventRecord(c->ev[1], st));
-
-    // drain: queue every (group, segment) piece as soon as its flag is up
-    int next_s[kMaxGroups] = {0};
-    int remaining = G * S;
-    uint8_t* hdst = static_cast<uint8_t*>(dst);
     const bool dbg = getenv("B200LZ4_DEBUG") != nullptr;
+    if (dbg) fprintf(stderr, "[b200lz4] streamed decompress: G %d S %d seg %d\n", geo.G, geo.S, geo.seg);
     struct PieceLog { int g, s; double issued_ms; cudaEvent_t done; };
     std::vector<PieceLog> plog;
-    const auto t_host0 = std::chrono::steady_clock::now();
-    auto send = [&](int g, int sgm) -> int {
-        const int b0 = g * per_group, b1 = std::min(n, b0 + per_group);
-        const int lo = sgm * seg, width = std::min(seg, L - lo);
-        int rows = b1 - b0;
-        if (b1 == n && cap_last < L) {
-            rows--;
-            const int wl = std::min(width, cap_last - lo);
-            if (wl > 0) CU(cudaMemcpyAsync(hdst + (int64_t)L * (n - 1) + lo, d_slots + (int64_t)L * (n - 1) + lo, (size_t)wl, cudaMemcpyDeviceToHost, c->dstream));
+
+    cudaStream_t st = c->stream;
+    auto enqueue = [&]() -> int {
+        CU(cudaEventRecord(c->ev.start, st));
+        CU(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * kMaxGroups * kMaxSegs, st));
+        CU(cudaMemcpyAsync(dd, hd, lay.upload, cudaMemcpyHostToDevice, st));
+        CU(cudaEventRecord(c->ev.d0, c->dstream));
+        for (int g = 0; g < geo.G; g++) {
+            cudaStream_t ks = c->kstream[g % nks];
+            if ((rc = start_range(c, g, ks, byte_span(src_off, src_len, groups[g].b0, groups[g].b1), d_src, hsrc))) return rc;
+            DecompressArgs a = launch_args<DecompressArgs>(lay, dd, d_src, d_slots, n, header, groups[g], c->scratch + g, false, false);
+            a.dst_cap = lay.cap_in(dd);
+            a.out_len = lay.out_len_in(hd);     // page-locked, device-visible: no small D2H copies that would queue behind the pieces
+            a.max_block = 0;
+            a.seg_count = d_counts + g * kMaxSegs;
+            a.host_ready = lay.ready_in(hd) + g * kMaxSegs;
+            a.seg_bytes = geo.seg; a.n_segs = geo.S;
+            CU(launch_decompress(a, ks));
+            c->launches += kernel_launches_per_decompress();
+            CU(cudaEventRecord(c->ev.k[g], ks));
         }
-        if (rows > 0) return copy_rows(hdst + (int64_t)L * b0 + lo, (size_t)L, d_slots + (int64_t)L * b0 + lo, (size_t)L, (size_t)width, (size_t)rows,
-                                       cudaMemcpyDeviceToHost, c->dstream);
+        CU(cudaEventRecord(c->ev.h2d_end, st));
+
+        // drain: queue every (group, segment) piece as soon as its flag is up
+        int next_s[kMaxGroups] = {0};
+        int remaining = geo.G * geo.S;
+        const auto t_host0 = std::chrono::steady_clock::now();
+        long spins = 0;
+        while (remaining) {
+            bool any = false;
+            for (int g = 0; g < geo.G; g++) {
+                while (next_s[g] < geo.S && ready[g * kMaxSegs + next_s[g]]) {
+                    if ((rc = copy_piece(static_cast<uint8_t*>(dst), (size_t)L, d_slots, (size_t)L, geo, groups[g], n, L, cap_last, next_s[g],
+                                         cudaMemcpyDeviceToHost, c->dstream))) return rc;
+                    if (dbg) {
+                        PieceLog pl{g, next_s[g], std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count(), nullptr};
+                        cudaEventCreate(&pl.done); cudaEventRecord(pl.done, c->dstream);
+                        plog.push_back(pl);
+                    }
+                    next_s[g]++; remaining--; any = true;
+                }
+            }
+            if (any) { spins = 0; continue; }
+#if defined(__x86_64__)
+            __builtin_ia32_pause();
+#endif
+            if (++spins % 4096 == 0) {          // a faulted or finished kernel must not leave this loop spinning
+                bool all_done = true;
+                for (int g = 0; g < geo.G; g++) {
+                    const cudaError_t q = cudaEventQuery(c->ev.k[g]);
+                    if (q == cudaErrorNotReady) { all_done = false; break; }
+                    if (q != cudaSuccess) return fail_cuda(q, "streamed decompress");
+                }
+                if (all_done) {                 // every block has ended, so every flag is up: one last look
+                    bool missing = false;
+                    for (int g = 0; g < geo.G; g++) for (int k = next_s[g]; k < geo.S; k++) if (!ready[g * kMaxSegs + k]) missing = true;
+                    if (missing) return fail(B200LZ4_E_CUDA, "streamed decompress: kernels ended without raising every segment flag");
+                }
+            }
+        }
         return 0;
     };
-    long spins = 0;
-    while (remaining) {
-        bool any = false;
-        for (int g = 0; g < G; g++) {
-            while (next_s[g] < S && ready[g * kMaxSegs + next_s[g]]) {
-                if ((rc = send(g, next_s[g]))) return rc;
-                if (dbg) {
-                    PieceLog pl{g, next_s[g], std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count(), nullptr};
-                    cudaEventCreate(&pl.done); cudaEventRecord(pl.done, c->dstream);
-                    plog.push_back(pl);
-                }
-                next_s[g]++; remaining--; any = true;
-            }
-        }
-        if (any) { spins = 0; continue; }
-#if defined(__x86_64__)
-        __builtin_ia32_pause();
-#endif
-        if (++spins % 4096 == 0) {          // a faulted or finished kernel must not leave this loop spinning
-            bool all_done = true;
-            for (int g = 0; g < G; g++) {
-                const cudaError_t q = cudaEventQuery(c->ev_k[g]);
-                if (q == cudaErrorNotReady) { all_done = false; break; }
-                if (q != cudaSuccess) return fail_cuda(q, "streamed decompress");
-            }
-            if (all_done) {                 // every block has ended, so every flag is up: one last look
-                bool missing = false;
-                for (int g = 0; g < G; g++) for (int k = next_s[g]; k < S; k++) if (!ready[g * kMaxSegs + k]) missing = true;
-                if (missing) return fail(B200LZ4_E_CUDA, "streamed decompress: kernels ended without raising every segment flag");
-            }
-        }
+    rc = finish_call(c, enqueue(), groups, geo.G, "group", "input landed", lay.out_len_in(hd), out_len, n, true);
+    for (auto& pl : plog) {     // (host time counts from the moment the drain loop started)
+        float x = 0; cudaEventElapsedTime(&x, c->ev.start, pl.done);
+        fprintf(stderr, "[b200lz4] piece g%d s%d: queued at host +%.2f ms, copied by %.2f\n", pl.g, pl.s, pl.issued_ms, x);
+        cudaEventDestroy(pl.done);
     }
-    CU(cudaEventRecord(c->ev_d1, c->dstream));
-    if ((rc = sync_all(c))) return rc;
-    cudaEventElapsedTime(&c->t_h2d, c->ev[0], c->ev[1]);
-    cudaEventElapsedTime(&c->t_kernel, c->ev_k0, c->ev_k[G - 1]);
-    cudaEventElapsedTime(&c->t_d2h, c->ev_d0, c->ev_d1);
-    memcpy(out_len, hd + o_out_len, sizeof(int32_t) * n);
-    if (getenv("B200LZ4_DEBUG")) {
-        fprintf(stderr, "[b200lz4] streamed decompress: G %d S %d seg %d\n", G, S, seg);
-        float t = 0;
-        for (int g = 0; g < G; g++) {
-            float x = 0, y = 0;
-            cudaEventElapsedTime(&x, c->ev[0], c->ev_h2d[g]); cudaEventElapsedTime(&y, c->ev[0], c->ev_k[g]);
-            fprintf(stderr, "[b200lz4] group %d: input landed %.2f  kernel done %.2f\n", g, x, y);
-        }
-        cudaEventElapsedTime(&t, c->ev[0], c->ev_d1); fprintf(stderr, "[b200lz4] d2h done %.2f\n", t);
-        for (auto& pl : plog) {     // (host time counts from the moment the drain loop started)
-            float x = 0; cudaEventElapsedTime(&x, c->ev[0], pl.done);
-            fprintf(stderr, "[b200lz4] piece g%d s%d: queued at host +%.2f ms, copied by %.2f\n", pl.g, pl.s, pl.issued_ms, x);
-            cudaEventDestroy(pl.done);
-        }
-    }
-    for (int i = 0; i < n; i++) if (out_len[i] < 0) return fail(B200LZ4_E_BLOCK, "block " + std::to_string(i) + " failed to decompress");
-    return 0;
+    return rc;
 }
 
 }  // namespace
@@ -1099,14 +820,7 @@ int b200lz4_ctx_create(int device, b200lz4_ctx** out)
     if (e2 == cudaSuccess) e2 = cudaHostAlloc(reinterpret_cast<void**>(&c->h_const), 64 * sizeof(uint32_t), cudaHostAllocPortable);
     if (e2 == cudaSuccess) for (uint32_t i = 0; i < 64; i++) c->h_const[i] = i;
     if (e2 == cudaSuccess) e2 = cudaDeviceGetAttribute(&c->clock_khz, cudaDevAttrClockRate, device);
-    for (int i = 0; i < 4 && e2 == cudaSuccess; i++) e2 = cudaEventCreate(&c->ev[i]);
-    for (int i = 0; i < kMaxGroups && e2 == cudaSuccess; i++) {
-        e2 = cudaEventCreate(&c->ev_h2d[i]);
-        if (e2 == cudaSuccess) e2 = cudaEventCreate(&c->ev_k[i]);
-    }
-    if (e2 == cudaSuccess) e2 = cudaEventCreate(&c->ev_k0);
-    if (e2 == cudaSuccess) e2 = cudaEventCreate(&c->ev_d0);
-    if (e2 == cudaSuccess) e2 = cudaEventCreate(&c->ev_d1);
+    c->ev.each([&](cudaEvent_t& ev) { if (e2 == cudaSuccess) e2 = cudaEventCreate(&ev); });
     if (e2 != cudaSuccess) { b200lz4_ctx_destroy(c); return fail_cuda(e2, "ctx_create"); }
     *out = c;
     return 0;
@@ -1121,12 +835,7 @@ void b200lz4_ctx_destroy(b200lz4_ctx* c)
     if (c->scratch) cudaFree(c->scratch);
     if (c->d_flags) cudaFree(c->d_flags);
     if (c->h_const) cudaFreeHost(c->h_const);
-    for (auto& e : c->ev) if (e) cudaEventDestroy(e);
-    for (auto& e : c->ev_h2d) if (e) cudaEventDestroy(e);
-    for (auto& e : c->ev_k) if (e) cudaEventDestroy(e);
-    if (c->ev_k0) cudaEventDestroy(c->ev_k0);
-    if (c->ev_d0) cudaEventDestroy(c->ev_d0);
-    if (c->ev_d1) cudaEventDestroy(c->ev_d1);
+    c->ev.each([](cudaEvent_t& e) { if (e) cudaEventDestroy(e); });
     for (auto& k : c->kstream) if (k) cudaStreamDestroy(k);
     if (c->fstream) cudaStreamDestroy(c->fstream);
     for (auto& e : c->ev_piece) if (e) cudaEventDestroy(e);
@@ -1309,48 +1018,23 @@ struct b200lz4_mctx {
 
 namespace {
 
-struct Stripe { int u0, u1, b0, b1; };
-
-// contiguous unit ranges with about equal source bytes
-std::vector<Stripe> plan_stripes(const int32_t* len, int n, const int32_t* first, int ns, int parts)
-{
-    const int units = first ? ns : n;
-    int64_t total = 0;
-    for (int i = 0; i < n; i++) total += len[i];
-    std::vector<Stripe> out;
-    int u = 0; int64_t done = 0;
-    for (int k = 0; k < parts; k++) {
-        Stripe s; s.u0 = u; s.b0 = first ? first[u] : u;
-        const int64_t target = total * (k + 1) / parts;
-        while (u < units && (done < target || k == parts - 1)) {
-            const int a = first ? first[u] : u, b = first ? first[u + 1] : u + 1;
-            for (int i = a; i < b; i++) done += len[i];
-            u++;
-        }
-        s.u1 = u; s.b1 = first ? first[u] : u;
-        out.push_back(s);
-    }
-    return out;
-}
-
 template <class Call>
 int run_striped(b200lz4_mctx* m, const int64_t* src_off, const int32_t* src_len, int n,
                 const int32_t* stream_first, int n_streams, const std::vector<int64_t>& region, /* n + 1 prefix of worst-case output */
                 int64_t* dst_off, int32_t* out_len, Call call)
 {
     const int parts = (int)m->ctx.size();
-    const std::vector<Stripe> st = plan_stripes(src_len, n, stream_first, n_streams, parts);
+    const std::vector<Range> st = plan_stripes(src_len, n, stream_first, n_streams, parts);
     std::vector<int> rcs(parts, 0);
     std::vector<std::string> errs(parts);
     std::vector<std::thread> pool;
     for (int d = 0; d < parts; d++) {
-        const Stripe s = st[d];
+        const Range s = st[d];
         if (s.b1 <= s.b0) continue;
         pool.emplace_back([&, d, s]() {
             const int nb = s.b1 - s.b0;
-            int64_t lo = INT64_MAX, hi = 0;
-            for (int i = s.b0; i < s.b1; i++) { lo = std::min(lo, src_off[i]); hi = std::max(hi, src_off[i] + (int64_t)src_len[i]); }
-            if (lo > hi) lo = hi = 0;
+            const Span sp = byte_span(src_off, src_len, s.b0, s.b1);
+            const int64_t lo = sp.lo, hi = sp.hi;
             std::vector<int64_t> off(nb), doff(nb + 1);
             for (int i = 0; i < nb; i++) off[i] = src_off[s.b0 + i] - lo;
             std::vector<int32_t> first;
@@ -1414,15 +1098,12 @@ int b200lz4_compress_batch_multi(b200lz4_mctx* m, const void* src, int64_t src_b
                                  int acceleration, int header_mode,
                                  void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
-    if (!m || m->ctx.empty()) return fail(B200LZ4_E_ARG, "mctx is NULL");
-    if (n_blocks < 0 || (n_blocks > 0 && (!src_off || !src_len || !dst_off || !out_len || !src || !dst))) return fail(B200LZ4_E_ARG, "NULL argument");
-    if (header_mode != 0 && header_mode != 4 && header_mode != 8) return fail(B200LZ4_E_ARG, "header_mode must be 0, 4 or 8");
+    const Verdict v = check_batch(Entry::Multi, false, (m && !m->ctx.empty()) ? m : nullptr, n_blocks, header_mode, 0, src, src_bytes,
+                                  src_off, src_len, dst, dst_off, out_len, stream_first, n_streams, false);
+    if (v.code) return fail(v);
     if (n_blocks == 0) { if (dst_off) dst_off[0] = 0; return 0; }
-    int rc;
-    if ((rc = check_blocks(src_off, src_len, n_blocks, src_bytes))) return rc;
-    if ((rc = check_streams(stream_first, n_streams, n_blocks))) return rc;
     std::vector<int64_t> region(n_blocks + 1, 0);
-    for (int i = 0; i < n_blocks; i++) region[i + 1] = region[i] + header_mode + bound_of(src_len[i]);
+    for (int i = 0; i < n_blocks; i++) region[i + 1] = region[i] + compress_cap(src_len[i], header_mode);
     if (region[n_blocks] > dst_cap) return fail(B200LZ4_E_NOMEM, "dst_cap too small: need " + std::to_string(region[n_blocks]));
     const uint8_t* hs = static_cast<const uint8_t*>(src);
     uint8_t* hd = static_cast<uint8_t*>(dst);
@@ -1440,23 +1121,15 @@ int b200lz4_decompress_batch_multi(b200lz4_mctx* m, const void* src, int64_t src
                                    int header_mode, int max_block,
                                    void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
-    if (!m || m->ctx.empty()) return fail(B200LZ4_E_ARG, "mctx is NULL");
-    if (n_blocks < 0 || (n_blocks > 0 && (!src_off || !src_len || !dst_off || !out_len || !src || !dst))) return fail(B200LZ4_E_ARG, "NULL argument");
-    if (header_mode != 0 && header_mode != 4 && header_mode != 8) return fail(B200LZ4_E_ARG, "header_mode must be 0, 4 or 8");
-    if (header_mode != 8 && max_block < 0) return fail(B200LZ4_E_ARG, "max_block");
+    const Verdict v = check_batch(Entry::Multi, true, (m && !m->ctx.empty()) ? m : nullptr, n_blocks, header_mode, max_block, src,
+                                  src_bytes, src_off, src_len, dst, dst_off, out_len, stream_first, n_streams, false);
+    if (v.code) return fail(v);
     if (n_blocks == 0) { if (dst_off) dst_off[0] = 0; return 0; }
-    int rc;
-    if ((rc = check_blocks(src_off, src_len, n_blocks, src_bytes))) return rc;
-    if ((rc = check_streams(stream_first, n_streams, n_blocks))) return rc;
     const uint8_t* hs = static_cast<const uint8_t*>(src);
     uint8_t* hd = static_cast<uint8_t*>(dst);
     std::vector<int64_t> region(n_blocks + 1, 0);
-    for (int i = 0; i < n_blocks; i++) {
-        int cap = max_block;
-        if (header_mode == 8) cap = src_len[i] >= 8 ? le32(hs + src_off[i] + 4) : 0;
-        if (cap < 0) cap = 0;
-        region[i + 1] = region[i] + (header_mode == 8 ? (int64_t)cap : align16((int64_t)cap));
-    }
+    for (int i = 0; i < n_blocks; i++)
+        region[i + 1] = region[i] + decode_slot(decode_cap(hs, src_off, src_len, i, header_mode, max_block), header_mode);
     if (region[n_blocks] > dst_cap) return fail(B200LZ4_E_NOMEM, "dst_cap too small: need " + std::to_string(region[n_blocks]));
     return run_striped(m, src_off, src_len, n_blocks, stream_first, n_streams, region, dst_off, out_len,
         [&](b200lz4_ctx* c, int64_t lo, int64_t bytes, const int64_t* off, const int32_t* len, int nb, const int32_t* first, int ns,
@@ -1488,8 +1161,9 @@ int b200lz4_compress_dev(const void* d_src, const int64_t* d_src_off, const int3
                          void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
                          int acceleration, int header_mode, void* d_scratch, void* cuda_stream)
 {
-    if (n_blocks < 0 || !d_scratch) return fail(B200LZ4_E_ARG, "bad argument");
-    if (header_mode != 0 && header_mode != 4 && header_mode != 8) return fail(B200LZ4_E_ARG, "header_mode must be 0, 4 or 8");
+    const Verdict v = check_batch(Entry::Dev, false, d_scratch, n_blocks, header_mode, 0, d_src, 0, d_src_off, d_src_len, d_dst,
+                                  d_dst_off, d_out_len, d_stream_first, n_streams, false);
+    if (v.code) return fail(v);
     if (n_blocks == 0) return 0;
     CompressArgs a{};
     a.src = static_cast<const uint8_t*>(d_src); a.src_off = d_src_off; a.src_len = d_src_len; a.n_blocks = n_blocks;
@@ -1505,8 +1179,9 @@ int b200lz4_decompress_dev(const void* d_src, const int64_t* d_src_off, const in
                            void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
                            int header_mode, int max_block, void* d_scratch, void* cuda_stream)
 {
-    if (n_blocks < 0 || !d_scratch) return fail(B200LZ4_E_ARG, "bad argument");
-    if (header_mode != 0 && header_mode != 4 && header_mode != 8) return fail(B200LZ4_E_ARG, "header_mode must be 0, 4 or 8");
+    const Verdict v = check_batch(Entry::Dev, true, d_scratch, n_blocks, header_mode, max_block, d_src, 0, d_src_off, d_src_len,
+                                  d_dst, d_dst_off, d_out_len, d_stream_first, n_streams, false);
+    if (v.code) return fail(v);
     if (n_blocks == 0) return 0;
     DecompressArgs a{};
     a.src = static_cast<const uint8_t*>(d_src); a.src_off = d_src_off; a.src_len = d_src_len; a.n_blocks = n_blocks;
@@ -1543,25 +1218,25 @@ int b200lz4_xxh32_batch(b200lz4_ctx* c, const void* src, int64_t src_bytes, cons
     if (!c) return fail(B200LZ4_E_ARG, "ctx is NULL");
     if (n < 0 || (n > 0 && (!off || !len || !out))) return fail(B200LZ4_E_ARG, "NULL argument");
     if (n == 0) return 0;
-    int rc;
-    if ((rc = check_blocks(off, len, n, src_bytes))) return rc;
+    const Verdict v = check_blocks(off, len, n, src_bytes);
+    if (v.code) return fail(v);
     CU(cudaSetDevice(c->device));
-    Carver cv;
-    const size_t o_off = cv.take(sizeof(int64_t) * n), o_len = cv.take(sizeof(int32_t) * n), o_up = cv.off, o_out = cv.take(sizeof(uint32_t) * n);
-    if ((rc = c->h_desc.ensure(cv.off))) return rc;
-    if ((rc = c->d_desc.ensure(cv.off))) return rc;
+    const DescLayout lay(n, 0, 0, 0, 0, 0, 0);     // out_len: the checksums
+    int rc;
+    if ((rc = ensure_desc(c, lay))) return rc;
     if ((rc = c->d_src.ensure((size_t)src_bytes + 64))) return rc;
-    uint8_t* hd = static_cast<uint8_t*>(c->h_desc.p); uint8_t* dd = static_cast<uint8_t*>(c->d_desc.p);
-    memcpy(hd + o_off, off, sizeof(int64_t) * n); memcpy(hd + o_len, len, sizeof(int32_t) * n);
+    void* hd = c->h_desc.p;
+    void* dd = c->d_desc.p;
+    memcpy(lay.src_off_in(hd), off, sizeof(int64_t) * n); memcpy(lay.src_len_in(hd), len, sizeof(int32_t) * n);
     cudaStream_t st = c->stream;
-    CU(cudaMemcpyAsync(dd, hd, o_up, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dd, hd, lay.upload, cudaMemcpyHostToDevice, st));
     if (src_bytes) CU(cudaMemcpyAsync(c->d_src.p, src, (size_t)src_bytes, cudaMemcpyHostToDevice, st));
-    CU(launch_xxh32(static_cast<const uint8_t*>(c->d_src.p), reinterpret_cast<const int64_t*>(dd + o_off), reinterpret_cast<const int32_t*>(dd + o_len),
-                    n, seed, reinterpret_cast<uint32_t*>(dd + o_out), st));
+    CU(launch_xxh32(static_cast<const uint8_t*>(c->d_src.p), lay.src_off_in(dd), lay.src_len_in(dd), n, seed,
+                    reinterpret_cast<uint32_t*>(lay.out_len_in(dd)), st));
     c->launches += 1;
-    CU(cudaMemcpyAsync(hd + o_out, dd + o_out, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(lay.out_len_in(hd), lay.out_len_in(dd), sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    memcpy(out, hd + o_out, sizeof(uint32_t) * n);
+    memcpy(out, lay.out_len_in(hd), sizeof(uint32_t) * n);
     return 0;
 }
 

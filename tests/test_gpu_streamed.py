@@ -1,4 +1,4 @@
-"""Streamed host call (csrc/api.cu: compress_host_streamed; compress.cu: kStreamed): a batch of equally long independent
+"""Streamed host call (csrc/api.cu: compress_host_streamed, schedule in csrc/host_plan.h; compress.cu: kStreamed): a batch of equally long independent
 blocks at a constant pitch is sent to the device segment by segment in deadline order, and the finders run while their
 blocks are still arriving.  The bytes must be the reference's whatever the order of arrival: every schedule extreme
 (plain block order, segment-major, the tuned default), each way of raising the arrival flags and of sending the decoded
