@@ -205,9 +205,16 @@ size_t b200lz4_scratch_bytes(void);
 /*
  * d_states: NULL (fresh state per stream, discarded) or device array of n_streams device
  * pointers to b200lz4_cstate_bytes() records (zero-filled = new stream).  A record's
- * dictionary buffer must have been sized with b200lz4_cstate_set_dict().
+ * dictionary buffer must have been sized with b200lz4_cstate_set_dict() to hold the
+ * largest array of its stream.  Records (compress and decompress alike) must be 16-byte
+ * aligned; both record sizes are multiples of 16, so records packed back to back from an
+ * aligned start are.
  * d_dst_cap: NULL (capacity = header_mode + compress_bound, i.e. never limiting) or per-block
- * slot capacities.
+ * slot capacities, header included.  Block i writes only inside
+ * d_dst[d_dst_off[i] .. d_dst_off[i] + d_dst_cap[i]).  It succeeds exactly when its LZ4 payload
+ * fits in d_dst_cap[i] - header_mode bytes (the limitedOutput rule of LZ4_compress_fast_continue);
+ * otherwise d_out_len[i] = 0.  A failed block whose slot holds the header gets compLen 0 there;
+ * a slot smaller than header_mode is not written at all.
  */
 int b200lz4_compress_dev(const void* d_src, const int64_t* d_src_off, const int32_t* d_src_len, int n_blocks,
                          const int32_t* d_stream_first, int n_streams, void* const* d_states,

@@ -1029,8 +1029,11 @@ __device__ void emitter_main(const CompressArgs& a, Queue* q)
             if (lane == 0 && blk >= 0) {
                 uint8_t* slot = a.dst + a.dst_off[blk];
                 a.out_len[blk] = r;
-                if (a.header >= 4) { uint32_t v = (uint32_t)r; for (int k = 0; k < 4; k++) slot[k] = (uint8_t)(v >> (8 * k)); }                 // LZ4.hs:262
-                if (a.header == 8) { uint32_t v = (uint32_t)a.src_len[blk]; for (int k = 0; k < 4; k++) slot[4 + k] = (uint8_t)(v >> (8 * k)); }   // LZ4.hs:261
+                // a slot smaller than its header has failed (cap < 0 above) and is left untouched: the header would land
+                // in the next block's slot
+                const bool room = !a.dst_cap || a.dst_cap[blk] >= a.header;
+                if (room && a.header >= 4) { uint32_t v = (uint32_t)r; for (int k = 0; k < 4; k++) slot[k] = (uint8_t)(v >> (8 * k)); }                 // LZ4.hs:262
+                if (room && a.header == 8) { uint32_t v = (uint32_t)a.src_len[blk]; for (int k = 0; k < 4; k++) slot[4 + k] = (uint8_t)(v >> (8 * k)); }   // LZ4.hs:261
             }
             op = 0; failed = false;
         }

@@ -7,7 +7,10 @@
   python tests/golden/make_golden.py checks    -> reference_checks.json: what tests/test_oracle.py compares the
                                                   restatement with (compress digests on every generator and
                                                   configuration, random edge sizes, the decoder's accept/reject verdict
-                                                  and output digest on truncated and bit-flipped blocks)
+                                                  and output digest on truncated and bit-flipped blocks, and the
+                                                  compressor's size and verdict at dstCapacity r - 1 and r)
+  python tests/golden/make_golden.py limited [LIB] -> only the `limited` section of reference_checks.json, from the
+                                                  upstream LZ4 shared library LIB (default: the system liblz4)
 
 Both need the reference build, oracle/_ref/libreflz4.so: oracle/ref_driver.c compiled with -DDRV_USE_REFERENCE against
 an LZ4 (oracle/Makefile builds it from the reference's own cbits/lz4.c when REF points at its tree).  The reference
@@ -138,6 +141,106 @@ def codec_name(ora) -> str:
     return f"LZ4 {v // 10000}.{v // 100 % 100}.{v % 100} through oracle/ref_driver.c"
 
 
+# ---- capacity-limited compression (LZ4_compress_fast_continue with dstCapacity below the bound) ----------------------
+
+def _nonzero(rng, n: int) -> bytes:
+    return rng.integers(1, 256, size=n, dtype=np.uint8).tobytes()
+
+
+def limited_inputs():
+    """Single arrays for the limitedOutput checks: every generator, the edge sizes, and two families shaped at the three
+    guards of LZ4_compress_generic (cbits/lz4.c:1024-1027 literals, :1097-1121 match length, :1207-1217 last literals):
+      tail  -- zeros then t non-zero random bytes: one match, then a last literal run of exactly t bytes;
+      match -- L random bytes repeated up to the end: one literal run of L, one match that stops at matchlimit (a last
+               run of exactly 5) with its length code around the 15 / 270 limits."""
+    rng = np.random.default_rng(11)
+    out = []
+    for kind in KINDS:
+        for n in (300, 5000, 70000):
+            out.append(datagen.make(kind, 7, n).tobytes())
+    for kind in ("text", "random", "zero"):
+        d = datagen.make(kind, 3, 65547).tobytes()
+        for n in (0, 1, 2, 3, 4, 5, 11, 12, 13, 14, 15, 16, 17, 31, 32, 33, 64, 255, 256, 270, 271, 300, 4096, 65535, 65547):
+            out.append(d[:n])
+    for t in list(range(5, 21)) + list(range(265, 276)) + [524, 525, 526]:
+        for p in (64, 300):
+            out.append(bytes(p) + _nonzero(rng, t))
+    for lit in list(range(1, 21)) + list(range(250, 275)):
+        r = _nonzero(rng, lit)
+        for m in (12, 13, 20, 23, 24, 25, 36, 270, 273, 274, 275, 290):
+            out.append((r * (m // lit + 2))[:lit + m])
+    return out
+
+
+def limited_linked_inputs():
+    """(dictionary, array) pairs: the array is compressed, capacity-limited, right after the dictionary on one stream."""
+    rng = np.random.default_rng(12)
+    pairs = []
+    for kind in ("text", "records", "mixed"):
+        d = datagen.make(kind, 19, 140000).tobytes()
+        for n in (20, 300, 5000, 70000):
+            a = d[70000:70000 + n]
+            pairs.append((d[:70000], a))
+            pairs.append((d[70000 - n // 2:70000 + n // 2], a))
+    for lit in (14, 15, 16, 255, 269, 270):
+        r = _nonzero(rng, lit)
+        pairs.append((r * 3, r[:7] + _nonzero(rng, lit)))
+    return pairs
+
+
+def limited_results(ora, pairs):
+    """For each (dictionary or None, array): [r, result at dstCapacity r - 1, result at r], r = the size at the bound,
+    each call on a fresh stream that first compressed the dictionary; and the SHA-256 of the payloads at capacity r.
+    A write past dstCapacity is an error."""
+    rows, payloads = [], []
+    for dic, a in pairs:
+        keep = [np.frombuffer(x, dtype=np.uint8).copy() if x else np.zeros(1, np.uint8) for x in (dic or b"", a)]
+        src = keep[1]
+        bound = ora.bound(len(a))
+        row = []
+        for cap in (None, "r-1", "r"):
+            c = bound if cap is None else row[0] - (cap == "r-1")
+            dst = np.full(bound + 64, 0xA5, dtype=np.uint8)
+            s = ora.ccreate()
+            if dic is not None:
+                scratch = np.zeros(ora.bound(len(dic)), dtype=np.uint8)
+                assert ora.ccont(s, keep[0].ctypes.data, scratch.ctypes.data, len(dic), scratch.size, 1) > 0
+            got = ora.ccont(s, src.ctypes.data, dst.ctypes.data, len(a), c, 1)
+            ora.cfree(s)
+            assert (dst[max(c, 0):] == 0xA5).all(), "write past dstCapacity"
+            row.append(int(got))
+            if cap == "r":
+                payloads.append(dst[:max(got, 0)].tobytes())
+        rows.append(row)
+    return rows, sha(payloads)
+
+
+class UpstreamLz4:
+    """The streaming compressor of an upstream LZ4 shared library (system liblz4 or oracle/_ref) through ctypes, with the
+    names Oracle uses (ccreate / cfree / ccont / bound)."""
+
+    def __init__(self, path: str):
+        import ctypes
+        self.lib = lib = ctypes.CDLL(path)
+        vp, ip = ctypes.c_void_p, ctypes.c_int
+        self.ccreate = lib.LZ4_createStream; self.ccreate.restype = vp; self.ccreate.argtypes = []
+        self.cfree = lib.LZ4_freeStream; self.cfree.argtypes = [vp]
+        self.bound = lib.LZ4_compressBound; self.bound.restype = ip; self.bound.argtypes = [ip]
+        self.ccont = lib.LZ4_compress_fast_continue; self.ccont.restype = ip
+        self.ccont.argtypes = [vp, vp, vp, ip, ip, ip]
+        self.path = path
+
+
+def make_limited(up: UpstreamLz4):
+    single, single_sha = limited_results(up, [(None, a) for a in limited_inputs()])
+    linked, linked_sha = limited_results(up, limited_linked_inputs())
+    v = up.lib.LZ4_versionNumber()
+    print("limited: single", len(single), "linked", len(linked))
+    return {"codec": f"LZ4 {v // 10000}.{v // 100 % 100}.{v % 100} ({os.path.basename(up.path)}, "
+                     "LZ4_compress_fast_continue through ctypes)",
+            "single": single, "single_payload_sha256": single_sha, "linked": linked, "linked_payload_sha256": linked_sha}
+
+
 def make_golden(ref):
     out = {"generator": "tests/golden/make_golden.py", "codec": codec_name(ref), "cases": []}
     for name, kind, seed, total, bs, accel, linked, cfg in CASES:
@@ -173,10 +276,21 @@ def make_checks(ref):
           "rejected", verdicts.count(None))
     return {"generator": "tests/golden/make_golden.py checks", "codec": codec_name(ref),
             "configs": configs, "edge_size_trials": edges,
-            "decoder": {"payload_sha256": hashlib.sha256(payload).hexdigest(), "verdicts": verdicts}}
+            "decoder": {"payload_sha256": hashlib.sha256(payload).hexdigest(), "verdicts": verdicts},
+            "limited": make_limited(UpstreamLz4(ref.lib._name))}
 
 
 def main():
+    if sys.argv[1:2] == ["limited"]:
+        # only the `limited` section of reference_checks.json, from any upstream LZ4 build (default: the system liblz4)
+        import ctypes.util
+        path = sys.argv[2] if len(sys.argv) > 2 else ctypes.util.find_library("lz4")
+        assert path, "no liblz4 found: name one, make_golden.py limited /path/to/liblz4.so"
+        out = load("reference_checks.json")
+        out["limited"] = make_limited(UpstreamLz4(path))
+        with open(os.path.join(HERE, "reference_checks.json"), "w") as f:
+            json.dump(out, f, indent=1)
+        return
     assert available("reference"), "needs the reference build oracle/_ref/libreflz4.so"
     ref = Oracle("reference")
     if sys.argv[1:] == ["checks"]:

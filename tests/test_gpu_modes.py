@@ -10,14 +10,15 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SUBSET = ["tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py", "-k",
-          "random_round_trips or echoing or split_over or generators or edge_sizes or acceleration_sweep or linked_state"]
+SUBSET = ["tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py", "tests/test_gpu_device_abi.py", "-k",
+          "random_round_trips or echoing or split_over or generators or edge_sizes or acceleration_sweep or linked_state or "
+          "(device_abi and not decompress_dev and not compact_dev)"]
 
 
-DECODE_SUBSET = ["tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py", "tests/test_gpu_configs.py", "-k",
+DECODE_SUBSET = ["tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py", "tests/test_gpu_configs.py", "tests/test_gpu_device_abi.py", "-k",
                  "handbuilt or corrupted or random_round_trips or echoing or split_over or generators or edge_sizes or "
                  "empty_and_tiny or block_max or large_blocks or linked_state or malformed or fragmented or "
-                 "config3 or config4"]       # config 3: 1 678 one-block streams = several streams per CTA in the wide kernel
+                 "config3 or config4 or (device_abi and (decompress_dev or scratch_shared))"]       # config 3: 1 678 one-block streams = several streams per CTA in the wide kernel
 
 
 @pytest.mark.parametrize("env", [{"B200LZ4_DWIDE": "0"},        # every decode through the narrow kernel (parser + copier warp per stream)
@@ -54,7 +55,9 @@ def test_decoder_bounds_checked_build_on_malformed_input(ctx):
     for wide in ("0", "1"):
         e = dict(os.environ, B200LZ4_LIB=lib, B200LZ4_DWIDE=wide)
         out = subprocess.run([sys.executable, "-m", "pytest", "-x", "-q", "-m", "gpu", "tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py",
-                              "-k", "handbuilt or corrupted or malformed or edge_sizes or echoing"], cwd=ROOT, env=e,
+                              "tests/test_gpu_device_abi.py",
+                              "-k", "handbuilt or corrupted or malformed or edge_sizes or echoing or (device_abi and decompress_dev)"],
+                             cwd=ROOT, env=e,
                              stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
         assert out.returncode == 0, out.stdout[-3000:]
         assert " passed" in out.stdout

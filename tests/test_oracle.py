@@ -100,6 +100,25 @@ def test_decoder_accept_reject_agrees_with_reference(built, port):
             assert golden.decode_verdict(ref, arr) == got, f"corrupted block {i}"
 
 
+@pytest.mark.parametrize("section", ["single", "linked"])
+def test_port_limited_output_agrees_with_reference(built, port, section):
+    """LZ4_compress_fast_continue with dstCapacity r - 1 and r (r = the size at the bound), on inputs shaped at each of the
+    three limitedOutput guards: the restatement must give upstream's sizes, verdicts and bytes and never write past
+    dstCapacity.  Only the first capacity-limited call of a stream is pinned: after a failure lz4.h leaves the state
+    undefined."""
+    want = CHECKS["limited"]
+    pairs = ([(None, a) for a in golden.limited_inputs()] if section == "single" else golden.limited_linked_inputs())
+    rows, digest = golden.limited_results(port, pairs)
+    assert len(rows) == len(want[section])
+    for i, (got, w) in enumerate(zip(rows, want[section])):
+        assert got == w, f"{section} input {i}: restatement {got}, upstream {w} ([r, at r - 1, at r])"
+    assert digest == want[f"{section}_payload_sha256"]
+    assert all(r1 == 0 and rr == r for r, r1, rr in rows)      # success exactly when the payload fits
+    ref = live_reference()
+    if ref is not None:
+        assert golden.limited_results(ref, pairs) == (rows, digest)
+
+
 # ---- resizeChunksD restatement (pure Python) --------------------------------------------------
 
 def _framed(port, n_arrays=20, bs=5000):
