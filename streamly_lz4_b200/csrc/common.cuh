@@ -35,7 +35,9 @@ struct DState {
 };
 static_assert(sizeof(CState) % 16 == 0 && sizeof(DState) % 16 == 0, "state records packed back to back stay 16-byte aligned");
 
-struct Scratch {                    // zero-filled once by the caller; kernels leave it zeroed
+// Zero-filled once by the caller; kernels leave it zeroed.  Each kernel that hands out streams through a work counter owns
+// one pair (claim counter, CTAs done): the compress kernels 0/1, the narrow decoder 2/3.
+struct Scratch {
     uint32_t work_counter[4];
     uint32_t pad_[60];
 };
@@ -43,6 +45,100 @@ struct Scratch {                    // zero-filled once by the caller; kernels l
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31; }
 __device__ __forceinline__ uint32_t lanemask_lt()
 { uint32_t m; asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m)); return m; }
+
+// ---- work distribution over a Scratch counter pair ------------------------
+// next stream for this warp (all lanes call): lane 0 draws it from the claim counter
+__device__ __forceinline__ int claim_stream(uint32_t* counter)
+{
+    int s = 0;
+    if (lane_id() == 0) s = (int)atomicAdd(counter, 1u);
+    return __shfl_sync(kFull, s, 0);
+}
+// all threads of the CTA call it at the end: the last CTA out resets counter pair `first` so that the scratch stays
+// zeroed for the next launch
+__device__ __forceinline__ void release_counters(Scratch* scratch, int first)
+{
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t done = atomicAdd(&scratch->work_counter[first + 1], 1u);
+        if (done == gridDim.x - 1) { scratch->work_counter[first] = 0; scratch->work_counter[first + 1] = 0; __threadfence(); }
+    }
+}
+
+// ---- shared memory, cp.async, mbarriers -----------------------------------
+// All shared-memory accesses of the kernels' hot loops use explicit 32-bit shared-space addresses.
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ uint32_t lds8(uint32_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
+__device__ __forceinline__ uint32_t lds16(uint32_t a) { uint32_t v; asm volatile("ld.shared.u16 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
+__device__ __forceinline__ uint32_t lds32(uint32_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
+__device__ __forceinline__ uint4 lds128(uint32_t a)
+{ uint4 v; asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a) : "memory"); return v; }
+__device__ __forceinline__ void sts8(uint32_t a, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void sts16(uint32_t a, uint32_t v) { asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void sts64(uint32_t a, uint32_t x, uint32_t y) { asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(a), "r"(x), "r"(y) : "memory"); }
+__device__ __forceinline__ void sts128(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w)
+{ asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory"); }
+
+// cp_async_4 caches in L1 (.ca: the compress finder's input lines, re-read by neighbouring probes); cp_async_16 bypasses
+// it (.cg: the decoders' compressed payload, read once)
+__device__ __forceinline__ void cp_async_4(uint32_t smem_addr, const void* g)
+{ asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_addr), "l"(g) : "memory"); }
+__device__ __forceinline__ void cp_async_16(uint32_t smem_addr, const void* g)
+{ asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(g) : "memory"); }
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
+__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count)
+{ asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory"); }
+__device__ __forceinline__ void mbar_arrive(unsigned long long* bar)
+{ asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory"); }
+// one attempt to wait for the phase of the given parity on the mbarrier at shared address bar_s, suspended in hardware
+// for up to about suspend_ns (a waiting warp does not burn issue slots); true once the phase has completed
+__device__ __forceinline__ bool mbar_try_wait(uint32_t bar_s, uint32_t parity, uint32_t suspend_ns)
+{
+    uint32_t ok;
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n"
+        "selp.u32 %0, 1, 0, p;\n"
+        "}\n" : "=r"(ok) : "r"(bar_s), "r"(parity), "r"(suspend_ns) : "memory");
+    return ok != 0;
+}
+// waits for the phase (loops inside the asm, with a 20 us suspend hint)
+__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity)
+{
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "WAIT_%=:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
+        "@p bra DONE_%=;\n"
+        "bra WAIT_%=;\n"
+        "DONE_%=:\n"
+        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"(20000u) : "memory");
+}
+// the same test without a suspend hint: returns after the hardware's own short time limit (the caller sleeps in between)
+__device__ __forceinline__ bool mbar_test(unsigned long long* bar, uint32_t parity)
+{
+    uint32_t ok;
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
+        "selp.u32 %0, 1, 0, p;\n"
+        "}\n" : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
+    return ok != 0;
+}
+
+// ---- global memory: system-scope flags, L2 prefetch -------------------------
+// a flag word written by the host or another stream (acquire: what it announces is visible once it is seen)
+__device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p)
+{ uint32_t v; asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
+__device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes)
+{ asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory"); }
 
 // ---- unaligned little-endian reads through the read-only path ------------
 // 4 bytes at p; touches only the aligned words that contain p[0..3].

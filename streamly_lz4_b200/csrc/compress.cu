@@ -41,7 +41,6 @@
 // The compaction pass (compact.cu) then gathers the per-block slots into one stream.
 #include <cstdio>
 #include <cstdlib>
-#include <mutex>
 #include "common.cuh"
 #include "kernels.h"
 
@@ -62,37 +61,6 @@ struct __align__(16) Queue {
     int pad_[4];
 };
 constexpr int kEndBlock = 1 << 30, kTerminate = 1 << 29;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count)
-{ asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory"); }
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar)
-{ asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory"); }
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"(20000u) : "memory");   // suspend-time hint: do not burn issue slots while idle
-}
-__device__ __forceinline__ bool mbar_test(unsigned long long* bar, uint32_t parity)
-{
-    uint32_t ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n" : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes)
-{ asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory"); }
 
 // offset (from the run start) and step of probe j >= 0 of a search run (cbits/lz4.c:957-967).
 __device__ __forceinline__ void probe_schedule(long long j, int accel, long long& off, int& step)
@@ -174,25 +142,12 @@ __device__ __forceinline__ uint32_t warp_common_suffix(const uint8_t* a, const u
 //   invariant while ip is in line L:  lines L-1, L, L+1 complete, L+2 in flight;
 //   data readable for positions [lo_pos, ready_end), hashes valid for [lo_pos, ready_end - 4).
 // All accesses use explicit 32-bit shared-space addresses (ld.shared / st.shared).
-constexpr int kWinLines = 4, kWinWords = kWinLines * 32, kWinBytes = kWinLines * 128;
+constexpr int kWinLines = 4, kWinBytes = kWinLines * 128;
 // WIDE mode (at most one stream per SM): the data ring is 128 KiB and indexed by stream position, so it holds the
 // previous array too -- every candidate within reach (65535 back, dictionary included), every catch-up and every
 // count is then served from shared memory and a block costs its instruction chain, not L2 round trips.
 constexpr int kWideLines = 1024, kWideBytes = kWideLines * 128;
 constexpr int kHashPos = 512;                    // hash ring: u16 hashes of the 512 most recent ring positions
-
-__device__ __forceinline__ void cp_async_4(uint32_t smem_addr, const void* g)
-{ asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_addr), "l"(g) : "memory"); }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ uint32_t lds32(uint32_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
-__device__ __forceinline__ uint32_t lds8(uint32_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
-__device__ __forceinline__ uint32_t lds16(uint32_t a) { uint32_t v; asm volatile("ld.shared.u16 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
-__device__ __forceinline__ void sts16(uint32_t a, uint32_t v) { asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void sts64(uint32_t a, uint32_t x, uint32_t y) { asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(a), "r"(x), "r"(y) : "memory"); }
-__device__ __forceinline__ void sts128(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w)
-{ asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory"); }
 
 struct BlockIn {
     const uint8_t* src; int n;
@@ -262,8 +217,6 @@ constexpr uint32_t kEpoch = 65536u, kRelMax = 2 * kEpoch - 1;       // rel in [1
 // windows, forward counts -- first makes sure the bytes it touches lie below it (wait_for polls the flag word the
 // copy stream bumps after each segment).  Reads at or behind ip need no check.
 constexpr long long kArrivalTimeoutCycles = 2000000000LL;        // ~1 s at 2 GHz
-__device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p)
-{ uint32_t v; asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
 
 template <bool kWide, bool kCompact, bool kStreamed>
 __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, const uint32_t hash_s, Producer& out,
@@ -832,12 +785,9 @@ __device__ void finder_main(const CompressArgs& a, uint32_t* table, uint32_t* ri
     probe_schedule(lane + 1, accel, off1, step1);       // ... starting at probe 1 (probe 0 was taken by the scalar path)
 
     for (;;) {
-        int s = 0;
-        if (lane == 0) s = (int)atomicAdd(counter, 1u);
-        s = __shfl_sync(kFull, s, 0);
+        const int s = claim_stream(counter);
         if (s >= a.n_streams) break;
-        const int b0 = a.stream_first ? a.stream_first[s] : a.first_block + s;
-        const int b1 = a.stream_first ? a.stream_first[s + 1] : b0 + 1;
+        const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
         CState* st = a.states ? reinterpret_cast<CState*>(a.states[s]) : nullptr;
 
         uint32_t offset = 0, dict_len = 0;
@@ -1040,120 +990,61 @@ __device__ void emitter_main(const CompressArgs& a, Queue* q)
     }
 }
 
-__global__ void __launch_bounds__(kPairs * 64, 3)
-compress_kernel(CompressArgs a)
+// Compact tables (see find_block): u16 entries + epoch bits, 8.5 KiB instead of 16 KiB
+constexpr int kCompactTableBytes = kHashEntries * 2 + kHashEntries / 8;
+
+// Dynamic shared memory of a compress CTA of kP finder/emitter pairs: hash rings | data rings | tables | queues from a
+// 1024-byte aligned start, plus the alignment slack.
+template <int kP, bool kWide, bool kCompact>
+constexpr size_t compress_smem()
 {
+    return 1024 + kP * (kHashPos * sizeof(uint16_t) + (kWide ? kWideBytes : kWinBytes)
+                        + (kCompact ? kCompactTableBytes : kHashEntries * sizeof(uint32_t)) + sizeof(Queue));
+}
+
+// One compress CTA: warps 0 .. kP-1 are the finders, warps kP .. 2kP-1 their emitters.
+template <int kP, bool kWide, bool kCompact, bool kStreamed>
+__device__ __forceinline__ void compress_cta(const CompressArgs& a)
+{
+    constexpr uint32_t kRingWords = (kWide ? kWideBytes : kWinBytes) / 4;
+    constexpr uint32_t kTableWords = (kCompact ? kCompactTableBytes : kHashEntries * sizeof(uint32_t)) / 4;
     extern __shared__ __align__(16) uint8_t smem_dyn[];
-    // layout (from a 1024-byte aligned start): hash rings | data rings | tables | queues
     uint8_t* smem_raw = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     uint16_t* hrings = reinterpret_cast<uint16_t*>(smem_raw);
-    uint32_t* rings = reinterpret_cast<uint32_t*>(smem_raw + kPairs * kHashPos * sizeof(uint16_t));
-    uint32_t* tables = rings + kPairs * kWinWords;
-    Queue* queues = reinterpret_cast<Queue*>(tables + kPairs * kHashEntries);
+    uint32_t* rings = reinterpret_cast<uint32_t*>(smem_raw + kP * kHashPos * sizeof(uint16_t));
+    uint32_t* tables = rings + kP * kRingWords;
+    Queue* queues = reinterpret_cast<Queue*>(tables + kP * kTableWords);
     const uint32_t warp = threadIdx.x >> 5;
-    const uint32_t pair = warp & (kPairs - 1);
-    if (threadIdx.x < kPairs) {
+    const uint32_t pair = warp & (kP - 1);
+    if (threadIdx.x < kP) {
         Queue* q = &queues[threadIdx.x];
         mbar_init(&q->full[0], 1); mbar_init(&q->full[1], 1);
         mbar_init(&q->empty[0], 1); mbar_init(&q->empty[1], 1);
     }
     __syncthreads();
-    if (warp < kPairs) finder_main<false, false>(a, tables + pair * kHashEntries, rings + pair * kWinWords, hrings + pair * kHashPos, &queues[pair]);
+    if (warp < kP) finder_main<kWide, kCompact, kStreamed>(a, tables + pair * kTableWords, rings + pair * kRingWords,
+                                                            hrings + pair * kHashPos, &queues[pair]);
     else emitter_main(a, &queues[pair]);
-    // last CTA out resets the work counter so the scratch stays zeroed for the next launch
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t done = atomicAdd(&a.scratch->work_counter[1], 1u);
-        if (done == gridDim.x - 1) { a.scratch->work_counter[0] = 0; a.scratch->work_counter[1] = 0; __threadfence(); }
-    }
+    release_counters(a.scratch, 0);
 }
+
+__global__ void __launch_bounds__(kPairs * 64, 3)
+compress_kernel(CompressArgs a) { compress_cta<kPairs, false, false, false>(a); }
 
 // Streamed launches (host batch calls, see api.cu): the classic geometry, finders wait for their input segment by segment.
 __global__ void __launch_bounds__(kPairs * 64, 3)
-compress_kernel_streamed(CompressArgs a)
-{
-    extern __shared__ __align__(16) uint8_t smem_dyn[];
-    uint8_t* smem_raw = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
-    uint16_t* hrings = reinterpret_cast<uint16_t*>(smem_raw);
-    uint32_t* rings = reinterpret_cast<uint32_t*>(smem_raw + kPairs * kHashPos * sizeof(uint16_t));
-    uint32_t* tables = rings + kPairs * kWinWords;
-    Queue* queues = reinterpret_cast<Queue*>(tables + kPairs * kHashEntries);
-    const uint32_t warp = threadIdx.x >> 5;
-    const uint32_t pair = warp & (kPairs - 1);
-    if (threadIdx.x < kPairs) {
-        Queue* q = &queues[threadIdx.x];
-        mbar_init(&q->full[0], 1); mbar_init(&q->full[1], 1);
-        mbar_init(&q->empty[0], 1); mbar_init(&q->empty[1], 1);
-    }
-    __syncthreads();
-    if (warp < kPairs) finder_main<false, false, true>(a, tables + pair * kHashEntries, rings + pair * kWinWords, hrings + pair * kHashPos, &queues[pair]);
-    else emitter_main(a, &queues[pair]);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t done = atomicAdd(&a.scratch->work_counter[1], 1u);
-        if (done == gridDim.x - 1) { a.scratch->work_counter[0] = 0; a.scratch->work_counter[1] = 0; __threadfence(); }
-    }
-}
+compress_kernel_streamed(CompressArgs a) { compress_cta<kPairs, false, false, true>(a); }
 
 // Compact mode: the dense kernel with 8.5 KiB position tables (see find_block): 4 CTAs of 4 pairs per SM = 16 streams in
 // flight per SM instead of 12.  Used for launches of more than one wave of the classic kernel.
-constexpr int kCompactTableBytes = kHashEntries * 2 + kHashEntries / 8;      // u16 entries + epoch bits
-constexpr size_t kCompactSmem = 1024 /* alignment slack */ + kPairs * (kHashPos * sizeof(uint16_t) + kWinBytes + kCompactTableBytes + sizeof(Queue));
-
 __global__ void __launch_bounds__(kPairs * 64, 4)
-compress_kernel_compact(CompressArgs a)
-{
-    extern __shared__ __align__(16) uint8_t smem_dyn[];
-    uint8_t* smem_raw = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
-    uint16_t* hrings = reinterpret_cast<uint16_t*>(smem_raw);
-    uint32_t* rings = reinterpret_cast<uint32_t*>(smem_raw + kPairs * kHashPos * sizeof(uint16_t));
-    uint8_t* tables = reinterpret_cast<uint8_t*>(rings + kPairs * kWinWords);
-    Queue* queues = reinterpret_cast<Queue*>(tables + kPairs * kCompactTableBytes);
-    const uint32_t warp = threadIdx.x >> 5;
-    const uint32_t pair = warp & (kPairs - 1);
-    if (threadIdx.x < kPairs) {
-        Queue* q = &queues[threadIdx.x];
-        mbar_init(&q->full[0], 1); mbar_init(&q->full[1], 1);
-        mbar_init(&q->empty[0], 1); mbar_init(&q->empty[1], 1);
-    }
-    __syncthreads();
-    if (warp < kPairs) finder_main<false, true>(a, reinterpret_cast<uint32_t*>(tables + pair * kCompactTableBytes), rings + pair * kWinWords,
-                                                 hrings + pair * kHashPos, &queues[pair]);
-    else emitter_main(a, &queues[pair]);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t done = atomicAdd(&a.scratch->work_counter[1], 1u);
-        if (done == gridDim.x - 1) { a.scratch->work_counter[0] = 0; a.scratch->work_counter[1] = 0; __threadfence(); }
-    }
-}
+compress_kernel_compact(CompressArgs a) { compress_cta<kPairs, false, true, false>(a); }
 
 // Wide mode: one finder/emitter pair per CTA, one CTA per SM (144 KiB: hash ring | 128 KiB data ring | table | queue).
 // Used when a launch has no more streams than the device has SMs (few linked streams, few large blocks, the tail
 // chunk of a host batch): per-stream latency is all that matters then.
-constexpr size_t kWideSmem = 1024 /* alignment slack */ + kHashPos * sizeof(uint16_t) + kWideBytes + kHashEntries * sizeof(uint32_t) + sizeof(Queue);
-
 __global__ void __launch_bounds__(64, 1)
-compress_kernel_wide(CompressArgs a)
-{
-    extern __shared__ __align__(16) uint8_t smem_dyn[];
-    uint8_t* smem_raw = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
-    uint16_t* hring = reinterpret_cast<uint16_t*>(smem_raw);
-    uint32_t* ring = reinterpret_cast<uint32_t*>(smem_raw + kHashPos * sizeof(uint16_t));
-    uint32_t* table = ring + kWideBytes / 4;
-    Queue* q = reinterpret_cast<Queue*>(table + kHashEntries);
-    if (threadIdx.x == 0) {
-        mbar_init(&q->full[0], 1); mbar_init(&q->full[1], 1);
-        mbar_init(&q->empty[0], 1); mbar_init(&q->empty[1], 1);
-    }
-    __syncthreads();
-    if (threadIdx.x < 32) finder_main<true, false>(a, table, ring, hring, q);
-    else emitter_main(a, q);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t done = atomicAdd(&a.scratch->work_counter[1], 1u);
-        if (done == gridDim.x - 1) { a.scratch->work_counter[0] = 0; a.scratch->work_counter[1] = 0; __threadfence(); }
-    }
-}
+compress_kernel_wide(CompressArgs a) { compress_cta<1, true, false, false>(a); }
 
 __global__ void set_flag_kernel(uint32_t* flag, uint32_t v) { *flag = v; __threadfence(); }
 
@@ -1199,32 +1090,24 @@ cudaError_t launch_alias_probe(const uint32_t* flag, uint32_t* result, long long
 
 cudaError_t launch_compress(const CompressArgs& a, cudaStream_t stream)
 {
-    static std::mutex mu;
-    static bool configured[64] = {false};   // per device: dynamic shared-memory limits of the three kernels set
-    const size_t smem = kPairs * kHashEntries * sizeof(uint32_t) + kPairs * sizeof(Queue) + kPairs * kWinWords * sizeof(uint32_t)
-                        + kPairs * kHashPos * sizeof(uint16_t) + 1024 /* alignment slack */;
+    constexpr size_t smem = compress_smem<kPairs, false, false>();         // classic and streamed
+    constexpr size_t kCompactSmem = compress_smem<kPairs, false, true>(), kWideSmem = compress_smem<1, true, false>();
     int sm_count = 0;
     cudaError_t e = device_sm_count(&sm_count); if (e != cudaSuccess) return e;
-    int dev = 0; e = cudaGetDevice(&dev); if (e != cudaSuccess) return e;
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        if (!configured[dev]) {
-            e = cudaFuncSetAttribute(compress_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(compress_kernel_streamed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(compress_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWideSmem);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(compress_kernel_compact, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCompactSmem);
-            if (e != cudaSuccess) return e;
-            configured[dev] = true;
-            if (getenv("B200LZ4_DEBUG")) {
-                int occ = 0;
-                cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, compress_kernel, kPairs * 64, smem);
-                fprintf(stderr, "[b200lz4] compress_kernel: %zu B dynamic smem, %d CTAs/SM, %d SMs\n", smem, occ, sm_count);
-            }
+    static PerDeviceOnce once;
+    e = once.run([&] {
+        cudaError_t r = cudaFuncSetAttribute(compress_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (r == cudaSuccess) r = cudaFuncSetAttribute(compress_kernel_streamed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (r == cudaSuccess) r = cudaFuncSetAttribute(compress_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWideSmem);
+        if (r == cudaSuccess) r = cudaFuncSetAttribute(compress_kernel_compact, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCompactSmem);
+        if (r == cudaSuccess && getenv("B200LZ4_DEBUG")) {
+            int occ = 0;
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, compress_kernel, kPairs * 64, smem);
+            fprintf(stderr, "[b200lz4] compress_kernel: %zu B dynamic smem, %d CTAs/SM, %d SMs\n", smem, occ, sm_count);
         }
-    }
+        return r;
+    });
+    if (e != cudaSuccess) return e;
     if (a.n_streams <= 0) return cudaSuccess;
     if (a.arrived) {                             // input still arriving: classic geometry, finders poll a.arrived
         const int want = (a.n_streams + kPairs - 1) / kPairs, max_ctas = sm_count * 3;

@@ -1,7 +1,7 @@
-// decode_common.cuh -- what the two decoder kernels share: constants, shared-memory / mbarrier helpers, the block
-// geometry of decompressChunk and the block PARSER (parse_block), which walks the token chain of one LZ4 block with
-// every accept/reject rule of the reference's safe decoder (cbits/lz4.c:1929-2151) and hands sequence descriptors to a
-// sink PT:
+// decode_common.cuh -- what the two decoder kernels share: constants, the in-order copy of matches that read recent
+// output (copy_near_matches, with overlap_inv), the block geometry of decompressChunk and the block PARSER (parse_block),
+// which walks the token chain of one LZ4 block with every accept/reject rule of the reference's safe decoder
+// (cbits/lz4.c:1929-2151) and hands sequence descriptors to a sink PT:
 //     decompress.cu       Parser   -- shared-memory double buffer read by ONE copier warp        (kWide == false)
 //     decompress_wide.cu  WParser  -- global-memory descriptor ring read by several copier warps (kWide == true)
 // Sink interface: kWide, kRing; ring_s, end, issued_end, ready_end, cur_start, fill; at(p), top_up(ip), ensure(ip, need),
@@ -45,35 +45,6 @@ constexpr int kEndBlock = 1 << 30;       // block finished; result[] holds what 
 constexpr int kTerminate = 1 << 29;
 constexpr int kFailed = 1 << 28;          // wide mode, with kEndBlock: the parser rejected the block
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ uint32_t lds8(uint32_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
-__device__ __forceinline__ void sts8(uint32_t a, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ uint4 lds128(uint32_t a)
-{ uint4 v; asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a) : "memory"); return v; }
-__device__ __forceinline__ void sts128(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w)
-{ asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory"); }
-__device__ __forceinline__ void cp_async_16(uint32_t smem_addr, const void* g)
-{ asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(g) : "memory"); }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count)
-{ asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory"); }
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar)
-{ asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory"); }
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"(20000u) : "memory");
-}
-
 __device__ __forceinline__ int read_le32(const uint8_t* p)
 { return (int)((uint32_t)__ldg(p) | ((uint32_t)__ldg(p + 1) << 8) | ((uint32_t)__ldg(p + 2) << 16) | ((uint32_t)__ldg(p + 3) << 24)); }
 
@@ -106,6 +77,33 @@ __device__ __forceinline__ void warp_copy_rw(uint8_t* dst, const uint8_t* src, u
     }
     const uint32_t done = nvec << 4, tail = len - done;
     if (lane < tail) dst[done + lane] = src[done + lane];
+}
+
+// Overlapping match (offset < length <= 64): byte i comes from source byte i mod offset.  i mod offset through a 16-bit
+// fixed-point reciprocal, exact for i < 64 (inv = 65536/offset plus at most 3); inv = 0 makes it the identity for
+// ordinary matches.
+__device__ __forceinline__ uint32_t overlap_inv(uint32_t dist, uint32_t mlen)
+{ return (dist < mlen) ? (uint32_t)(65536.0f * __frcp_rn((float)dist)) + 2u : 0u; }
+
+// Matches that read recent output, in order, each copied by all lanes within the output ring at out_s (kMask: ring size
+// - 1).  par_s + 16 * i holds {destination, length <= 64, offset, overlap_inv} of match i, for every bit i of dep != 0;
+// lane is the caller's lane_id().
+template <uint32_t kMask>
+__device__ __forceinline__ void copy_near_matches(uint32_t out_s, uint32_t par_s, uint32_t dep, const uint32_t lane)
+{
+    const uint32_t i1 = lane + 32;
+    uint4 nx = lds128(par_s + 16u * (uint32_t)(__ffs(dep) - 1));
+    for (;;) {
+        dep &= dep - 1;
+        const uint4 cu = nx;
+        if (dep) nx = lds128(par_s + 16u * (uint32_t)(__ffs(dep) - 1));      // next match's parameters, early
+        const uint32_t csa = cu.x - cu.z;
+        const uint32_t k0 = lane - ((lane * cu.w) >> 16) * cu.z, k1 = i1 - ((i1 * cu.w) >> 16) * cu.z;
+        if (lane < cu.y) sts8(out_s + ((cu.x + lane) & kMask), lds8(out_s + ((csa + k0) & kMask)));
+        if (i1 < cu.y) sts8(out_s + ((cu.x + i1) & kMask), lds8(out_s + ((csa + k1) & kMask)));
+        __syncwarp();
+        if (!dep) break;
+    }
 }
 
 // Header fields and the checks of decompressChunk (src/Streamly/Internal/LZ4.hs:303-318): both warps

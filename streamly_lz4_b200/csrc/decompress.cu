@@ -145,19 +145,15 @@ struct Parser {
 
 __device__ void parser_main(const DecompressArgs& a, DQueue* q, uint32_t ring_s)
 {
-    const uint32_t lane = lane_id();
     uint32_t* counter = &a.scratch->work_counter[2];
     Parser P;
     P.q = q; P.ring_s = ring_s; P.batch = 0; P.fill = 0; P.flags = 0; P.prev_pending = false; P.prev_start = 0; P.cur_start = 0;
     P.block = -1; P.stream = -1;
     P.begin();
     for (;;) {
-        int s = 0;
-        if (lane == 0) s = (int)atomicAdd(counter, 1u);
-        s = __shfl_sync(kFull, s, 0);
+        const int s = claim_stream(counter);
         if (s >= a.n_streams) break;
-        const int b0 = a.stream_first ? a.stream_first[s] : a.first_block + s;
-        const int b1 = a.stream_first ? a.stream_first[s + 1] : b0 + 1;
+        const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
         const DState* st = a.states ? reinterpret_cast<const DState*>(a.states[s]) : nullptr;
         uint32_t dict_len = st ? st->prev_len : 0u;
         for (int b = b0; b < b1; b++) {
@@ -415,31 +411,14 @@ __device__ void copier_main(const DecompressArgs& a, DQueue* q, uint32_t in_s, u
             __syncwarp();
             // phase B: matches that read bytes of this batch, in order, each copied by all lanes.  Their sources lie
             // within 64 bytes of the batch start, which the ring always holds (see preload()).
-            uint32_t dep = __ballot_sync(kFull, has_match && !indep);
+            const uint32_t dep = __ballot_sync(kFull, has_match && !indep);
             if (dep) {
-                // every lane leaves {destination, length, offset, reciprocal} of its match in the (already consumed)
-                // descriptor slot, so the loop below reads one broadcast 128-bit word per match instead of shuffling
+                // every lane leaves the parameters of its match in the (already consumed) descriptor slot, so the loop
+                // reads one broadcast 128-bit word per match instead of shuffling
                 const uint32_t par_s = smem_u32(&q->desc[b][0]);
-                {   // overlapping match (offset < length <= 64): byte i comes from source byte i mod offset; i mod offset
-                    // through a 16-bit fixed-point reciprocal, exact for i < 64 (inv = 65536/offset plus at most 3);
-                    // inv = 0 makes it the identity for ordinary matches
-                    const uint32_t inv = (dist < mlen) ? (uint32_t)(65536.0f * __frcp_rn((float)dist)) + 2u : 0u;
-                    sts128(par_s + 16u * lane, da, mlen, dist, inv);
-                }
+                sts128(par_s + 16u * lane, da, mlen, dist, overlap_inv(dist, mlen));
                 __syncwarp();
-                const uint32_t i1 = lane + 32;
-                uint4 nx = lds128(par_s + 16u * (uint32_t)(__ffs(dep) - 1));
-                for (;;) {
-                    dep &= dep - 1;
-                    const uint4 cu = nx;
-                    if (dep) nx = lds128(par_s + 16u * (uint32_t)(__ffs(dep) - 1));      // next match's parameters, early
-                    const uint32_t csa = cu.x - cu.z;
-                    const uint32_t k0 = lane - ((lane * cu.w) >> 16) * cu.z, k1 = i1 - ((i1 * cu.w) >> 16) * cu.z;
-                    if (lane < cu.y) sts8(out_s + ((cu.x + lane) & M), lds8(out_s + ((csa + k0) & M)));
-                    if (i1 < cu.y) sts8(out_s + ((cu.x + i1) & M), lds8(out_s + ((csa + k1) & M)));
-                    __syncwarp();
-                    if (!dep) break;
-                }
+                copy_near_matches<M>(out_s, par_s, dep, lane);
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(&q->empty[b]);  // literals copied, descriptor slots no longer in use
@@ -489,11 +468,19 @@ decompress_kernel(DecompressArgs a)
     asm volatile("mov.u32 %0, %1;" : "=r"(out_s) : "r"(smem_u32(out_ring)));
     if (threadIdx.x < 32) parser_main(a, &queue, in_s);
     else copier_main<kPublish, kMirror>(a, &queue, in_s, out_s);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t done = atomicAdd(&a.scratch->work_counter[3], 1u);
-        if (done == gridDim.x - 1) { a.scratch->work_counter[2] = 0; a.scratch->work_counter[3] = 0; __threadfence(); }
+    release_counters(a.scratch, 2);
+}
+
+// 12 CTAs per SM while every stream gets a CTA of its own, else 16 per SM (one wave; CTAs claim further streams)
+template <bool kPublish, bool kMirror>
+cudaError_t launch_narrow(const DecompressArgs& a, int sm_count, cudaStream_t stream)
+{
+    if (a.n_streams <= sm_count * 12) decompress_kernel<12, kPublish, kMirror><<<a.n_streams, 64, 0, stream>>>(a);
+    else {
+        const int max_ctas = sm_count * 16;
+        decompress_kernel<16, kPublish, kMirror><<<a.n_streams < max_ctas ? a.n_streams : max_ctas, 64, 0, stream>>>(a);
     }
+    return cudaGetLastError();
 }
 
 }  // namespace
@@ -524,32 +511,14 @@ cudaError_t launch_decompress(const DecompressArgs& a, cudaStream_t stream)
     // them that the narrow kernel would leave most of the GPU idle (measured: 128 streams 17 -> 35 GB/s on mixed data, 11 ->
     // 49 GB/s on text; with more than two streams per SM the narrow kernel's 16 CTAs per SM win).  Independent blocks gain
     // nothing from it -- a block has ONE token chain, so only one of the eight parsers would work.
-    if (a.host_dst) {                       // host call with a page-locked destination: the output goes home from inside the kernel
-        if (a.n_streams <= sm_count * 12) decompress_kernel<12, false, true><<<a.n_streams, 64, 0, stream>>>(b);
-        else {
-            const int max_ctas = sm_count * 16;
-            decompress_kernel<16, false, true><<<a.n_streams < max_ctas ? a.n_streams : max_ctas, 64, 0, stream>>>(b);
-        }
-        return cudaGetLastError();
-    }
-    if (a.seg_count) {                      // streamed host call: independent blocks, output leaves segment by segment
-        if (a.n_streams <= sm_count * 12) decompress_kernel<12, true><<<a.n_streams, 64, 0, stream>>>(b);
-        else {
-            const int max_ctas = sm_count * 16;
-            decompress_kernel<16, true><<<a.n_streams < max_ctas ? a.n_streams : max_ctas, 64, 0, stream>>>(b);
-        }
-        return cudaGetLastError();
-    }
+    if (a.host_dst)                         // host call with a page-locked destination: the output goes home from inside the kernel
+        return launch_narrow<false, true>(b, sm_count, stream);
+    if (a.seg_count)                        // streamed host call: independent blocks, output leaves segment by segment
+        return launch_narrow<true, false>(b, sm_count, stream);
     bool wide = a.stream_first != nullptr && a.n_streams <= 2 * sm_count;
     if (wide_env) wide = wide_env[0] == '1';
     if (wide && a.wide_arena) return launch_decompress_wide(b, sm_count, stream);
-    if (a.n_streams <= sm_count * 12) {
-        decompress_kernel<12><<<a.n_streams, 64, 0, stream>>>(b);
-    } else {
-        const int max_ctas = sm_count * 16;
-        decompress_kernel<16><<<a.n_streams < max_ctas ? a.n_streams : max_ctas, 64, 0, stream>>>(b);
-    }
-    return cudaGetLastError();
+    return launch_narrow<false, false>(b, sm_count, stream);
 }
 
 }  // namespace b200lz4

@@ -31,7 +31,6 @@
 // batches sit in shared memory); long sequences are cut into pieces of 16 KiB by the parser so that every batch is small
 // against that window.
 #include <cstdlib>
-#include <mutex>
 #include "decode_common.cuh"
 
 namespace b200lz4 {
@@ -63,12 +62,12 @@ constexpr uint32_t kSeedBase = 65536;             // stream position of the firs
 #ifdef B200LZ4_WIDE_STATS
 #define WSTAT_DECL(n) unsigned long long wst_[n] = {0}; long long wst_t_ = clock64();
 #define WSTAT(i) { const long long now_ = clock64(); wst_[i] += (unsigned long long)(now_ - wst_t_); wst_t_ = now_; }
-#define WSTAT_COUNT(i) { wst_[i]++; }
+#define WSTAT_COUNT(i, n) { wst_[i] += (unsigned long long)(n); }
 #define WSTAT_FLUSH(a, base, n) { if (lane_id() == 0) for (int q_ = 0; q_ < (n); q_++) atomicAdd(reinterpret_cast<unsigned long long*>((a).scratch->pad_) + (base) + q_, wst_[q_]); }
 #else
 #define WSTAT_DECL(n)
 #define WSTAT(i)
-#define WSTAT_COUNT(i)
+#define WSTAT_COUNT(i, n)
 #define WSTAT_FLUSH(a, base, n)
 #endif
 
@@ -97,8 +96,6 @@ struct WCtl {                                     // shared memory
 
 __device__ __forceinline__ uint32_t vld(const uint32_t* p) { return *reinterpret_cast<const volatile uint32_t*>(p); }
 __device__ __forceinline__ void vst(uint32_t* p, uint32_t v) { *reinterpret_cast<volatile uint32_t*>(p) = v; }
-__device__ __forceinline__ uint32_t lds32(uint32_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
-__device__ __forceinline__ void sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 __device__ __forceinline__ uint4 ld_cg_128(const uint4* p)
 { uint4 v; asm volatile("ld.global.cg.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory"); return v; }
 
@@ -328,8 +325,7 @@ __device__ void wparser_main(const DecompressArgs& a, int j, WCtl* ctl, uint32_t
     const long long p0_ = clock64();
 #endif
     for (int s = blockIdx.x; s < a.n_streams; s += gridDim.x) {
-        const int b0 = a.stream_first ? a.stream_first[s] : a.first_block + s;
-        const int b1 = a.stream_first ? a.stream_first[s + 1] : b0 + 1;
+        const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
         for (int b = b0 + j; b < b1; b += kWP) {        // block (b - b0) of a stream belongs to parser (b - b0) % 8
             const BlockGeom g = block_geom(a, b);
             P.flags = kBegin; P.need = 0; P.op_start = P.op_end = 0;
@@ -380,8 +376,7 @@ __device__ void wdispatch_main(const DecompressArgs& a, WCtl* ctl, uint32_t out_
     WDispatch D{ctl, 0u, 0u, kSeedBase};
     WSTAT_DECL(4)       // 0 other, 1 waiting for the parser, 2 waiting for flow control, 3 stream open / close
     for (int s = blockIdx.x; s < a.n_streams; s += gridDim.x) {
-        const int b0 = a.stream_first ? a.stream_first[s] : a.first_block + s;
-        const int b1 = a.stream_first ? a.stream_first[s + 1] : b0 + 1;
+        const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
         DState* st = a.states ? reinterpret_cast<DState*>(a.states[s]) : nullptr;
         // ---- open the stream: the ring restarts at kSeedBase with the kept tail of the previous call as dictionary
         WSTAT(0)
@@ -476,16 +471,7 @@ __device__ void wdispatch_main(const DecompressArgs& a, WCtl* ctl, uint32_t out_
 // ---------------------------------------------------------------------- copiers ----
 // one attempt to wait (suspended in hardware for up to ~1 us) for the phase of ticket t on its slot's barrier
 __device__ __forceinline__ bool bar_try(unsigned long long* bars, uint32_t t)
-{
-    uint32_t ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n" : "=r"(ok) : "r"(smem_u32(&bars[t & (kTickets - 1)])), "r"((t >> 6) & 1u), "r"(1000u) : "memory");
-    return ok != 0;
-}
+{ return mbar_try_wait(smem_u32(&bars[t & (kTickets - 1)]), (t >> 6) & 1u, 1000u); }
 __device__ __forceinline__ void bar_wait(unsigned long long* bars, uint32_t t) { while (!bar_try(bars, t)) { } }
 // all lanes' earlier writes, then one arrival for ticket t
 __device__ __forceinline__ void bar_signal(unsigned long long* bars, uint32_t t)
@@ -520,7 +506,7 @@ __device__ void wstage_literals(const DecompressArgs& a, int w, WCtl* ctl, uint3
     WSTAT_DECL(4)       // 0 waiting for a ticket, 1 loads, 2 copy, 3 tickets
     for (uint32_t t = (uint32_t)w;; t += kWL) {
         if (!wait_ticket(ctl, t)) break;
-        WSTAT(0) WSTAT_COUNT(3)
+        WSTAT(0) WSTAT_COUNT(3, 1)
         const WTk k = read_ticket(ctl, t);
         const int cnt = k.cf & 0xFF;
         uint32_t nvec = ((uint32_t)k.cf >> 8) & 0xFFu, lo = k.aux;       // where the batch's literals lie (0 vectors: not given)
@@ -569,10 +555,8 @@ __device__ void wstage_literals(const DecompressArgs& a, int w, WCtl* ctl, uint3
 }
 
 // stage F: matches whose source is final before the ticket starts, lane-parallel (tickets w, w + kWF, ...).  It also
-// prepares the serial stage's work: the parameters {destination, length, offset, reciprocal} of every match replace the
-// (consumed) descriptors, and one word says which of them are NEAR, so that stage N spends nothing on bookkeeping.
-// An overlapping match (offset < length <= 64) repeats its first `offset` bytes: byte i comes from source byte i mod
-// offset, through a 16-bit fixed-point reciprocal that is exact for i < 64 (0 makes it the identity).
+// prepares the serial stage's work: the parameters of every match (see copy_near_matches) replace the (consumed)
+// descriptors, and one word says which of them are NEAR, so that stage N spends nothing on bookkeeping.
 __device__ void wstage_far(const DecompressArgs& a, int w, WCtl* ctl, uint32_t out_s, uint32_t desc_s)
 {
     const uint32_t lane = lane_id();
@@ -601,10 +585,7 @@ __device__ void wstage_far(const DecompressArgs& a, int w, WCtl* ctl, uint32_t o
                 const bool live = (int)lane < cnt && mlen != 0 && (int)(from - k.valid_lo) >= 0;     // (a match below the dictionary: block rejected)
                 const bool far = live && (int)(from + mlen - k.safe) <= 0;
                 nmask = __ballot_sync(kFull, live && !far);
-                if (nmask) {
-                    const uint32_t inv = (dist < mlen) ? (uint32_t)(65536.0f * __frcp_rn((float)dist)) + 2u : 0u;
-                    sts128(dslot + 16u * lane, m_pos, mlen, dist, inv);     // (every lane has read its own descriptor)
-                }
+                if (nmask) sts128(dslot + 16u * lane, m_pos, mlen, dist, overlap_inv(dist, mlen));     // (every lane has read its own descriptor)
                 // everything below `safe` (the start of ticket t - kWDepth) is final once stage N has finished ticket t - kWDepth - 1
                 if (__ballot_sync(kFull, far)) {
                     if (t > (uint32_t)kWDepth) bar_wait(ctl->bar_near, t - kWDepth - 1);
@@ -623,16 +604,14 @@ __device__ void wstage_far(const DecompressArgs& a, int w, WCtl* ctl, uint32_t o
 // stage N: the serial chain -- near matches in stream order, each copied by all lanes; long match pieces
 __device__ void wstage_near(const DecompressArgs& a, WCtl* ctl, uint32_t out_s, uint32_t desc_s)
 {
-    constexpr uint32_t M = kWM;
     const uint32_t lane = lane_id();
-    const uint32_t i1 = lane + 32;
     WSTAT_DECL(4)       // 0 waiting for stage F, 1 near matches, 2 long matches, 3 near matches (count)
     for (uint32_t t = 0;; t++) {
         bool fin = false;
         while (!bar_try(ctl->bar_far, t))                                   // (stage F has waited for the ticket and for stage L)
             if (vld(&ctl->finished) && (int)(t - vld(&ctl->t_final)) >= 0) { fin = true; break; }
         if (fin) break;
-        uint32_t dep = vld(&ctl->near_mask[t & (kWSlots - 1)]);
+        const uint32_t dep = vld(&ctl->near_mask[t & (kWSlots - 1)]);
         const uint32_t is_long = vld(&ctl->near_long[t & (kWSlots - 1)]);
         const uint32_t dslot = desc_s + (t & (kWSlots - 1)) * 512u;
         WSTAT(0)
@@ -641,19 +620,8 @@ __device__ void wstage_near(const DecompressArgs& a, WCtl* ctl, uint32_t out_s, 
             coop_long_match(out_s, d.x, d.y, d.z);
             WSTAT(2)
         } else if (dep) {
-            uint4 nx = lds128(dslot + 16u * (uint32_t)(__ffs(dep) - 1));
-            for (;;) {
-                dep &= dep - 1;
-                const uint4 cu = nx;
-                if (dep) nx = lds128(dslot + 16u * (uint32_t)(__ffs(dep) - 1));
-                const uint32_t csa = cu.x - cu.z;
-                const uint32_t k0 = lane - ((lane * cu.w) >> 16) * cu.z, k1 = i1 - ((i1 * cu.w) >> 16) * cu.z;
-                if (lane < cu.y) sts8(out_s + ((cu.x + lane) & M), lds8(out_s + ((csa + k0) & M)));
-                if (i1 < cu.y) sts8(out_s + ((cu.x + i1) & M), lds8(out_s + ((csa + k1) & M)));
-                __syncwarp();
-                WSTAT_COUNT(3)
-                if (!dep) break;
-            }
+            copy_near_matches<kWM>(out_s, dslot, dep, lane);
+            WSTAT_COUNT(3, __popc(dep))
             WSTAT(1)
         }
         bar_signal(ctl->bar_near, t);
@@ -731,18 +699,11 @@ decompress_kernel_wide(DecompressArgs a)
 
 cudaError_t launch_decompress_wide(const DecompressArgs& a, int sm_count, cudaStream_t stream)
 {
-    static std::mutex mu;
-    static bool configured[64] = {false};
-    int dev = 0; cudaError_t e = cudaGetDevice(&dev); if (e != cudaSuccess) return e;
-    if (dev < 0 || dev >= 64) return cudaErrorInvalidDevice;
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        if (!configured[dev]) {
-            e = cudaFuncSetAttribute(decompress_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWSmem);
-            if (e != cudaSuccess) return e;
-            configured[dev] = true;
-        }
-    }
+    static PerDeviceOnce once;
+    const cudaError_t e = once.run([] {
+        return cudaFuncSetAttribute(decompress_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWSmem);
+    });
+    if (e != cudaSuccess) return e;
     int grid = a.n_streams < sm_count ? a.n_streams : sm_count;
     if (grid > a.wide_ctas) grid = a.wide_ctas;
     if (grid <= 0) return cudaErrorInvalidValue;

@@ -1,6 +1,7 @@
 // kernels.h -- launch interfaces between the C ABI (api.cu) and the kernels.
 #pragma once
 #include <cstdint>
+#include <mutex>
 #include <cuda_runtime.h>
 #include "common.cuh"
 
@@ -37,6 +38,13 @@ struct DecompressArgs {
     uint8_t* host_dst;
 };
 
+// Blocks [b0, b1) of stream s of a launch: its run in stream_first, or in independent mode the one block first_block + s.
+// (Two scalar functions: returning the pair as one struct changes the register allocation of the narrow decoder.)
+template <class Args> __device__ __forceinline__ int stream_begin(const Args& a, int s)
+{ return a.stream_first ? a.stream_first[s] : a.first_block + s; }
+template <class Args> __device__ __forceinline__ int stream_end(const Args& a, int s, int b0)
+{ return a.stream_first ? a.stream_first[s + 1] : b0 + 1; }
+
 // decompress_kernel_wide keeps its parsed-ahead sequence descriptors in global memory (L2): per CTA, kWideParsers rings of
 // kWideRingBatches batches of 32 descriptors of 16 bytes.
 constexpr int kWideParsers = 8;
@@ -52,6 +60,22 @@ struct CompactArgs {
     // optional mirrors in mapped pinned HOST memory (written by the scan kernel over PCIe, so the host learns the
     // sizes without a D2H memcpy that would queue behind bulk transfers on the copy engine)
     int64_t* host_off; int32_t* host_len;
+};
+
+// Per-device setup a launcher does once (dynamic shared-memory limits), safe for host threads launching on several devices.
+struct PerDeviceOnce {
+    std::mutex mu;
+    bool done[64] = {};
+    template <class F> cudaError_t run(F configure)
+    {
+        int dev = 0; cudaError_t e = cudaGetDevice(&dev); if (e != cudaSuccess) return e;
+        if (dev < 0 || dev >= 64) return cudaErrorInvalidDevice;
+        std::lock_guard<std::mutex> lk(mu);
+        if (done[dev]) return cudaSuccess;
+        e = configure();
+        if (e == cudaSuccess) done[dev] = true;
+        return e;
+    }
 };
 
 cudaError_t launch_compress(const CompressArgs& a, cudaStream_t stream);
