@@ -67,6 +67,7 @@ extern "C" {
 typedef struct b200lz4_ctx b200lz4_ctx;               /* one per (host thread, device) */
 typedef struct b200lz4_cstream b200lz4_cstream;       /* device-resident LZ4_stream_t equivalent (cbits/lz4.h:595-603) */
 typedef struct b200lz4_dstream b200lz4_dstream;       /* device-resident LZ4_streamDecode_t equivalent (cbits/lz4.h:605-610) */
+typedef struct b200lz4_dict b200lz4_dict;             /* a dictionary loaded on one ctx's device (LZ4_loadDict semantics) */
 
 /* ---------------------------------------------------------------- misc -- */
 
@@ -162,6 +163,39 @@ int b200lz4_decompress_batch(b200lz4_ctx* ctx,
                              int header_mode, int max_block,
                              void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len);
 
+/* ---------------------------------------------------------- dictionaries -- */
+/*
+ * A shared dictionary, byte-exact with upstream LZ4 (1.9.3 / 1.9.4):
+ *   compress    = LZ4_createStream -> LZ4_loadDict(s, dict, len) -> LZ4_compress_fast_continue per array.  Only the last
+ *                 64 KiB count; a dictionary shorter than 8 bytes loads nothing but still moves currentOffset to 64 KiB,
+ *                 so the output differs from a fresh stream's.
+ *   decompress  = LZ4_decompress_safe_usingDict(src, dst, n, cap, dict, len) for a stream's first block (linked streams:
+ *                 LZ4_setStreamDecode(dict, len) then _continue).  The whole length counts for the offset check.
+ * b200lz4_dict_create copies len host bytes to the ctx's device and loads them there; the dict belongs to that ctx and may
+ * be used by any number of calls until b200lz4_dict_free.
+ * *_batch_dict: the arguments of b200lz4_{de,}compress_batch plus the dictionary.  Every stream starts from it (independent
+ * mode: every block; linked mode: the first block of each stream, later blocks see the previous array as usual).  Passing
+ * persistent `streams` as well is B200LZ4_E_ARG: load the dictionary into the handles instead (b200lz4_cstream_load_dict,
+ * b200lz4_dstream_set_dict), which is LZ4_loadDict / LZ4_setStreamDecode on a stream that persists across calls.
+ * The multi-device calls take no dictionary.
+ */
+int  b200lz4_dict_create(b200lz4_ctx* ctx, const void* dict, int64_t len, b200lz4_dict** out);
+void b200lz4_dict_free(b200lz4_dict* d);
+int  b200lz4_cstream_load_dict(b200lz4_cstream* s, const b200lz4_dict* d);
+int  b200lz4_dstream_set_dict(b200lz4_dstream* s, const b200lz4_dict* d);
+int b200lz4_compress_batch_dict(b200lz4_ctx* ctx,
+                                const void* src, int64_t src_bytes,
+                                const int64_t* src_off, const int32_t* src_len, int n_blocks,
+                                const int32_t* stream_first, int n_streams, b200lz4_cstream* const* streams,
+                                int acceleration, int header_mode,
+                                void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len, const b200lz4_dict* dict);
+int b200lz4_decompress_batch_dict(b200lz4_ctx* ctx,
+                                  const void* src, int64_t src_bytes,
+                                  const int64_t* src_off, const int32_t* src_len, int n_blocks,
+                                  const int32_t* stream_first, int n_streams, b200lz4_dstream* const* streams,
+                                  int header_mode, int max_block,
+                                  void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len, const b200lz4_dict* dict);
+
 /* ------------------------------------------- batched, HOST data, N devices -- */
 /* One batch striped over several GPUs of one box (SURVEY.md section 8e): contiguous ranges of blocks (independent
  * mode) or of whole streams (linked mode), balanced by source bytes; one host thread and one b200lz4_ctx per device;
@@ -172,7 +206,7 @@ int b200lz4_decompress_batch(b200lz4_ctx* ctx,
  *     the end of block i where two devices' ranges meet (each device writes into its own worst-case region), so
  *     dst_cap must be >= the sum of header_mode + b200lz4_compress_bound(src_len[i]) (compress) / of the block
  *     capacities (decompress).
- * devices == NULL: the first n usable devices (n <= 0: all). */
+ * devices == NULL: the first n usable devices (n <= 0: all).  There are no dictionary variants of these calls. */
 typedef struct b200lz4_mctx b200lz4_mctx;
 int  b200lz4_mctx_create(const int* devices, int n, b200lz4_mctx** out);
 void b200lz4_mctx_destroy(b200lz4_mctx* m);
@@ -231,6 +265,25 @@ int b200lz4_decompress_dev(const void* d_src, const int64_t* d_src_off, const in
                            void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
                            int header_mode, int max_block,
                            void* d_scratch, void* cuda_stream);
+
+/*
+ * Dictionaries on the device.  b200lz4_dict_load_dev enqueues LZ4_loadDict(d_dict, len) into the record d_cstate
+ * (b200lz4_cstate_bytes(), 16-byte aligned; it points into d_dict, which must stay unchanged while the record is used)
+ * and LZ4_setStreamDecode(d_dict, len) into d_dstate (b200lz4_dstate_bytes(); the bytes are copied in).  Either may be
+ * NULL.  The *_dev_dict calls take the arguments of the *_dev calls plus such a record, which every stream starts from
+ * and which no kernel writes; d_states must be NULL then (B200LZ4_E_ARG otherwise).
+ */
+int b200lz4_dict_load_dev(const void* d_dict, int64_t len, void* d_cstate, void* d_dstate, void* cuda_stream);
+int b200lz4_compress_dev_dict(const void* d_src, const int64_t* d_src_off, const int32_t* d_src_len, int n_blocks,
+                              const int32_t* d_stream_first, int n_streams, void* const* d_states, const void* d_dict_cstate,
+                              void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
+                              int acceleration, int header_mode,
+                              void* d_scratch, void* cuda_stream);
+int b200lz4_decompress_dev_dict(const void* d_src, const int64_t* d_src_off, const int32_t* d_src_len, int n_blocks,
+                                const int32_t* d_stream_first, int n_streams, void* const* d_states, const void* d_dict_dstate,
+                                void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
+                                int header_mode, int max_block,
+                                void* d_scratch, void* cuda_stream);
 
 /*
  * Compaction pass: gather per-block slots into one contiguous framed stream.
@@ -296,6 +349,10 @@ int LZ4_freeStreamDecode(LZ4_streamDecode_t* s);
 int LZ4_compressBound(int inputSize);
 int LZ4_compress_fast_continue(LZ4_stream_t* s, const char* src, char* dst, int srcSize, int dstCapacity, int acceleration);
 int LZ4_decompress_safe_continue(LZ4_streamDecode_t* s, const char* src, char* dst, int srcSize, int dstCapacity);
+/* upstream's dictionary calls, same signatures and results: LZ4_loadDict returns the dictionary size it kept (the last
+ * 64 KiB, 0 below 8 bytes), LZ4_setStreamDecode returns 1 (0 on a failure upstream cannot have, e.g. no device) */
+int LZ4_loadDict(LZ4_stream_t* s, const char* dictionary, int dictSize);
+int LZ4_setStreamDecode(LZ4_streamDecode_t* s, const char* dictionary, int dictSize);
 
 #ifdef __cplusplus
 }

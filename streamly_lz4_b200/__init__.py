@@ -5,14 +5,14 @@ this package is the host-side mirror of the reference's `Streamly.LZ4` interface
 plus the ctypes binding used by tests and bench.  No CPU codec lives here.
 """
 from .api import (BlockConfig, BlockSize, FrameConfig, Context, MultiContext, CompressStream, DecompressStream, LZ4Error,
-                  compress_chunks, decompress_chunks, decompress_chunks_raw, resize_chunks,
+                  Dictionary, compress_chunks, decompress_chunks, decompress_chunks_raw, resize_chunks,
                   default_block_config, default_frame_config, set_block_max_size,
                   set_block_independence, set_frame_end_mark,
                   simple_frame_parser, frame_header, compress_chunks_frame, decompress_chunks_with,
                   parse_frame_header, write_frame, read_frame, FrameInfo)
 
 __all__ = ["BlockConfig", "BlockSize", "FrameConfig", "Context", "MultiContext", "CompressStream", "DecompressStream", "LZ4Error",
-           "compress_chunks", "decompress_chunks", "decompress_chunks_raw", "resize_chunks",
+           "Dictionary", "compress_chunks", "decompress_chunks", "decompress_chunks_raw", "resize_chunks",
            "default_block_config", "default_frame_config", "set_block_max_size",
            "set_block_independence", "set_frame_end_mark",
            "simple_frame_parser", "frame_header", "compress_chunks_frame", "decompress_chunks_with",

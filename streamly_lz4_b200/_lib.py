@@ -53,6 +53,14 @@ PROTOTYPES = {
                                        c_int, c_int, c_vp, c_i64, c_vp, c_vp]),
     "b200lz4_decompress_batch": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_int, c_vp, c_int, c_vp,
                                          c_int, c_int, c_vp, c_i64, c_vp, c_vp]),
+    "b200lz4_dict_create": (c_int, [c_vp, c_vp, c_i64, ctypes.POINTER(c_vp)]),
+    "b200lz4_dict_free": (None, [c_vp]),
+    "b200lz4_cstream_load_dict": (c_int, [c_vp, c_vp]),
+    "b200lz4_dstream_set_dict": (c_int, [c_vp, c_vp]),
+    "b200lz4_compress_batch_dict": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_int, c_vp, c_int, c_vp,
+                                            c_int, c_int, c_vp, c_i64, c_vp, c_vp, c_vp]),
+    "b200lz4_decompress_batch_dict": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_int, c_vp, c_int, c_vp,
+                                              c_int, c_int, c_vp, c_i64, c_vp, c_vp, c_vp]),
     "b200lz4_cstate_bytes": (c_sz, []),
     "b200lz4_dstate_bytes": (c_sz, []),
     "b200lz4_scratch_bytes": (c_sz, []),
@@ -61,6 +69,11 @@ PROTOTYPES = {
                                      c_int, c_int, c_vp, c_vp]),
     "b200lz4_decompress_dev": (c_int, [c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
                                        c_int, c_int, c_vp, c_vp]),
+    "b200lz4_dict_load_dev": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp]),
+    "b200lz4_compress_dev_dict": (c_int, [c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                          c_int, c_int, c_vp, c_vp]),
+    "b200lz4_decompress_dev_dict": (c_int, [c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                            c_int, c_int, c_vp, c_vp]),
     "b200lz4_compact_dev": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp]),
     "b200lz4_reframe": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_i64,
                                 ctypes.POINTER(c_i64), ctypes.POINTER(c_i64), ctypes.POINTER(c_int)]),
@@ -75,6 +88,8 @@ PROTOTYPES = {
     "LZ4_compressBound": (c_int, [c_int]),
     "LZ4_compress_fast_continue": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int]),
     "LZ4_decompress_safe_continue": (c_int, [c_vp, c_vp, c_vp, c_int, c_int]),
+    "LZ4_loadDict": (c_int, [c_vp, c_vp, c_int]),
+    "LZ4_setStreamDecode": (c_int, [c_vp, c_vp, c_int]),
 }
 
 _LIB = None

@@ -149,10 +149,16 @@ class Context:
             raise LZ4Error("b200lz4_copy_probe: " + _lib.last_error())
         return rc
 
+    def dictionary(self, data) -> "Dictionary":
+        """Load `data` as a shared dictionary on this ctx's device (LZ4_loadDict / LZ4_setStreamDecode semantics)."""
+        return Dictionary(self, data)
+
     # ---- raw batch calls on numpy buffers --------------------------------
     def compress_batch(self, src: np.ndarray, src_off: np.ndarray, src_len: np.ndarray,
                        accel: int, header: int, dst: np.ndarray,
-                       stream_first: Optional[np.ndarray] = None, streams: Optional[Sequence] = None):
+                       stream_first: Optional[np.ndarray] = None, streams: Optional[Sequence] = None,
+                       dictionary: Optional["Dictionary"] = None):
+        """dictionary: every stream without a persistent handle starts from it (b200lz4_compress_batch_dict)."""
         n = len(src_len)
         dst_off = np.zeros(n + 1, dtype=np.int64)
         out_len = np.zeros(n, dtype=np.int32)
@@ -161,15 +167,20 @@ class Context:
         sh = None
         if streams is not None:
             sh = (ctypes.c_void_p * ns)(*[s.handle for s in streams])
-        rc = self.lib.b200lz4_compress_batch(
-            self.handle, src.ctypes.data, src.size, src_off.ctypes.data, src_len.ctypes.data, n,
-            None if sf is None else sf.ctypes.data, ns, sh, accel, header,
-            dst.ctypes.data, dst.size, dst_off.ctypes.data, out_len.ctypes.data)
+        args = (self.handle, src.ctypes.data, src.size, src_off.ctypes.data, src_len.ctypes.data, n,
+                None if sf is None else sf.ctypes.data, ns, sh, accel, header,
+                dst.ctypes.data, dst.size, dst_off.ctypes.data, out_len.ctypes.data)
+        if dictionary is None:
+            rc = self.lib.b200lz4_compress_batch(*args)
+        else:
+            rc = self.lib.b200lz4_compress_batch_dict(*args, dictionary.handle)
         return rc, dst_off, out_len
 
     def decompress_batch(self, src: np.ndarray, src_off: np.ndarray, src_len: np.ndarray,
                          header: int, max_block: int, dst: np.ndarray,
-                         stream_first: Optional[np.ndarray] = None, streams: Optional[Sequence] = None):
+                         stream_first: Optional[np.ndarray] = None, streams: Optional[Sequence] = None,
+                         dictionary: Optional["Dictionary"] = None):
+        """dictionary: every stream without a persistent handle starts from it (b200lz4_decompress_batch_dict)."""
         n = len(src_len)
         dst_off = np.zeros(n + 1, dtype=np.int64)
         out_len = np.zeros(n, dtype=np.int32)
@@ -178,11 +189,43 @@ class Context:
         sh = None
         if streams is not None:
             sh = (ctypes.c_void_p * ns)(*[s.handle for s in streams])
-        rc = self.lib.b200lz4_decompress_batch(
-            self.handle, src.ctypes.data, src.size, src_off.ctypes.data, src_len.ctypes.data, n,
-            None if sf is None else sf.ctypes.data, ns, sh, header, max_block,
-            dst.ctypes.data, dst.size, dst_off.ctypes.data, out_len.ctypes.data)
+        args = (self.handle, src.ctypes.data, src.size, src_off.ctypes.data, src_len.ctypes.data, n,
+                None if sf is None else sf.ctypes.data, ns, sh, header, max_block,
+                dst.ctypes.data, dst.size, dst_off.ctypes.data, out_len.ctypes.data)
+        if dictionary is None:
+            rc = self.lib.b200lz4_decompress_batch(*args)
+        else:
+            rc = self.lib.b200lz4_decompress_batch_dict(*args, dictionary.handle)
         return rc, dst_off, out_len
+
+
+class Dictionary:
+    """A dictionary loaded on one Context's device (b200lz4_dict).  Only the last 64 KiB reach the codec; `len(d)` is the
+    full length, which the decoder's offset check uses."""
+
+    def __init__(self, ctx: Context, data):
+        self.ctx = ctx
+        self.data = bytes(data)
+        h = ctypes.c_void_p()
+        rc = ctx.lib.b200lz4_dict_create(ctx.handle, self.data, len(self.data), ctypes.byref(h))
+        if rc != 0:
+            raise LZ4Error("b200lz4_dict_create: " + _lib.last_error())
+        self.handle = h
+
+    def __len__(self) -> int:
+        return len(self.data)
+
+    def free(self):
+        if self.handle:
+            self.ctx.lib.b200lz4_dict_free(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            if self.ctx.handle:
+                self.free()
+        except Exception:
+            pass
 
 
 class CompressStream:
@@ -203,6 +246,11 @@ class CompressStream:
         if rc != 0:
             raise LZ4Error(_lib.last_error())
         return table, off.value
+
+    def load_dict(self, d: Dictionary):
+        """LZ4_loadDict on this stream: the next array is compressed with `d` as its dictionary."""
+        if self.ctx.lib.b200lz4_cstream_load_dict(self.handle, d.handle) != 0:
+            raise LZ4Error("b200lz4_cstream_load_dict: " + _lib.last_error())
 
     def free(self):
         if self.handle:
@@ -227,6 +275,11 @@ class DecompressStream:
         if rc != 0:
             raise LZ4Error("b200lz4_dstream_create: " + _lib.last_error())
         self.handle = h
+
+    def set_dict(self, d: Dictionary):
+        """LZ4_setStreamDecode(d): the next block is decoded with `d` as the previous output."""
+        if self.ctx.lib.b200lz4_dstream_set_dict(self.handle, d.handle) != 0:
+            raise LZ4Error("b200lz4_dstream_set_dict: " + _lib.last_error())
 
     def free(self):
         if self.handle:
@@ -379,18 +432,23 @@ def _staged(ctx: Context, name: str, groups):
 
 
 def compress_chunks(cfg: BlockConfig, speed: int, chunks: Iterable, *, ctx: Optional[Context] = None,
-                    batch_arrays: int = 4096, batch_bytes: int = 256 << 20, copy: bool = True) -> Iterator[bytes]:
+                    batch_arrays: int = 4096, batch_bytes: int = 256 << 20, copy: bool = True,
+                    dictionary: Optional[Dictionary] = None) -> Iterator[bytes]:
     """compressChunks cfg speed (LZ4.hs:94-100): each input array becomes one framed LZ4 block.
 
     Linked mode (default, like the reference): one device stream state for the whole
     stream, arrays strictly in order.  cfg.independent: fresh state per array.
+    dictionary: a Dictionary of the same ctx; every array (independent) or the first one (linked) is compressed as after
+    LZ4_loadDict.
     copy=False yields numpy views into the pinned result buffer instead of bytes objects (what the Haskell shim does
     with array slices); a view stays valid until the batch after the next one has been produced.
     """
-    ctx = ctx or default_context()
+    ctx = ctx or (dictionary.ctx if dictionary is not None else default_context())
     speed = max(int(speed), 0)                                   # Internal/LZ4.hs:364
     header = cfg.meta_size
     stream = None if cfg.independent else CompressStream(ctx)    # CompressInit, Internal/LZ4.hs:367-376
+    if stream is not None and dictionary is not None:
+        stream.load_dict(dictionary)
 
     def checked(groups):
         for group in groups:
@@ -409,7 +467,8 @@ def compress_chunks(cfg: BlockConfig, speed: int, chunks: Iterable, *, ctx: Opti
             k ^= 1
             sf = None if stream is None else np.array([0, len(group)], dtype=np.int32)
             rc, dst_off, out_len = ctx.compress_batch(src, offs, lens, speed, header, dst, sf,
-                                                      None if stream is None else [stream])
+                                                      None if stream is None else [stream],
+                                                      dictionary if stream is None else None)
             if rc != 0:                                          # Internal/LZ4.hs:257-260
                 raise LZ4Error(f"compressChunk: c_compressFastContinue failed ({rc}): {ctx.last_error()}")
             for i in range(len(group)):
@@ -443,13 +502,16 @@ def _decode_batches(chunks: Iterable, batch_arrays: int, batch_bytes: int, cap_o
 
 def decompress_chunks_raw(cfg: BlockConfig, chunks: Iterable, *, ctx: Optional[Context] = None,
                           batch_arrays: int = 4096, batch_bytes: int = 256 << 20, out_budget: int = 1 << 30,
-                          copy: bool = True) -> Iterator[bytes]:
+                          copy: bool = True, dictionary: Optional[Dictionary] = None) -> Iterator[bytes]:
     """decompressChunksRawD (Internal/LZ4.hs:539-567): every input array is exactly one framed block.
-    A batch is flushed as soon as its worst-case output would exceed out_budget bytes (1 GiB)."""
-    ctx = ctx or default_context()
+    A batch is flushed as soon as its worst-case output would exceed out_budget bytes (1 GiB).
+    dictionary: every block (independent) or the first one (linked) is decoded as LZ4_decompress_safe_usingDict would."""
+    ctx = ctx or (dictionary.ctx if dictionary is not None else default_context())
     header = cfg.meta_size
     max_block = 0 if cfg.block_size is BlockSize.BlockHasSize else cfg.block_size.value
     stream = None if cfg.independent else DecompressStream(ctx)
+    if stream is not None and dictionary is not None:
+        stream.set_dict(dictionary)
 
     def cap_of(a) -> int:
         if header == 8:
@@ -463,7 +525,8 @@ def decompress_chunks_raw(cfg: BlockConfig, chunks: Iterable, *, ctx: Optional[C
             k ^= 1
             sf = None if stream is None else np.array([0, len(group)], dtype=np.int32)
             rc, dst_off, out_len = ctx.decompress_batch(src, offs, lens, header, max_block, dst, sf,
-                                                        None if stream is None else [stream])
+                                                        None if stream is None else [stream],
+                                                        dictionary if stream is None else None)
             if rc != 0:                                          # Internal/LZ4.hs:309-330
                 raise LZ4Error(f"decompressChunk: c_decompressSafeContinue failed ({rc}): {ctx.last_error()}")
             for i in range(len(group)):
@@ -550,6 +613,7 @@ class FrameInfo:
     content_checksum: bool = False
     content_size: Optional[int] = None
     header_len: int = 7
+    dict_id: Optional[int] = None
 
 
 def simple_frame_parser(header: bytes, *, allow_independent: bool = False):
@@ -582,20 +646,24 @@ def simple_frame_parser(header: bytes, *, allow_independent: bool = False):
 
 
 def frame_header(block_size: BlockSize, *, independent: bool = False, block_checksum: bool = False,
-                 content_size: Optional[int] = None, content_checksum: bool = False, checksum: bool = True) -> bytes:
-    """A frame header [magic][FLG][BD][content size?][HC].  checksum=False writes HC = 0 like benchmark/Main.hs:92-100
-    (which only the reference's own stub parser accepts); the default is the real (XXH32(descriptor) >> 8) & 0xFF."""
+                 content_size: Optional[int] = None, content_checksum: bool = False, checksum: bool = True,
+                 dict_id: Optional[int] = None) -> bytes:
+    """A frame header [magic][FLG][BD][content size?][dict id?][HC].  checksum=False writes HC = 0 like
+    benchmark/Main.hs:92-100 (which only the reference's own stub parser accepts); the default is the real
+    (XXH32(descriptor) >> 8) & 0xFF."""
     code = {v: k for k, v in _BD_CODES.items()}[block_size]
     flg = 0x40 | (0x20 if independent else 0) | (0x10 if block_checksum else 0) | (0x08 if content_size is not None else 0) \
-        | (0x04 if content_checksum else 0)
-    desc = bytes([flg, code << 4]) + (b"" if content_size is None else int(content_size).to_bytes(8, "little"))
+        | (0x04 if content_checksum else 0) | (0x01 if dict_id is not None else 0)
+    desc = bytes([flg, code << 4]) + (b"" if content_size is None else int(content_size).to_bytes(8, "little")) \
+        + (b"" if dict_id is None else int(dict_id).to_bytes(4, "little"))
     hc = (_xxh32_short(desc) >> 8) & 0xFF if checksum else 0
     return FRAME_MAGIC.to_bytes(4, "little") + desc + bytes([hc])
 
 
-def parse_frame_header(head: bytes):
+def parse_frame_header(head: bytes, allow_dict_id: bool = False):
     """The complete descriptor parser: (BlockConfig, FrameConfig, FrameInfo).  Verifies the version, the reserved bits and
-    the header checksum; dictionary ids are not supported.  `head` must hold at least 15 bytes or the whole header."""
+    the header checksum.  A dictionary id is rejected unless allow_dict_id (then FrameInfo.dict_id holds it).  `head` must
+    hold at least 19 bytes or the whole header."""
     if len(head) < 7:
         raise LZ4Error("frame: input ended inside the frame header")
     magic = int.from_bytes(head[0:4], "little")
@@ -606,19 +674,24 @@ def parse_frame_header(head: bytes):
         raise LZ4Error("Version is not 01")
     if flg & 0x02 or bd & 0x8F:
         raise LZ4Error("frame: reserved bits are set")
-    if flg & 0x01:
+    if flg & 0x01 and not allow_dict_id:
         raise LZ4Error("Dict is not yet supported")
     bs = _BD_CODES.get(bd >> 4)
     if bs is None:
         raise LZ4Error("parseBD: Unknown block max size")
-    at, size = 6, None
+    at, size, dict_id = 6, None, None
     if flg & 0x08:
         if len(head) < 15:
             raise LZ4Error("frame: input ended inside the frame header")
         size = int.from_bytes(head[6:14], "little"); at = 14
+    if flg & 0x01:
+        if len(head) < at + 5:
+            raise LZ4Error("frame: input ended inside the frame header")
+        dict_id = int.from_bytes(head[at:at + 4], "little"); at += 4
     if head[at] != (_xxh32_short(bytes(head[4:at])) >> 8) & 0xFF:
         raise LZ4Error("frame: header checksum mismatch")
-    info = FrameInfo(block_checksum=bool(flg & 0x10), content_checksum=bool(flg & 0x04), content_size=size, header_len=at + 1)
+    info = FrameInfo(block_checksum=bool(flg & 0x10), content_checksum=bool(flg & 0x04), content_size=size, header_len=at + 1,
+                     dict_id=dict_id)
     return BlockConfig(block_size=bs, independent=bool(flg & 0x20)), FrameConfig(has_end_mark=True), info
 
 
@@ -650,16 +723,21 @@ def decompress_chunks_with(parser, chunks: Iterable, *, ctx: Optional[Context] =
 
 
 def write_frame(block_size: BlockSize, speed: int, chunks: Iterable, *, independent: bool = False, block_checksum: bool = False,
-                content_checksum: bool = False, content_size: Optional[int] = None, ctx: Optional[Context] = None, **kw) -> Iterator[bytes]:
+                content_checksum: bool = False, content_size: Optional[int] = None, ctx: Optional[Context] = None,
+                dictionary: Optional[Dictionary] = None, dict_id: Optional[int] = None, **kw) -> Iterator[bytes]:
     """A complete LZ4 frame (what the stock `lz4` tool reads): header with its real checksum, one block per input array
     ([size LE32][LZ4 block][XXH32 of the block iff block_checksum]), end mark, XXH32 of the content iff content_checksum.
     Arrays must not exceed the block maximum.  Linked blocks use the previous ARRAY as dictionary (the reference's
     semantics), which every frame decoder accepts.  Checksums are computed on the device; the content checksum needs the
-    whole content in one page-locked buffer."""
-    ctx = ctx or default_context()
+    whole content in one page-locked buffer.
+    dictionary: every block (independent) or the first one (linked) is compressed against it (`lz4 -D`); dict_id: the
+    descriptor's dictionary id (FLG bit 0), which tells a reader which dictionary to load."""
+    ctx = ctx or (dictionary.ctx if dictionary is not None else default_context())
+    if dictionary is not None:
+        kw["dictionary"] = dictionary
     cfg = BlockConfig(block_size=block_size, independent=independent)
     yield frame_header(block_size, independent=independent, block_checksum=block_checksum, content_size=content_size,
-                       content_checksum=content_checksum)
+                       content_checksum=content_checksum, dict_id=dict_id)
     import collections
     kept: List[bytes] = []
     raws = collections.deque()
@@ -707,13 +785,19 @@ def _with_block_checksums(ctx: Context, blocks: Sequence[bytes]) -> Iterator[byt
         yield b + int(h).to_bytes(4, "little")
 
 
-def read_frame(chunks: Iterable, *, ctx: Optional[Context] = None, verify: bool = True, **kw) -> Iterator[bytes]:
+def read_frame(chunks: Iterable, *, ctx: Optional[Context] = None, verify: bool = True,
+               dictionary: Optional[Dictionary] = None, **kw) -> Iterator[bytes]:
     """Decode one complete LZ4 frame from an arbitrarily fragmented byte stream: header (checksum verified), blocks
     (stored blocks pass through as literal-only LZ4 blocks, so a linked chain stays intact), block checksums, end
-    mark, content size and content checksum.  Yields one array per block."""
-    ctx = ctx or default_context()
+    mark, content size and content checksum.  Yields one array per block.
+    dictionary: the blocks are decoded as LZ4F_decompress_usingDict does (every block of an independent frame, the first
+    of a linked one).  A frame with a dictionary id is refused without one; the id itself is not checked (it names the
+    dictionary the writer used, and only the caller knows which one that is)."""
+    ctx = ctx or (dictionary.ctx if dictionary is not None else default_context())
     data = b"".join(bytes(c) for c in chunks)
-    cfg, _, info = parse_frame_header(data[:15])
+    cfg, _, info = parse_frame_header(data[:19], allow_dict_id=dictionary is not None)
+    if dictionary is not None:
+        kw["dictionary"] = dictionary
     at = info.header_len
     framed: List[bytes] = []
     check_off, check_len, check_want = [], [], []

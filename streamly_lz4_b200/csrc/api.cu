@@ -105,6 +105,10 @@ struct b200lz4_cstream {
 struct b200lz4_dstream {
     b200lz4_ctx* ctx; DState* d_state;
 };
+// a loaded dictionary: its bytes in HBM and the state records LZ4_loadDict / LZ4_setStreamDecode make of them
+struct b200lz4_dict {
+    b200lz4_ctx* ctx; uint8_t* d_bytes; int64_t len; CState* d_cstate; DState* d_dstate;
+};
 
 namespace {
 
@@ -359,7 +363,7 @@ int finish_call(b200lz4_ctx* c, int rc, const Range* r, int nr, const char* labe
 constexpr int kStreamedGaveUp = -1000;  // internal: compress_host retries through the plain pipeline
 
 int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_off, const int32_t* src_len, int n,
-                           const StreamShape& shp, int accel, int header,
+                           const StreamShape& shp, int accel, int header, const CState* dict_state,
                            void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
     int rc;
@@ -424,6 +428,7 @@ int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_o
             if ((rc = start_range(c, pc.g, ks, Span{0, 0}, d_src, hsrc))) return rc;
             CompressArgs a = launch_args<CompressArgs>(lay, dd, d_src, d_slots, n, header, groups[pc.g], c->scratch + pc.g, false, false);
             a.accel = accel; a.arrived = c->d_flags + pc.g; a.seg_bytes = geo.seg; a.busy_cycles = d_busy;
+            a.dict_state = dict_state;
             if ((rc = compress_range(c, a, lay, groups[pc.g], pc.g, d_out, ks))) return rc;
         }
         CU(cudaEventRecord(c->ev.h2d_end, st));
@@ -453,7 +458,7 @@ int compress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_o
 int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                   const int64_t* src_off, const int32_t* src_len, int n,
                   const int32_t* stream_first, int n_streams, b200lz4_cstream* const* streams,
-                  int accel, int header, const int32_t* block_cap,
+                  int accel, int header, const int32_t* block_cap, const CState* dict_state,
                   void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
     const Verdict v = check_batch(Entry::Ctx, false, c, n, header, 0, src, src_bytes, src_off, src_len, dst, dst_off, out_len,
@@ -469,7 +474,7 @@ int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
     if (shp.ok) {
         if ((rc = probe_stream_aliasing(c))) return rc;
         if (c->n_kgood >= 2) {
-            rc = compress_host_streamed(c, src, src_off, src_len, n, shp, accel, header, dst, dst_cap, dst_off, out_len);
+            rc = compress_host_streamed(c, src, src_off, src_len, n, shp, accel, header, dict_state, dst, dst_cap, dst_off, out_len);
             if (rc != kStreamedGaveUp) return rc;
             // finders gave up waiting for their input (should not happen on verified streams): never again on this
             // ctx, and this batch goes through the plain pipeline
@@ -527,6 +532,7 @@ int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                                                        stream_first != nullptr, streams != nullptr);
             a.dst_cap = block_cap ? lay.cap_in(dd) : nullptr;
             a.accel = accel;
+            a.dict_state = dict_state;
             if ((rc = compress_range(c, a, lay, chunks[k], k, d_out, ks))) return rc;
         }
         CU(cudaEventRecord(c->ev.h2d_end, st));
@@ -540,12 +546,13 @@ int compress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
 }
 
 int decompress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_off, const int32_t* src_len, int n,
-                             int L, int cap_last, void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len);
+                             int L, int cap_last, const DState* dict_state, void* dst, int64_t dst_cap, int64_t* dst_off,
+                             int32_t* out_len);
 
 int decompress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                     const int64_t* src_off, const int32_t* src_len, int n,
                     const int32_t* stream_first, int n_streams, b200lz4_dstream* const* streams,
-                    int header, int max_block,
+                    int header, int max_block, const DState* dict_state,
                     void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
     const Verdict v = check_batch(Entry::Ctx, true, c, n, header, max_block, src, src_bytes, src_off, src_len, dst, dst_off, out_len,
@@ -574,7 +581,8 @@ int decompress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                                            getenv("B200LZ4_NO_STREAMED") != nullptr, dwide_env && dwide_env[0] == '1',
                                            mirror_dst != nullptr);
     if (route.out == DecodeOut::Pieces)
-        return decompress_host_streamed(c, src, src_off, src_len, n, route.L, route.cap_last, dst, dst_cap, dst_off, out_len);
+        return decompress_host_streamed(c, src, src_off, src_len, n, route.L, route.cap_last, dict_state, dst, dst_cap, dst_off,
+                                        out_len);
     if (route.out != DecodeOut::Mirror) mirror_dst = nullptr;
     Range chunks[kMaxChunks];
     const int nchunks = plan_chunks(src_len, n, stream_first, ns, mirror_dst != nullptr, chunks);
@@ -626,6 +634,7 @@ int decompress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
             a.wide_arena = reinterpret_cast<uint4*>(static_cast<uint8_t*>(c->d_wide.p) + (size_t)wide_first[k] * kWideArenaPerCta);
             a.wide_ctas = wide_first[k + 1] - wide_first[k];
             a.host_dst = mirror_dst;
+            a.dict_state = dict_state;
             CU(launch_decompress(a, ks));
             c->launches += kernel_launches_per_decompress();
             const int nk = ch.b1 - ch.b0;
@@ -662,7 +671,8 @@ int decompress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
 // a flag in page-locked host memory, the calling thread polls the flags and queues that segment of every block of the
 // group as one 2-D D2H copy.  The copy engine then runs from "first group landed + one SEGMENT latency" to the end.
 int decompress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src_off, const int32_t* src_len, int n,
-                             int L, int cap_last, void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
+                             int L, int cap_last, const DState* dict_state, void* dst, int64_t dst_cap, int64_t* dst_off,
+                             int32_t* out_len)
 {
     int rc;
     const int header = 8;
@@ -719,6 +729,7 @@ int decompress_host_streamed(b200lz4_ctx* c, const void* src, const int64_t* src
             a.seg_count = d_counts + g * kMaxSegs;
             a.host_ready = lay.ready_in(hd) + g * kMaxSegs;
             a.seg_bytes = geo.seg; a.n_segs = geo.S;
+            a.dict_state = dict_state;
             CU(launch_decompress(a, ks));
             c->launches += kernel_launches_per_decompress();
             CU(cudaEventRecord(c->ev.k[g], ks));
@@ -981,6 +992,63 @@ void b200lz4_dstream_free(b200lz4_dstream* s)
     delete s;
 }
 
+// ---- dictionaries (LZ4_loadDict / LZ4_setStreamDecode) ----
+int b200lz4_dict_create(b200lz4_ctx* c, const void* dict, int64_t len, b200lz4_dict** out)
+{
+    if (!c || !out || len < 0 || (len > 0 && !dict)) return fail(B200LZ4_E_ARG, "NULL argument or negative length");
+    if (len > kMaxInput) return fail(B200LZ4_E_ARG, "dictionary longer than LZ4_MAX_INPUT_SIZE");
+    *out = nullptr;
+    CU(cudaSetDevice(c->device));
+    b200lz4_dict* d = new (std::nothrow) b200lz4_dict{c, nullptr, len, nullptr, nullptr};
+    if (!d) return fail(B200LZ4_E_NOMEM, "out of host memory");
+    cudaError_t e = cudaMalloc(&d->d_bytes, (size_t)len + 16);
+    if (e == cudaSuccess) e = cudaMalloc(&d->d_cstate, sizeof(CState));
+    if (e == cudaSuccess) e = cudaMalloc(&d->d_dstate, sizeof(DState));
+    if (e == cudaSuccess && len) e = cudaMemcpyAsync(d->d_bytes, dict, (size_t)len, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = launch_load_dict(d->d_bytes, len, d->d_cstate, d->d_dstate, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) { b200lz4_dict_free(d); return fail_cuda(e, "dict_create"); }
+    c->launches++;
+    *out = d;
+    return 0;
+}
+void b200lz4_dict_free(b200lz4_dict* d)
+{
+    if (!d) return;
+    cudaSetDevice(d->ctx->device);
+    sync_all(d->ctx);
+    if (d->d_bytes) cudaFree(d->d_bytes);
+    if (d->d_cstate) cudaFree(d->d_cstate);
+    if (d->d_dstate) cudaFree(d->d_dstate);
+    delete d;
+}
+int b200lz4_cstream_load_dict(b200lz4_cstream* s, const b200lz4_dict* d)
+{
+    if (!s || !d) return fail(B200LZ4_E_ARG, "NULL argument");
+    if (s->ctx != d->ctx) return fail(B200LZ4_E_ARG, "dictionary belongs to another ctx");
+    b200lz4_ctx* c = s->ctx;
+    CU(cudaSetDevice(c->device));
+    // the kernel overwrites the stream's dict_buf with its last array, so the stream keeps a copy of the dictionary's tail
+    const uint32_t dict_len = d->len < 8 ? 0u : (uint32_t)std::min<int64_t>(d->len, 65536);
+    int rc;
+    if ((rc = cstream_reserve(s, dict_len))) return rc;
+    static_assert(offsetof(CState, dict_len) == offsetof(CState, table) + sizeof(CState::table) + 4, "CState layout");
+    CU(cudaMemcpyAsync(s->d_state, d->d_cstate, offsetof(CState, dict_len) + sizeof(uint32_t), cudaMemcpyDeviceToDevice, c->stream));
+    if (dict_len) CU(cudaMemcpyAsync(s->d_dict, d->d_bytes + (d->len - dict_len), dict_len, cudaMemcpyDeviceToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    s->last_len = dict_len;
+    return 0;
+}
+int b200lz4_dstream_set_dict(b200lz4_dstream* s, const b200lz4_dict* d)
+{
+    if (!s || !d) return fail(B200LZ4_E_ARG, "NULL argument");
+    if (s->ctx != d->ctx) return fail(B200LZ4_E_ARG, "dictionary belongs to another ctx");
+    CU(cudaSetDevice(s->ctx->device));
+    CU(cudaMemcpyAsync(s->d_state, d->d_dstate, sizeof(DState), cudaMemcpyDeviceToDevice, s->ctx->stream));
+    CU(cudaStreamSynchronize(s->ctx->stream));
+    return 0;
+}
+
 int b200lz4_compress_batch(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                            const int64_t* src_off, const int32_t* src_len, int n_blocks,
                            const int32_t* stream_first, int n_streams, b200lz4_cstream* const* streams,
@@ -988,7 +1056,7 @@ int b200lz4_compress_batch(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                            void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
     const int rc = compress_host(c, src, src_bytes, src_off, src_len, n_blocks, stream_first, n_streams, streams,
-                                 acceleration, header_mode, nullptr, dst, dst_cap, dst_off, out_len);
+                                 acceleration, header_mode, nullptr, nullptr, dst, dst_cap, dst_off, out_len);
     if (c && rc) c->err = g_err;
     return rc;
 }
@@ -1000,7 +1068,43 @@ int b200lz4_decompress_batch(b200lz4_ctx* c, const void* src, int64_t src_bytes,
                              void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
 {
     const int rc = decompress_host(c, src, src_bytes, src_off, src_len, n_blocks, stream_first, n_streams, streams,
-                                   header_mode, max_block, dst, dst_cap, dst_off, out_len);
+                                   header_mode, max_block, nullptr, dst, dst_cap, dst_off, out_len);
+    if (c && rc) c->err = g_err;
+    return rc;
+}
+
+namespace {
+int check_dict(const b200lz4_ctx* c, const b200lz4_dict* d, bool streams_given)
+{
+    if (!d) return fail(B200LZ4_E_ARG, "dictionary is NULL");
+    if (c && d->ctx != c) return fail(B200LZ4_E_ARG, "dictionary belongs to another ctx");
+    if (streams_given) return fail(B200LZ4_E_ARG, "a dictionary together with persistent streams: load it into the streams instead");
+    return 0;
+}
+}  // namespace
+
+int b200lz4_compress_batch_dict(b200lz4_ctx* c, const void* src, int64_t src_bytes,
+                                const int64_t* src_off, const int32_t* src_len, int n_blocks,
+                                const int32_t* stream_first, int n_streams, b200lz4_cstream* const* streams,
+                                int acceleration, int header_mode,
+                                void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len, const b200lz4_dict* dict)
+{
+    int rc = check_dict(c, dict, streams != nullptr);
+    if (!rc) rc = compress_host(c, src, src_bytes, src_off, src_len, n_blocks, stream_first, n_streams, streams,
+                                acceleration, header_mode, nullptr, dict->d_cstate, dst, dst_cap, dst_off, out_len);
+    if (c && rc) c->err = g_err;
+    return rc;
+}
+
+int b200lz4_decompress_batch_dict(b200lz4_ctx* c, const void* src, int64_t src_bytes,
+                                  const int64_t* src_off, const int32_t* src_len, int n_blocks,
+                                  const int32_t* stream_first, int n_streams, b200lz4_dstream* const* streams,
+                                  int header_mode, int max_block,
+                                  void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len, const b200lz4_dict* dict)
+{
+    int rc = check_dict(c, dict, streams != nullptr);
+    if (!rc) rc = decompress_host(c, src, src_bytes, src_off, src_len, n_blocks, stream_first, n_streams, streams,
+                                  header_mode, max_block, dict->d_dstate, dst, dst_cap, dst_off, out_len);
     if (c && rc) c->err = g_err;
     return rc;
 }
@@ -1110,7 +1214,7 @@ int b200lz4_compress_batch_multi(b200lz4_mctx* m, const void* src, int64_t src_b
     return run_striped(m, src_off, src_len, n_blocks, stream_first, n_streams, region, dst_off, out_len,
         [&](b200lz4_ctx* c, int64_t lo, int64_t bytes, const int64_t* off, const int32_t* len, int nb, const int32_t* first, int ns,
             int64_t r0, int64_t rcap, int64_t* doff, int32_t* olen) {
-            return compress_host(c, hs + lo, bytes, off, len, nb, first, ns, nullptr, acceleration, header_mode, nullptr,
+            return compress_host(c, hs + lo, bytes, off, len, nb, first, ns, nullptr, acceleration, header_mode, nullptr, nullptr,
                                  hd + r0, rcap, doff, olen);
         });
 }
@@ -1134,7 +1238,7 @@ int b200lz4_decompress_batch_multi(b200lz4_mctx* m, const void* src, int64_t src
     return run_striped(m, src_off, src_len, n_blocks, stream_first, n_streams, region, dst_off, out_len,
         [&](b200lz4_ctx* c, int64_t lo, int64_t bytes, const int64_t* off, const int32_t* len, int nb, const int32_t* first, int ns,
             int64_t r0, int64_t rcap, int64_t* doff, int32_t* olen) {
-            return decompress_host(c, hs + lo, bytes, off, len, nb, first, ns, nullptr, header_mode, max_block,
+            return decompress_host(c, hs + lo, bytes, off, len, nb, first, ns, nullptr, header_mode, max_block, nullptr,
                                    hd + r0, rcap, doff, olen);
         });
 }
@@ -1189,6 +1293,58 @@ int b200lz4_decompress_dev(const void* d_src, const int64_t* d_src_off, const in
     a.dst = static_cast<uint8_t*>(d_dst); a.dst_off = d_dst_off; a.dst_cap = d_dst_cap; a.out_len = d_out_len;
     a.header = header_mode; a.max_block = max_block; a.scratch = static_cast<Scratch*>(d_scratch);
     a.wide_arena = reinterpret_cast<uint4*>(static_cast<uint8_t*>(d_scratch) + sizeof(Scratch)); a.wide_ctas = kWideMaxCtas;
+    CU(launch_decompress(a, static_cast<cudaStream_t>(cuda_stream)));
+    return 0;
+}
+
+int b200lz4_dict_load_dev(const void* d_dict, int64_t len, void* d_cstate, void* d_dstate, void* cuda_stream)
+{
+    if (len < 0 || (len > 0 && !d_dict)) return fail(B200LZ4_E_ARG, "NULL dictionary or negative length");
+    if (len > kMaxInput) return fail(B200LZ4_E_ARG, "dictionary longer than LZ4_MAX_INPUT_SIZE");
+    CU(launch_load_dict(static_cast<const uint8_t*>(d_dict), len, static_cast<CState*>(d_cstate), static_cast<DState*>(d_dstate),
+                        static_cast<cudaStream_t>(cuda_stream)));
+    return 0;
+}
+
+int b200lz4_compress_dev_dict(const void* d_src, const int64_t* d_src_off, const int32_t* d_src_len, int n_blocks,
+                              const int32_t* d_stream_first, int n_streams, void* const* d_states, const void* d_dict_cstate,
+                              void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
+                              int acceleration, int header_mode, void* d_scratch, void* cuda_stream)
+{
+    if (!d_dict_cstate) return fail(B200LZ4_E_ARG, "dictionary state is NULL");
+    if (d_states) return fail(B200LZ4_E_ARG, "a dictionary together with stream records: load it into the records instead");
+    const Verdict v = check_batch(Entry::Dev, false, d_scratch, n_blocks, header_mode, 0, d_src, 0, d_src_off, d_src_len, d_dst,
+                                  d_dst_off, d_out_len, d_stream_first, n_streams, false);
+    if (v.code) return fail(v);
+    if (n_blocks == 0) return 0;
+    CompressArgs a{};
+    a.src = static_cast<const uint8_t*>(d_src); a.src_off = d_src_off; a.src_len = d_src_len; a.n_blocks = n_blocks;
+    a.stream_first = d_stream_first; a.n_streams = d_stream_first ? n_streams : n_blocks;
+    a.dst = static_cast<uint8_t*>(d_dst); a.dst_off = d_dst_off; a.dst_cap = d_dst_cap; a.out_len = d_out_len;
+    a.accel = acceleration; a.header = header_mode; a.scratch = static_cast<Scratch*>(d_scratch);
+    a.dict_state = static_cast<const CState*>(d_dict_cstate);
+    CU(launch_compress(a, static_cast<cudaStream_t>(cuda_stream)));
+    return 0;
+}
+
+int b200lz4_decompress_dev_dict(const void* d_src, const int64_t* d_src_off, const int32_t* d_src_len, int n_blocks,
+                                const int32_t* d_stream_first, int n_streams, void* const* d_states, const void* d_dict_dstate,
+                                void* d_dst, const int64_t* d_dst_off, const int32_t* d_dst_cap, int32_t* d_out_len,
+                                int header_mode, int max_block, void* d_scratch, void* cuda_stream)
+{
+    if (!d_dict_dstate) return fail(B200LZ4_E_ARG, "dictionary state is NULL");
+    if (d_states) return fail(B200LZ4_E_ARG, "a dictionary together with stream records: load it into the records instead");
+    const Verdict v = check_batch(Entry::Dev, true, d_scratch, n_blocks, header_mode, max_block, d_src, 0, d_src_off, d_src_len,
+                                  d_dst, d_dst_off, d_out_len, d_stream_first, n_streams, false);
+    if (v.code) return fail(v);
+    if (n_blocks == 0) return 0;
+    DecompressArgs a{};
+    a.src = static_cast<const uint8_t*>(d_src); a.src_off = d_src_off; a.src_len = d_src_len; a.n_blocks = n_blocks;
+    a.stream_first = d_stream_first; a.n_streams = d_stream_first ? n_streams : n_blocks;
+    a.dst = static_cast<uint8_t*>(d_dst); a.dst_off = d_dst_off; a.dst_cap = d_dst_cap; a.out_len = d_out_len;
+    a.header = header_mode; a.max_block = max_block; a.scratch = static_cast<Scratch*>(d_scratch);
+    a.wide_arena = reinterpret_cast<uint4*>(static_cast<uint8_t*>(d_scratch) + sizeof(Scratch)); a.wide_ctas = kWideMaxCtas;
+    a.dict_state = static_cast<const DState*>(d_dict_dstate);
     CU(launch_decompress(a, static_cast<cudaStream_t>(cuda_stream)));
     return 0;
 }
@@ -1348,7 +1504,7 @@ int LZ4_compress_fast_continue(LZ4_stream_t* h, const char* src, char* dst, int 
     std::vector<char> tmp((size_t)bound_of(srcSize) + 16);
     b200lz4_cstream* ss = h->s;
     int rc = compress_host(ss->ctx, srcSize ? src : &empty, srcSize, &off, &len, 1, first, 1, &ss,
-                           acceleration, 0, &cap, tmp.data(), (int64_t)tmp.size(), dst_off, &out_len);
+                           acceleration, 0, &cap, nullptr, tmp.data(), (int64_t)tmp.size(), dst_off, &out_len);
     if (rc != 0 || out_len <= 0 || out_len > dstCapacity) return 0;
     memcpy(dst, tmp.data(), (size_t)out_len);
     return out_len;
@@ -1361,11 +1517,38 @@ int LZ4_decompress_safe_continue(LZ4_streamDecode_t* h, const char* src, char* d
     int64_t off = 0, dst_off[2] = {0, 0}; int32_t len = srcSize, out_len = -1, first[2] = {0, 1};
     std::vector<char> tmp((size_t)dstCapacity + 16);
     b200lz4_dstream* ss = h->s;
-    int rc = decompress_host(ss->ctx, src, srcSize, &off, &len, 1, first, 1, &ss, 0, dstCapacity,
+    int rc = decompress_host(ss->ctx, src, srcSize, &off, &len, 1, first, 1, &ss, 0, dstCapacity, nullptr,
                              tmp.data(), (int64_t)tmp.size(), dst_off, &out_len);
     if (rc != 0 && rc != B200LZ4_E_BLOCK) return -1;
     if (out_len > 0) memcpy(dst, tmp.data() + dst_off[0], (size_t)out_len);
     return out_len;
+}
+
+// LZ4_loadDict / LZ4_setStreamDecode: the dictionary is loaded on the device and copied into the stream, so the caller's
+// buffer is not referenced afterwards (upstream keeps pointing at it; either way it must not change before the next call)
+int LZ4_loadDict(LZ4_stream_t* h, const char* dict, int size)
+{
+    if (!h || !h->s) return 0;
+    if (size < 0 || !dict) size = 0;
+    std::lock_guard<std::mutex> lk(g_legacy_mu);
+    b200lz4_dict* d = nullptr;
+    if (b200lz4_dict_create(h->s->ctx, dict, size, &d) != 0) return 0;
+    const int rc = b200lz4_cstream_load_dict(h->s, d);
+    b200lz4_dict_free(d);
+    if (rc != 0) return 0;
+    return size < 8 ? 0 : std::min(size, 65536);
+}
+
+int LZ4_setStreamDecode(LZ4_streamDecode_t* h, const char* dict, int size)
+{
+    if (!h || !h->s) return 0;
+    if (size < 0 || !dict) size = 0;
+    std::lock_guard<std::mutex> lk(g_legacy_mu);
+    b200lz4_dict* d = nullptr;
+    if (b200lz4_dict_create(h->s->ctx, dict, size, &d) != 0) return 0;
+    const int rc = b200lz4_dstream_set_dict(h->s, d);
+    b200lz4_dict_free(d);
+    return rc == 0 ? 1 : 0;
 }
 
 }  // extern "C"

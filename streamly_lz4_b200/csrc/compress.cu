@@ -789,30 +789,31 @@ __device__ void finder_main(const CompressArgs& a, uint32_t* table, uint32_t* ri
         if (s >= a.n_streams) break;
         const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
         CState* st = a.states ? reinterpret_cast<CState*>(a.states[s]) : nullptr;
+        const CState* init = a.states ? st : a.dict_state;                 // where the stream starts from (read only)
 
         uint32_t offset = 0, dict_len = 0;
         const uint8_t* dict_end = nullptr;
         uint32_t tbase = 0;
         uint16_t* const t16 = reinterpret_cast<uint16_t*>(table);          // compact layout: 4096 x u16, then 128 x u32 epoch bits
         uint32_t* const tfl = table + kHashEntries / 2;
-        {   // table: zero (fresh LZ4_initStream, :1443-1451) or restored
+        {   // table: zero (fresh LZ4_initStream, :1443-1451) or restored (the stream's record, or the dictionary's)
             uint4* t4 = reinterpret_cast<uint4*>(table);
-            if (st) {
-                offset = st->offset; dict_len = st->dict_len;
-                dict_end = st->dict_buf + dict_len;
+            if (init) {
+                offset = init->offset; dict_len = init->dict_len;
+                dict_end = init->dict_buf + dict_len;
                 if (kCompact) {         // positions within reach become rel = pos - tbase + 1 in the lower half, the rest is dropped
                     // (d == 65535 only for the zero entries of a stream that has not compressed anything yet: position 0 == offset)
                     tbase = offset - (kEpoch - 1);
                     for (int k = 0; k < kHashEntries / 32; k++) {
                         const int i = (int)lane + 32 * k;
-                        const uint32_t d = st->table[i] - tbase;
+                        const uint32_t d = init->table[i] - tbase;
                         const uint32_t rel = (d <= kEpoch - 1) ? d + 1u : 0u;
                         t16[i] = (uint16_t)rel;
                         const uint32_t hi = __ballot_sync(kFull, (rel >> 16) != 0);
                         if (lane == 0) tfl[k] = hi;
                     }
                 } else {
-                    const uint4* g4 = reinterpret_cast<const uint4*>(st->table);
+                    const uint4* g4 = reinterpret_cast<const uint4*>(init->table);
                     for (int i = lane; i < kHashEntries / 4; i += 32) t4[i] = g4[i];
                 }
             } else if (kCompact) {      // every bucket = stream position 0 (what a zero-filled table means): rel = 65536

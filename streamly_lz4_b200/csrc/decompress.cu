@@ -154,7 +154,7 @@ __device__ void parser_main(const DecompressArgs& a, DQueue* q, uint32_t ring_s)
         const int s = claim_stream(counter);
         if (s >= a.n_streams) break;
         const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
-        const DState* st = a.states ? reinterpret_cast<const DState*>(a.states[s]) : nullptr;
+        const DState* st = a.states ? reinterpret_cast<const DState*>(a.states[s]) : a.dict_state;   // the stream's record, or the dictionary's
         uint32_t dict_len = st ? st->prev_len : 0u;
         for (int b = b0; b < b1; b++) {
             const BlockGeom g = block_geom(a, b);
@@ -288,7 +288,7 @@ __device__ void copier_main(const DecompressArgs& a, DQueue* q, uint32_t in_s, u
             pub = 0;
             gbase = g.payload - (reinterpret_cast<uintptr_t>(g.payload) & 15);
             if (cf & kStreamBegin) {
-                const DState* st = a.states ? reinterpret_cast<const DState*>(a.states[q->stream[b]]) : nullptr;
+                const DState* st = a.states ? reinterpret_cast<const DState*>(a.states[q->stream[b]]) : a.dict_state;
                 C.dict_end = nullptr; C.dict_len = 0; last_out = nullptr; last_len = 0;
                 if (st && st->prev_len) { C.dict_len = st->prev_len; C.dict_end = st->tail + 65536; }
             }

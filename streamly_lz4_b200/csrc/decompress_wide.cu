@@ -378,11 +378,12 @@ __device__ void wdispatch_main(const DecompressArgs& a, WCtl* ctl, uint32_t out_
     for (int s = blockIdx.x; s < a.n_streams; s += gridDim.x) {
         const int b0 = stream_begin(a, s), b1 = stream_end(a, s, b0);
         DState* st = a.states ? reinterpret_cast<DState*>(a.states[s]) : nullptr;
+        const DState* init = a.states ? st : a.dict_state;              // what the stream starts from: its record, or the dictionary's
         // ---- open the stream: the ring restarts at kSeedBase with the kept tail of the previous call as dictionary
         WSTAT(0)
         D.drain();
         uint32_t dict_len = 0, kept = 0;
-        if (st && st->prev_len) { dict_len = st->prev_len; kept = st->kept; wseed(out_s, st->tail + 65536 - kept, kept); }
+        if (init && init->prev_len) { dict_len = init->prev_len; kept = init->kept; wseed(out_s, init->tail + 65536 - kept, kept); }
         else wseed(out_s, nullptr, 0u);
         uint32_t base = kSeedBase, valid_lo = kSeedBase - kept;
         D.fpos = kSeedBase;
@@ -439,9 +440,9 @@ __device__ void wdispatch_main(const DecompressArgs& a, WCtl* ctl, uint32_t out_
                         if (last_out) {
                             dict_len = (uint32_t)last_len; kept = dict_len < 65536u ? dict_len : 65536u;
                             wseed(out_s, last_out + last_len - kept, kept);
-                        } else if (st && st->prev_len) {
-                            dict_len = st->prev_len; kept = st->kept;
-                            wseed(out_s, st->tail + 65536 - kept, kept);
+                        } else if (init && init->prev_len) {
+                            dict_len = init->prev_len; kept = init->kept;
+                            wseed(out_s, init->tail + 65536 - kept, kept);
                         } else wseed(out_s, nullptr, 0u);
                         base = kSeedBase; valid_lo = kSeedBase - kept; D.fpos = kSeedBase;
                         #pragma unroll

@@ -18,6 +18,9 @@ struct CompressArgs {
     // segment; *arrived segments of seg_bytes (a multiple of 128) bytes of EVERY block of the launch have landed.
     // Block starts must be 128-byte aligned.  busy_cycles[0] += finder cycles net of waiting, [1] += bytes.
     const uint32_t* arrived; int seg_bytes; unsigned long long* busy_cycles;
+    // dictionary (NULL: none): a stream without a record of its own (states == NULL) starts from this read-only state,
+    // written by launch_load_dict; shared by every stream of the launch and never written
+    const CState* dict_state;
 };
 
 struct DecompressArgs {
@@ -36,6 +39,9 @@ struct DecompressArgs {
     // mirrored launch (NULL: off; independent blocks only): block i's output is ALSO stored at host_dst + dst_off[i], page-locked
     // host memory with host_dst congruent to dst modulo 16
     uint8_t* host_dst;
+    // dictionary (NULL: none): a stream without a record of its own (states == NULL) starts with this read-only
+    // previous output (launch_load_dict); never written
+    const DState* dict_state;
 };
 
 // Blocks [b0, b1) of stream s of a launch: its run in stream_first, or in independent mode the one block first_block + s.
@@ -89,6 +95,10 @@ cudaError_t device_sm_count(int* out);
 cudaError_t launch_compact(const CompactArgs& a, cudaStream_t stream);
 cudaError_t launch_reframe(const uint8_t* buf, int64_t len, int header, int has_end_mark,
                            int64_t* block_off, int32_t* block_len, int64_t max_blocks, int64_t* result, cudaStream_t stream);
+// LZ4_loadDict on the device: d_cstate (if not NULL) becomes the state LZ4_loadDict(dict, len) leaves in a fresh stream
+// (its dict_buf points into dict, which must outlive every use of the record), d_dstate (if not NULL) the decode state
+// LZ4_setStreamDecode(dict, len) sets up (the last 64 KiB copied in).  len >= 0.
+cudaError_t launch_load_dict(const uint8_t* dict, int64_t len, CState* d_cstate, DState* d_dstate, cudaStream_t stream);
 cudaError_t launch_xxh32(const uint8_t* buf, const int64_t* off, const int32_t* len, int n, uint32_t seed, uint32_t* out, cudaStream_t stream);
 int kernel_launches_per_compress();
 int kernel_launches_per_decompress();
