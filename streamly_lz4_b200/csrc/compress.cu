@@ -619,6 +619,69 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
             return true;
         };
 
+        // A run of re-tests in the classic geometry without a dictionary (dict_len == 0, so the only lower bound on a
+        // candidate is S and every candidate that passes it lies in the block): the same steps as retest_probe + push,
+        // arranged so that one sequence costs one dependent chain and one branch.  Inside the inner loop ip stays below
+        // both the next ring window (no move_window) and mlimit - 31 (32-byte compares need no cap); the hash-ring and
+        // byte loads of the next sequence are issued as soon as this one's length is known, ahead of the descriptor
+        // store; the queue is flushed when the loop leaves it full.  Anything else -- a miss, a match of 32+ bytes, the
+        // window edge, a full queue -- leaves the inner loop and is settled here.
+        // Returns 0: the re-test at ip missed (ip unchanged), 1: ip reached mflimit, 2: ip is within 32 bytes of
+        // matchlimit (the caller finishes the run with retest_probe).
+        auto retest_run = [&](int& ip) -> int {
+            const uint32_t gl_s = g32 + lane - S;                   // ring position of byte lane of candidate index cand: gl_s + cand
+            const uint8_t* const src_s = src + lane - S;            // its global address: src_s + cand (cand >= S)
+            for (;;) {
+                if (ip >= trigger) move_window(ip);
+                if (ip > mlimit - 32) return 2;
+                const int lim = min(trigger, mlimit - 31);
+                const uint32_t ring_lo = S + (uint32_t)lo_pos;         // candidates from here on are in the ring
+                const uint32_t slot0 = out.slot_s, slot_end = slot0 + 16u * (uint32_t)(kQueueDepth - out.fill);
+                uint32_t slot = slot0;
+                const uint32_t ap = g32 + (uint32_t)ip;
+                uint32_t cur = S + (uint32_t)ip;
+                uint32_t h = hash_at(ap), h2 = hash_at(ap - 2), mine = ring8(ap + lane);
+                uint32_t m, ne;
+                bool near, hit;
+                do {
+                    t_put(h2, cur - 2);                                                              // :1146
+                    m = t_swap(h, cur);                                                              // :1185
+                    near = (m >= S) && (m + kMaxDistance >= cur);                                    // :1187-1188
+                    // ring bytes unless the candidate is older than the ring (a far miss compares garbage: near decides)
+                    uint32_t theirs = ring8(gl_s + m);
+                    if (near && m < ring_lo) theirs = __ldg(src_s + m);
+                    ne = __ballot_sync(kFull, mine != theirs);
+                    const uint32_t L = (uint32_t)__ffs(ne) - 1u;
+                    hit = near && L - 4u < 28u;                                                      // 4 <= L < 32
+                    // The next sequence's loads.  On the iteration that leaves the loop (a miss, where L may be
+                    // ffs(0) - 1, or ip + L at the window edge) they may read ring bytes past ready_end, including the
+                    // line cp.async is still filling: on purpose -- the addresses are masked into this finder's rings,
+                    // the values are dropped, and the outer loop reloads h / h2 / mine after move_window.
+                    const uint32_t na = g32 + (uint32_t)ip + L;
+                    const uint32_t nh = hash_at(na), nh2 = hash_at(na - 2), nmine = ring8(na + lane);
+                    sts128(slot, (uint32_t)ip, 0u, L - 4, cur - m);      // after a miss: a stale slot past the fill mark
+                    if (hit) { slot += 16; ip += (int)L; cur += L; h = nh; h2 = nh2; mine = nmine; }
+                } while (hit && ip < lim && slot != slot_end);
+                out.fill += (int)((slot - slot0) >> 4);
+                out.slot_s = slot;
+                anchor = ip;
+                if (!hit) {
+                    // a miss: out of reach, or fewer than 4 equal bytes (4..31 would have been a hit)      :1187-1189
+                    if (!near || ne != 0) return 0;
+                    // 32 equal bytes; cap >= 32 below lim
+                    const uint32_t cap = (uint32_t)(mlimit - ip);
+                    uint32_t L = 32u;
+                    if (cap > 32u) L += count_ahead(ip + 32, src + (m - S) + 32, cap - 32u);
+                    out.push((uint32_t)ip, 0u, L - 4, cur - m, in.block);
+                    ip += (int)L;
+                    anchor = ip;
+                } else if (out.fill == kQueueDepth) {
+                    out.flush(in.block, 0);
+                }
+                if (ip >= mfl) return 1;                                                             // :1143
+            }
+        };
+
         wait_for(128);
         { t_sweep_to(S); uint2 v = ldg_5bytes(src); t_put(hash5(v.x, v.y), S); }    // :924
         __syncwarp();
@@ -632,7 +695,12 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
             if (after_match) {
                 // ---- put(ip-2), re-test ip (cbits/lz4.c:1146, :1159-1196); ip == anchor here.
                 // Loops for as long as a match immediately follows a match.
-                while (retest_probe(ip)) {
+                int run = 2;
+                if constexpr (!kWide && !kCompact) {
+                    if (in.dict_len == 0) run = retest_run(ip);
+                }
+                if (run == 1) goto tail;
+                if (run == 2) while (retest_probe(ip)) {
                     out.push((uint32_t)ip, 0u, mlen - 4, dist, in.block);
                     ip += (int)mlen;
                     anchor = ip;
