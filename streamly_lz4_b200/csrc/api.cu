@@ -586,6 +586,7 @@ int decompress_host(b200lz4_ctx* c, const void* src, int64_t src_bytes,
     if (route.out != DecodeOut::Mirror) mirror_dst = nullptr;
     Range chunks[kMaxChunks];
     const int nchunks = plan_chunks(src_len, n, stream_first, ns, mirror_dst != nullptr, chunks);
+    if (getenv("B200LZ4_DEBUG")) fprintf(stderr, "[b200lz4] decompress: %s output, %d chunks\n", mirror_dst ? "mirror" : "copy", nchunks);
 
     const DescLayout lay(n, n, n, ns + 1, ns, n + nchunks, 0);
     if ((rc = ensure_desc(c, lay))) return rc;
