@@ -63,6 +63,13 @@ extern "C" {
 #define B200LZ4_E_NOMEM  (-3)                 /* host or device allocation failed / dst too small */
 #define B200LZ4_E_BLOCK  (-4)                 /* at least one block failed; see out_len[] */
 #define B200LZ4_E_FRAME  (-5)                 /* re-frame: incomplete block / missing end mark / bad header */
+#define B200LZ4_E_CHECKSUM (-6)               /* LZ4 frame: header, block or content checksum mismatch (per frame) */
+
+/* LZ4 frame options: the FLG bits of the frame format (lz4_Frame_format.md) */
+#define B200LZ4_FRAME_INDEPENDENT      0x20   /* blocks are independent (clear: each block may reference the previous 64 KiB) */
+#define B200LZ4_FRAME_BLOCK_CHECKSUM   0x10   /* XXH32 of every block's data follows it */
+#define B200LZ4_FRAME_CONTENT_SIZE     0x08   /* the header holds the content size */
+#define B200LZ4_FRAME_CONTENT_CHECKSUM 0x04   /* XXH32 of the whole content follows the end mark */
 
 typedef struct b200lz4_ctx b200lz4_ctx;               /* one per (host thread, device) */
 typedef struct b200lz4_cstream b200lz4_cstream;       /* device-resident LZ4_stream_t equivalent (cbits/lz4.h:595-603) */
@@ -335,6 +342,51 @@ int b200lz4_reframe_dev(const void* d_buf, int64_t len, int header_mode, int has
 int b200lz4_xxh32_dev(const void* d_buf, const int64_t* d_off, const int32_t* d_len, int n, uint32_t seed, uint32_t* d_out, void* cuda_stream);
 int b200lz4_xxh32_batch(b200lz4_ctx* ctx, const void* src, int64_t src_bytes, const int64_t* off, const int32_t* len, int n,
                         uint32_t seed, uint32_t* out);
+
+/* ---------------------------------------------------------- LZ4 frames -- */
+/*
+ * Standard LZ4 frames (what the `lz4` tool, LZ4F_compressFrame and lz4.frame write), n at a time: array i <-> frame i.
+ *
+ * b200lz4_frame_bound: the largest frame an n-byte array can become with this block maximum and these flags (header of at
+ * most 15 bytes, per block 4 + its raw bytes + 4 with block checksums, the end mark, 4 with a content checksum); < 0 for
+ * an invalid argument.
+ *
+ * b200lz4_frame_info: parse one frame header on the host (magic, version, reserved bits, block maximum, header checksum).
+ * Returns B200LZ4_OK, B200LZ4_E_FRAME (not a frame header, or one with a dictionary id), B200LZ4_E_CHECKSUM (header
+ * checksum) or B200LZ4_E_ARG (fewer bytes than the header needs).  *content_size = -1 if the header holds none; *flags:
+ * B200LZ4_FRAME_* bits.  Any output pointer may be NULL.
+ *
+ * b200lz4_frame_compress_batch: array i = src[src_off[i] .. +src_len[i]) becomes frame i, cut into blocks of block_max
+ * (65536, 262144, 1048576 or 4194304) bytes.  The blocks are this library's byte-exact LZ4 blocks (independent frames: a
+ * fresh stream per block; linked frames: one stream per frame, the previous block as dictionary), stored raw (size bit 31)
+ * when the payload is not shorter than the raw bytes.  flags: B200LZ4_FRAME_* (content size = the array's length).  Frames
+ * are written back to back: frame i = dst[dst_off[i] .. dst_off[i+1]), out_len[i] = its size; dst_off has n_frames + 1
+ * entries.  dst_cap >= the sum of b200lz4_frame_bound(src_len[i]) is always enough.  Not byte-identical to
+ * LZ4F_compressFrame (its block tables differ below 65 547 bytes), but every frame decoder reads the output.
+ *
+ * b200lz4_frame_decompress_batch: range i = src[src_off[i] .. +src_len[i]) holds exactly one frame; its content goes to
+ * dst[dst_off[i] ..) with capacity dst_cap[i].  out_len[i] = content bytes, or
+ *     B200LZ4_E_FRAME     bad header / reserved bits / dictionary id / block above the maximum / truncation / missing end
+ *                         mark / bytes after the frame / content size mismatch,
+ *     B200LZ4_E_BLOCK     the safe decoder rejected a block,
+ *     B200LZ4_E_CHECKSUM  header, block or content checksum mismatch,
+ *     B200LZ4_E_NOMEM     the content exceeds dst_cap[i].
+ * A failing frame never aborts the batch (the call returns B200LZ4_E_BLOCK then) and leaves its destination untouched,
+ * except with a content checksum mismatch, found after the content was written.  Linked blocks see the last 64 KiB of
+ * decoded data, as upstream's frame decoder does, whatever the sizes of earlier blocks.
+ *
+ * Both calls take host or device pointers for the data and for the descriptor arrays (told apart with
+ * cudaPointerGetAttributes).  Device data never leaves the device; host data is copied in once and out once.
+ */
+int64_t b200lz4_frame_bound(int64_t n, int block_max, int flags);
+int b200lz4_frame_info(const void* buf, int64_t len, int* block_max, int* flags, int64_t* content_size, int* header_len);
+int b200lz4_frame_compress_batch(b200lz4_ctx* ctx, const void* src, int64_t src_bytes,
+                                 const int64_t* src_off, const int32_t* src_len, int n_frames,
+                                 int block_max, int flags, int acceleration,
+                                 void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len);
+int b200lz4_frame_decompress_batch(b200lz4_ctx* ctx, const void* src, int64_t src_bytes,
+                                   const int64_t* src_off, const int32_t* src_len, int n_frames,
+                                   void* dst, const int32_t* dst_cap, const int64_t* dst_off, int32_t* out_len);
 
 /* ------------------------------------------------------ legacy aliases -- */
 /* Same names, signatures and return conventions as the 7 symbols the unmodified reference

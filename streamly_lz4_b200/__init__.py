@@ -9,11 +9,11 @@ from .api import (BlockConfig, BlockSize, FrameConfig, Context, MultiContext, Co
                   default_block_config, default_frame_config, set_block_max_size,
                   set_block_independence, set_frame_end_mark,
                   simple_frame_parser, frame_header, compress_chunks_frame, decompress_chunks_with,
-                  parse_frame_header, write_frame, read_frame, FrameInfo)
+                  parse_frame_header, write_frame, read_frame, FrameInfo, frame_bound, frame_info)
 
 __all__ = ["BlockConfig", "BlockSize", "FrameConfig", "Context", "MultiContext", "CompressStream", "DecompressStream", "LZ4Error",
            "Dictionary", "compress_chunks", "decompress_chunks", "decompress_chunks_raw", "resize_chunks",
            "default_block_config", "default_frame_config", "set_block_max_size",
            "set_block_independence", "set_frame_end_mark",
            "simple_frame_parser", "frame_header", "compress_chunks_frame", "decompress_chunks_with",
-           "parse_frame_header", "write_frame", "read_frame", "FrameInfo"]
+           "parse_frame_header", "write_frame", "read_frame", "FrameInfo", "frame_bound", "frame_info"]

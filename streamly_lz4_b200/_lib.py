@@ -80,6 +80,12 @@ PROTOTYPES = {
     "b200lz4_reframe_dev": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_i64, c_vp, c_vp]),
     "b200lz4_xxh32_dev": (c_int, [c_vp, c_vp, c_vp, c_int, ctypes.c_uint32, c_vp, c_vp]),
     "b200lz4_xxh32_batch": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_int, ctypes.c_uint32, c_vp]),
+    "b200lz4_frame_bound": (c_i64, [c_i64, c_int, c_int]),
+    "b200lz4_frame_info": (c_int, [c_vp, c_i64, ctypes.POINTER(c_int), ctypes.POINTER(c_int), ctypes.POINTER(c_i64),
+                                   ctypes.POINTER(c_int)]),
+    "b200lz4_frame_compress_batch": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_int, c_int, c_int, c_int,
+                                             c_vp, c_i64, c_vp, c_vp]),
+    "b200lz4_frame_decompress_batch": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp]),
     # legacy aliases of the reference's 7 foreign imports (src/Streamly/Internal/LZ4.hs:105-140)
     "LZ4_createStream": (c_vp, []),
     "LZ4_freeStream": (c_int, [c_vp]),

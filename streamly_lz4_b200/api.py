@@ -198,6 +198,75 @@ class Context:
             rc = self.lib.b200lz4_decompress_batch_dict(*args, dictionary.handle)
         return rc, dst_off, out_len
 
+    # ---- LZ4 frames: n arrays <-> n frames in one call -------------------
+    def frame_compress_batch(self, src, src_off, src_len, block_max: int, flags: int = 0, accel: int = 1, dst=None):
+        """Array i = src[src_off[i] : +src_len[i]] becomes frame i (b200lz4_frame_compress_batch).  src / dst: numpy uint8
+        arrays or CUDA uint8 tensors (device pointers; then src_off / src_len may be tensors too).  dst=None: a numpy buffer
+        of frame_bound size.  Returns (rc, dst, dst_off, out_len): frame i = dst[dst_off[i] : dst_off[i + 1]]."""
+        s_ptr, s_size = _buffer(src)
+        offp, _ = _buffer(src_off, np.int64)
+        lenp, _ = _buffer(src_len, np.int32)
+        n = len(src_len)
+        if dst is None:
+            lens = src_len.cpu().numpy() if hasattr(src_len, "cpu") else np.asarray(src_len)
+            dst = np.zeros(max(1, sum(frame_bound(int(x), block_max, flags) for x in lens)), dtype=np.uint8)
+        d_ptr, d_size = _buffer(dst)
+        dst_off = np.zeros(n + 1, dtype=np.int64)
+        out_len = np.zeros(n, dtype=np.int32)
+        rc = self.lib.b200lz4_frame_compress_batch(self.handle, s_ptr, s_size, offp, lenp, n, block_max, flags, accel,
+                                                   d_ptr, d_size, dst_off.ctypes.data, out_len.ctypes.data)
+        return rc, dst, dst_off, out_len
+
+    def frame_decompress_batch(self, src, src_off, src_len, dst, dst_off, dst_cap):
+        """Range i = src[src_off[i] : +src_len[i]] holds one frame; its content goes to dst[dst_off[i] :] with capacity
+        dst_cap[i] (b200lz4_frame_decompress_batch).  Returns (rc, out_len): content bytes per frame, or a negative
+        B200LZ4_E_* code (FRAME -5, BLOCK -4, CHECKSUM -6, NOMEM -3)."""
+        s_ptr, s_size = _buffer(src)
+        d_ptr, _ = _buffer(dst)
+        offp, _ = _buffer(src_off, np.int64)
+        lenp, _ = _buffer(src_len, np.int32)
+        doffp, _ = _buffer(dst_off, np.int64)
+        capp, _ = _buffer(dst_cap, np.int32)
+        n = len(src_len)
+        out_len = np.zeros(n, dtype=np.int32)
+        rc = self.lib.b200lz4_frame_decompress_batch(self.handle, s_ptr, s_size, offp, lenp, n, d_ptr, capp, doffp,
+                                                     out_len.ctypes.data)
+        return rc, out_len
+
+
+FRAME_INDEPENDENT, FRAME_BLOCK_CHECKSUM, FRAME_CONTENT_SIZE, FRAME_CONTENT_CHECKSUM = 0x20, 0x10, 0x08, 0x04
+E_NOMEM, E_BLOCK, E_FRAME, E_CHECKSUM = -3, -4, -5, -6
+
+
+def _buffer(x, dtype=np.uint8):
+    """(pointer, element count) of a numpy array (made contiguous and of `dtype`; kept alive by the caller's reference) or
+    of a CUDA tensor (a device pointer, used as it is)."""
+    if hasattr(x, "data_ptr"):
+        assert x.is_contiguous() and x.element_size() == np.dtype(dtype).itemsize, "tensor must be contiguous and of the right dtype"
+        return x.data_ptr(), x.numel()
+    if not (isinstance(x, np.ndarray) and x.dtype == dtype and x.flags.c_contiguous):
+        raise TypeError(f"expected a contiguous numpy array of {np.dtype(dtype)} or a CUDA tensor")
+    return x.ctypes.data, x.size
+
+
+def frame_bound(n: int, block_max: int, flags: int = 0) -> int:
+    """b200lz4_frame_bound: the largest frame an n-byte array can become."""
+    r = int(_lib.load().b200lz4_frame_bound(n, block_max, flags))
+    if r < 0:
+        raise LZ4Error("b200lz4_frame_bound: " + _lib.last_error())
+    return r
+
+
+def frame_info(buf: bytes):
+    """b200lz4_frame_info: (block_max, flags, content_size or None, header_len) of the frame header at the start of buf."""
+    bm, fl, hl = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
+    cs = ctypes.c_int64()
+    b = bytes(buf)
+    rc = _lib.load().b200lz4_frame_info(b, len(b), ctypes.byref(bm), ctypes.byref(fl), ctypes.byref(cs), ctypes.byref(hl))
+    if rc != 0:
+        raise LZ4Error(f"b200lz4_frame_info ({rc}): " + _lib.last_error())
+    return bm.value, fl.value, (None if cs.value < 0 else cs.value), hl.value
+
 
 class Dictionary:
     """A dictionary loaded on one Context's device (b200lz4_dict).  Only the last 64 KiB reach the codec; `len(d)` is the

@@ -79,6 +79,8 @@ struct b200lz4_ctx {
     Scratch* scratch = nullptr;                     // kMaxGroups records: one work counter per in-flight kernel
     Buf<false> d_src, d_slots, d_out, d_desc, d_wide;   // d_wide: descriptor rings of decompress_kernel_wide (one slice per chunk)
     Buf<true> h_desc;
+    Buf<false> d_fframe, d_fblock, d_fstage;        // frame calls: per-frame and per-block descriptors, staged stored blocks
+    Buf<true> h_fframe, h_fout;                     // ... their host side, and decoded content on its way to a host destination
     CallEvents ev;
     // streamed compress call (compress_host_streamed): per-group arrival flags + finder cycle counters in HBM, the
     // constants the copy stream writes into the flags, and what earlier calls measured (the copy schedule is tuned by it)
@@ -844,6 +846,7 @@ void b200lz4_ctx_destroy(b200lz4_ctx* c)
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     c->d_src.release(); c->d_slots.release(); c->d_out.release(); c->d_desc.release(); c->d_wide.release(); c->h_desc.release();
+    c->d_fframe.release(); c->d_fblock.release(); c->d_fstage.release(); c->h_fframe.release(); c->h_fout.release();
     if (c->scratch) cudaFree(c->scratch);
     if (c->d_flags) cudaFree(c->d_flags);
     if (c->h_const) cudaFreeHost(c->h_const);
@@ -1438,6 +1441,368 @@ int b200lz4_reframe_dev(const void* d_buf, int64_t len, int header_mode, int has
     CU(launch_reframe(static_cast<const uint8_t*>(d_buf), len, header_mode, has_end_mark, d_block_off, d_block_len, max_blocks,
                       d_result, static_cast<cudaStream_t>(cuda_stream)));
     return 0;
+}
+
+}  // extern "C"
+
+// ---- LZ4 frames ------------------------------------------------------------------------------------------------------
+// Both frame calls run on the ctx's H2D stream only: descriptors and (host) data go in once, the kernels of frame.cu and
+// the codec kernels run in order, results and (host) output come back once.  One small read-back in the middle tells the
+// host how many blocks there are (decode) or how large the frames are (encode).
+namespace {
+
+bool on_device(const void* p)
+{
+    cudaPointerAttributes pa{};
+    if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    return pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged;
+}
+
+// Bump allocation of 16-byte aligned arrays inside one buffer: a first pass with base NULL measures, the second carves.
+struct Carve {
+    uint8_t* base; size_t at = 0;
+    template <class T> T* take(int64_t count) { at = (at + 15) & ~size_t(15); T* p = reinterpret_cast<T*>(base + at); at += sizeof(T) * (size_t)std::max<int64_t>(count, 0); return p; }
+};
+
+int frame_class(int block_max)
+{
+    for (int k = 0; k < 4; k++) if (block_max == (65536 << (2 * k))) return k;
+    return -1;
+}
+
+// XXH32 of the frame descriptor (fewer than 16 bytes), as frame.cu's xxh32_short
+uint32_t xxh32_short_host(const uint8_t* p, int n)
+{
+    auto rotl = [](uint32_t x, int r) { return (x << r) | (x >> (32 - r)); };
+    uint32_t h = 374761393u + (uint32_t)n;
+    int at = 0;
+    for (; at + 4 <= n; at += 4) h = rotl(h + (uint32_t)le32(p + at) * 3266489917u, 17) * 668265263u;
+    for (; at < n; at++) h = rotl(h + p[at] * 374761393u, 11) * 2654435761u;
+    h ^= h >> 15; h *= 2246822519u; h ^= h >> 13; h *= 3266489917u; h ^= h >> 16;
+    return h;
+}
+
+struct FrameTimer {         // the call's device timeline, as finish_call records it for the block calls
+    b200lz4_ctx* c;
+    int done()
+    {
+        CU(cudaEventSynchronize(c->ev.d1));
+        cudaEventElapsedTime(&c->t_h2d, c->ev.start, c->ev.h2d_end);
+        cudaEventElapsedTime(&c->t_kernel, c->ev.k0, c->ev.k[0]);
+        cudaEventElapsedTime(&c->t_d2h, c->ev.d0, c->ev.d1);
+        return 0;
+    }
+};
+
+int frame_decompress(b200lz4_ctx* c, const void* src, int64_t src_bytes, const int64_t* src_off, const int32_t* src_len, int n,
+                     void* dst, const int32_t* dst_cap, const int64_t* dst_off, int32_t* out_len)
+{
+    if (!c) return fail(B200LZ4_E_ARG, "ctx is NULL");
+    if (n < 0 || src_bytes < 0 || (n > 0 && (!src || !src_off || !src_len || !dst || !dst_cap || !dst_off || !out_len)))
+        return fail(B200LZ4_E_ARG, "NULL argument or negative count");
+    if (n == 0) return 0;
+    CU(cudaSetDevice(c->device));
+    const bool src_dev = on_device(src), dst_dev = on_device(dst);
+    cudaStream_t st = c->stream;
+    int rc;
+    // host side: the caller's descriptors (from host or device memory), then what comes back
+    auto host_layout = [&](Carve& h) {
+        struct { int64_t* src_off; int32_t* src_len; int32_t* cap; int64_t* dst_off; int32_t* result; long long* totals; int64_t* fout; } v;
+        v.src_off = h.take<int64_t>(n); v.src_len = h.take<int32_t>(n); v.cap = h.take<int32_t>(n); v.dst_off = h.take<int64_t>(n);
+        v.result = h.take<int32_t>(n); v.totals = h.take<long long>(kFrameTotals); v.fout = h.take<int64_t>(n + 1);
+        return v;
+    };
+    Carve hm{nullptr}; host_layout(hm);
+    if ((rc = c->h_fframe.ensure(hm.at))) return rc;
+    Carve hc{static_cast<uint8_t*>(c->h_fframe.p)};
+    const auto h = host_layout(hc);
+    CU(cudaMemcpy(h.src_off, src_off, sizeof(int64_t) * n, cudaMemcpyDefault));
+    CU(cudaMemcpy(h.src_len, src_len, sizeof(int32_t) * n, cudaMemcpyDefault));
+    CU(cudaMemcpy(h.cap, dst_cap, sizeof(int32_t) * n, cudaMemcpyDefault));
+    CU(cudaMemcpy(h.dst_off, dst_off, sizeof(int64_t) * n, cudaMemcpyDefault));
+    const Verdict v = check_blocks(h.src_off, h.src_len, n, src_bytes);
+    if (v.code) return fail(v);
+    for (int i = 0; i < n; i++) if (h.cap[i] < 0 || h.dst_off[i] < 0) return fail(B200LZ4_E_ARG, "negative dst_cap or dst_off");
+
+    // device side, per frame
+    FrameDecodeArgs a{};
+    auto frame_layout = [&](Carve& d) {
+        a.src_off = d.take<int64_t>(n); a.src_len = d.take<int32_t>(n); a.dst_cap = d.take<int32_t>(n);
+        a.rec = d.take<FrameRec>(n); a.totals = d.take<long long>(kFrameTotals);
+        a.content = d.take<int32_t>(n); a.cclen = d.take<int32_t>(n); a.ccsum_got = d.take<uint32_t>(n); a.result = d.take<int32_t>(n);
+        return std::make_pair(d.take<int64_t>(n), d.take<int64_t>(n + 1));     // the caller's dst_off, the packed content offsets
+    };
+    Carve dm{nullptr}; frame_layout(dm);
+    if ((rc = c->d_fframe.ensure(dm.at))) return rc;
+    Carve dc{static_cast<uint8_t*>(c->d_fframe.p)};
+    const auto fb = frame_layout(dc);
+    int64_t* d_dst_off = fb.first;
+    int64_t* d_fout = fb.second;
+    a.n = n;
+    if (!src_dev && (rc = c->d_src.ensure((size_t)src_bytes + 64))) return rc;
+    a.base = src_dev ? static_cast<const uint8_t*>(src) : static_cast<const uint8_t*>(c->d_src.p);
+
+    CU(cudaEventRecord(c->ev.start, st));
+    CU(cudaMemcpyAsync(const_cast<int64_t*>(a.src_off), h.src_off, sizeof(int64_t) * n, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int32_t*>(a.src_len), h.src_len, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int32_t*>(a.dst_cap), h.cap, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_dst_off, h.dst_off, sizeof(int64_t) * n, cudaMemcpyHostToDevice, st));
+    if (!src_dev && src_bytes) CU(cudaMemcpyAsync(c->d_src.p, src, (size_t)src_bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(c->ev.h2d_end, st));
+    CU(cudaEventRecord(c->ev.k0, st));
+    CU(launch_frame_walk(a, false, st));
+    CU(launch_frame_scan(a, st));
+    c->launches += 2;
+    CU(cudaMemcpyAsync(h.totals, a.totals, sizeof(long long) * kFrameTotals, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    long long T[kFrameTotals];
+    memcpy(T, h.totals, sizeof T);
+    const long long nb_all = T[0] + T[1] + T[2] + T[3];
+    const long long ns_all = T[4] + T[5] + T[6] + T[7] + 4;
+    if (nb_all > INT_MAX / 2) return fail(B200LZ4_E_NOMEM, "too many blocks in one call");
+    const int nb = (int)nb_all;
+
+    // device side, per block
+    auto block_layout = [&](Carve& d) {
+        a.dsrc_off = d.take<int64_t>(nb); a.dsrc_len = d.take<int32_t>(nb); a.slot_off = d.take<int64_t>(nb);
+        a.raw_off = d.take<int64_t>(nb); a.meta = d.take<int32_t>(nb); a.csum_len = d.take<int32_t>(nb);
+        a.csum_exp = d.take<uint32_t>(nb); a.csum_got = d.take<uint32_t>(nb); a.bframe = d.take<int32_t>(nb);
+        a.sf = d.take<int32_t>(ns_all); a.out_len = d.take<int32_t>(nb); a.gout_off = d.take<int64_t>(nb); a.glen = d.take<int32_t>(nb);
+    };
+    Carve bm{nullptr}; block_layout(bm);
+    if ((rc = c->d_fblock.ensure(bm.at))) return rc;
+    Carve bc{static_cast<uint8_t*>(c->d_fblock.p)};
+    block_layout(bc);
+    if ((rc = c->d_fstage.ensure((size_t)T[12] + 64))) return rc;
+    if ((rc = c->d_slots.ensure((size_t)T[13] + 64))) return rc;
+    if (!dst_dev && (rc = c->d_out.ensure((size_t)T[13] + 64))) return rc;
+    a.stage_delta = (long long)(reinterpret_cast<uintptr_t>(c->d_fstage.p) - reinterpret_cast<uintptr_t>(a.base));
+    CU(launch_frame_walk(a, true, st));
+    CU(launch_frame_stage(a, nb, st));
+    c->launches += 2;
+    long long blk0 = 0, str0 = 0;
+    for (int k = 0; k < 4; k++) {          // one decoder launch per block maximum: it is the decoders' capacity
+        const int nbk = (int)T[k], nsk = (int)T[4 + k];
+        if (nbk) {
+            DecompressArgs d{};
+            d.src = a.base; d.src_off = a.dsrc_off + blk0; d.src_len = a.dsrc_len + blk0; d.n_blocks = nbk;
+            d.stream_first = nsk == nbk ? nullptr : a.sf + str0;      // every frame independent: one stream per block
+            d.n_streams = nsk;
+            d.dst = static_cast<uint8_t*>(c->d_slots.p); d.dst_off = a.slot_off + blk0; d.out_len = a.out_len + blk0;
+            d.header = 0; d.max_block = 65536 << (2 * k); d.scratch = c->scratch;
+            if (T[8 + k]) CU(launch_decompress_window(d, st));
+            else {
+                const int wide_ctas = std::min(nsk, kWideMaxCtas);
+                if ((rc = c->d_wide.ensure((size_t)wide_ctas * kWideArenaPerCta))) return rc;
+                d.wide_arena = reinterpret_cast<uint4*>(c->d_wide.p); d.wide_ctas = wide_ctas;
+                CU(launch_decompress(d, st));
+            }
+            c->launches += kernel_launches_per_decompress();
+        }
+        blk0 += nbk; str0 += nsk + 1;
+    }
+    CU(launch_xxh32(a.base, a.raw_off, a.csum_len, nb, 0u, a.csum_got, st));
+    CU(launch_frame_settle(a, st));
+    c->launches += 2;
+    uint8_t* out = dst_dev ? static_cast<uint8_t*>(dst) : static_cast<uint8_t*>(c->d_out.p);
+    const int64_t* fbase = d_dst_off;
+    if (!dst_dev) { CU(launch_scan(a.content, n, 0, d_fout, st)); fbase = d_fout; c->launches += 1; }
+    CU(launch_frame_place(a, nb, fbase, st));
+    CompactArgs g{static_cast<const uint8_t*>(c->d_slots.p), a.slot_off, a.glen, nb, 0, out, a.gout_off, nullptr, nullptr};
+    CU(launch_gather(g, st));
+    CU(launch_xxh32(out, fbase, a.cclen, n, 0u, a.ccsum_got, st));
+    CU(launch_frame_verdict(a, st));
+    c->launches += 4;
+    CU(cudaEventRecord(c->ev.k[0], st));
+    CU(cudaEventRecord(c->ev.d0, st));
+    CU(cudaMemcpyAsync(h.result, a.result, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
+    if (!dst_dev) {
+        CU(cudaMemcpyAsync(h.fout, d_fout, sizeof(int64_t) * (n + 1), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        const int64_t total = h.fout[n];
+        if ((rc = c->h_fout.ensure((size_t)total + 64))) return rc;
+        if (total) CU(cudaMemcpyAsync(c->h_fout.p, out, (size_t)total, cudaMemcpyDeviceToHost, st));
+    }
+    CU(cudaEventRecord(c->ev.d1, st));
+    if ((rc = FrameTimer{c}.done())) return rc;
+    if (!dst_dev) {
+        const uint8_t* hp = static_cast<const uint8_t*>(c->h_fout.p);
+        for (int i = 0; i < n; i++)         // what the gather wrote (a content checksum mismatch is found after it)
+            if (h.fout[i + 1] > h.fout[i]) memcpy(static_cast<uint8_t*>(dst) + h.dst_off[i], hp + h.fout[i], (size_t)(h.fout[i + 1] - h.fout[i]));
+    }
+    CU(cudaMemcpy(out_len, h.result, sizeof(int32_t) * n, cudaMemcpyDefault));
+    for (int i = 0; i < n; i++)
+        if (h.result[i] < 0) return fail(B200LZ4_E_BLOCK, "frame " + std::to_string(i) + " failed to decompress (" + std::to_string(h.result[i]) + ")");
+    return 0;
+}
+
+int frame_compress(b200lz4_ctx* c, const void* src, int64_t src_bytes, const int64_t* src_off, const int32_t* src_len, int n,
+                   int block_max, int flags, int accel, void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
+{
+    if (!c) return fail(B200LZ4_E_ARG, "ctx is NULL");
+    const int cls = frame_class(block_max);
+    if (cls < 0) return fail(B200LZ4_E_ARG, "block_max must be 65536, 262144, 1048576 or 4194304");
+    if (flags & ~0x3C) return fail(B200LZ4_E_ARG, "unknown frame flags");
+    if (n < 0 || src_bytes < 0 || (n > 0 && (!src || !src_off || !src_len || !dst || !dst_off || !out_len)))
+        return fail(B200LZ4_E_ARG, "NULL argument or negative count");
+    if (n == 0) { const int64_t zero = 0; if (dst_off) CU(cudaMemcpy(dst_off, &zero, sizeof zero, cudaMemcpyDefault)); return 0; }
+    CU(cudaSetDevice(c->device));
+    const bool src_dev = on_device(src), dst_dev = on_device(dst);
+    const bool linked = !(flags & B200LZ4_FRAME_INDEPENDENT);
+    cudaStream_t st = c->stream;
+    int rc;
+    std::vector<int64_t> h_off(n);
+    std::vector<int32_t> h_len(n);
+    CU(cudaMemcpy(h_off.data(), src_off, sizeof(int64_t) * n, cudaMemcpyDefault));
+    CU(cudaMemcpy(h_len.data(), src_len, sizeof(int32_t) * n, cudaMemcpyDefault));
+    const Verdict v = check_blocks(h_off.data(), h_len.data(), n, src_bytes);
+    if (v.code) return fail(v);
+    // the block split, as LZ4F_compressFrame cuts its input
+    int64_t nb64 = 0;
+    for (int i = 0; i < n; i++) nb64 += (h_len[i] + (int64_t)block_max - 1) / block_max;
+    if (nb64 > INT_MAX / 2) return fail(B200LZ4_E_NOMEM, "too many blocks in one call");
+    const int nb = (int)nb64;
+    FrameEncodeArgs a{};
+    int32_t* h_first = nullptr; int64_t* h_boff = nullptr; int32_t* h_blen = nullptr; int32_t* h_bframe = nullptr;
+    int64_t* h_slot = nullptr; int32_t* h_sf = nullptr; int64_t* h_foff = nullptr; int32_t* h_fsize = nullptr;
+    int32_t* d_sf = nullptr;
+    auto host_layout = [&](Carve& h) {
+        h_first = h.take<int32_t>(n + 1); h_boff = h.take<int64_t>(nb); h_blen = h.take<int32_t>(nb); h_bframe = h.take<int32_t>(nb);
+        h_slot = h.take<int64_t>(nb); h_sf = h.take<int32_t>(n + 1); h_foff = h.take<int64_t>(n + 1); h_fsize = h.take<int32_t>(n);
+    };
+    auto device_layout = [&](Carve& d) {
+        a.src_off = d.take<int64_t>(n); a.src_len = d.take<int32_t>(n); a.frame_first = d.take<int32_t>(n + 1);
+        a.blk_off = d.take<int64_t>(nb); a.blk_len = d.take<int32_t>(nb); a.blk_frame = d.take<int32_t>(nb);
+        a.slot_off = d.take<int64_t>(nb); d_sf = d.take<int32_t>(n + 1);
+        a.pay_len = d.take<int32_t>(nb); a.blk_at = d.take<int64_t>(nb); a.fsize = d.take<int32_t>(n); a.foff = d.take<int64_t>(n + 1);
+        a.csum_off = d.take<int64_t>(nb); a.csum_len = d.take<int32_t>(nb); a.bsum = d.take<uint32_t>(nb);
+        a.csum_content = d.take<uint32_t>(n);
+    };
+    Carve hm{nullptr}; host_layout(hm);
+    Carve dm{nullptr}; device_layout(dm);
+    if ((rc = c->h_fframe.ensure(hm.at))) return rc;
+    if ((rc = c->d_fframe.ensure(dm.at))) return rc;
+    Carve hc{static_cast<uint8_t*>(c->h_fframe.p)}; host_layout(hc);
+    Carve dc{static_cast<uint8_t*>(c->d_fframe.p)}; device_layout(dc);
+    int g = 0, ns = 0;
+    int64_t slots = 0;
+    for (int i = 0; i < n; i++) {
+        h_first[i] = g;
+        if (h_len[i] > 0) h_sf[ns++] = g;
+        for (int64_t at = 0; at < h_len[i]; at += block_max, g++) {
+            h_boff[g] = h_off[i] + at; h_blen[g] = (int32_t)std::min<int64_t>(block_max, h_len[i] - at); h_bframe[g] = i;
+            h_slot[g] = slots; slots += compress_slot(compress_cap(h_blen[g], 0));
+        }
+    }
+    h_first[n] = g; h_sf[ns] = g;
+    if (!src_dev && (rc = c->d_src.ensure((size_t)src_bytes + 64))) return rc;
+    if ((rc = c->d_slots.ensure((size_t)slots + 64))) return rc;
+    a.src = src_dev ? static_cast<const uint8_t*>(src) : static_cast<const uint8_t*>(c->d_src.p);
+    a.n = n; a.flags = flags; a.cls = cls; a.slots = static_cast<const uint8_t*>(c->d_slots.p);
+
+    CU(cudaEventRecord(c->ev.start, st));
+    CU(cudaMemcpyAsync(const_cast<int64_t*>(a.src_off), h_off.data(), sizeof(int64_t) * n, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int32_t*>(a.src_len), h_len.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int32_t*>(a.frame_first), h_first, sizeof(int32_t) * (n + 1), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int64_t*>(a.blk_off), h_boff, sizeof(int64_t) * nb, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int32_t*>(a.blk_len), h_blen, sizeof(int32_t) * nb, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int32_t*>(a.blk_frame), h_bframe, sizeof(int32_t) * nb, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(const_cast<int64_t*>(a.slot_off), h_slot, sizeof(int64_t) * nb, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_sf, h_sf, sizeof(int32_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+    if (!src_dev && src_bytes) CU(cudaMemcpyAsync(c->d_src.p, src, (size_t)src_bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(c->ev.h2d_end, st));
+    CU(cudaEventRecord(c->ev.k0, st));
+    if (nb) {
+        CompressArgs ca{};
+        ca.src = a.src; ca.src_off = a.blk_off; ca.src_len = a.blk_len; ca.n_blocks = nb;
+        ca.stream_first = linked ? d_sf : nullptr; ca.n_streams = linked ? ns : nb;
+        ca.dst = static_cast<uint8_t*>(c->d_slots.p); ca.dst_off = a.slot_off; ca.out_len = const_cast<int32_t*>(a.pay_len);
+        ca.accel = accel; ca.header = 0; ca.scratch = c->scratch;
+        CU(launch_compress(ca, st));
+        c->launches += kernel_launches_per_compress();
+    }
+    CU(launch_frame_csize(a, st));
+    CU(launch_scan(a.fsize, n, 0, const_cast<int64_t*>(a.foff), st));
+    c->launches += 2;
+    CU(cudaMemcpyAsync(h_foff, a.foff, sizeof(int64_t) * (n + 1), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_fsize, a.fsize, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const int64_t total = h_foff[n];
+    if (total > dst_cap) return fail(B200LZ4_E_NOMEM, "dst_cap too small: need " + std::to_string(total));
+    if (!dst_dev && (rc = c->d_out.ensure((size_t)total + 64))) return rc;
+    a.out = dst_dev ? static_cast<uint8_t*>(dst) : static_cast<uint8_t*>(c->d_out.p);
+    CU(launch_frame_cpack(a, nb, st));
+    c->launches += 1;
+    if (flags & B200LZ4_FRAME_BLOCK_CHECKSUM) { CU(launch_xxh32(a.out, a.csum_off, a.csum_len, nb, 0u, const_cast<uint32_t*>(a.bsum), st)); c->launches += 1; }
+    if (flags & B200LZ4_FRAME_CONTENT_CHECKSUM) { CU(launch_xxh32(a.src, a.src_off, a.src_len, n, 0u, const_cast<uint32_t*>(a.csum_content), st)); c->launches += 1; }
+    CU(launch_frame_cfinish(a, nb, st));
+    c->launches += 1;
+    CU(cudaEventRecord(c->ev.k[0], st));
+    CU(cudaEventRecord(c->ev.d0, st));
+    if (!dst_dev && total) CU(cudaMemcpyAsync(dst, a.out, (size_t)total, cudaMemcpyDeviceToHost, st));
+    CU(cudaEventRecord(c->ev.d1, st));
+    if ((rc = FrameTimer{c}.done())) return rc;
+    CU(cudaMemcpy(dst_off, h_foff, sizeof(int64_t) * (n + 1), cudaMemcpyDefault));
+    CU(cudaMemcpy(out_len, h_fsize, sizeof(int32_t) * n, cudaMemcpyDefault));
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int64_t b200lz4_frame_bound(int64_t n, int block_max, int flags)
+{
+    if (n < 0 || frame_class(block_max) < 0 || (flags & ~0x3C)) return fail(B200LZ4_E_ARG, "bad argument");
+    const int64_t blocks = (n + block_max - 1) / block_max;
+    return 7 + ((flags & B200LZ4_FRAME_CONTENT_SIZE) ? 8 : 0) + blocks * (4 + ((flags & B200LZ4_FRAME_BLOCK_CHECKSUM) ? 4 : 0)) + n
+           + 4 + ((flags & B200LZ4_FRAME_CONTENT_CHECKSUM) ? 4 : 0);
+}
+
+int b200lz4_frame_info(const void* buf, int64_t len, int* block_max, int* flags, int64_t* content_size, int* header_len)
+{
+    const uint8_t* p = static_cast<const uint8_t*>(buf);
+    if (!p || len < 7) return fail(B200LZ4_E_ARG, "fewer bytes than a frame header");
+    const int flg = p[4], bd = p[5];
+    if ((uint32_t)le32(p) != 0x184D2204u) return fail(B200LZ4_E_FRAME, "bad magic number");
+    if ((flg >> 6) != 1) return fail(B200LZ4_E_FRAME, "frame version is not 01");
+    if ((flg & 0x02) || (bd & 0x8F)) return fail(B200LZ4_E_FRAME, "reserved bits are set");
+    if (flg & 0x01) return fail(B200LZ4_E_FRAME, "frames with a dictionary id are not supported");
+    if (((bd >> 4) & 7) < 4) return fail(B200LZ4_E_FRAME, "unknown block maximum");
+    int at = 6;
+    int64_t cs = -1;
+    if (flg & 0x08) {
+        if (len < 15) return fail(B200LZ4_E_ARG, "fewer bytes than a frame header");
+        uint64_t x = 0;
+        for (int k = 7; k >= 0; k--) x = (x << 8) | p[6 + k];
+        cs = x > (uint64_t)INT64_MAX ? INT64_MAX : (int64_t)x;
+        at = 14;
+    }
+    if (p[at] != ((xxh32_short_host(p + 4, at - 4) >> 8) & 0xFF)) return fail(B200LZ4_E_CHECKSUM, "header checksum mismatch");
+    if (block_max) *block_max = 65536 << (2 * (((bd >> 4) & 7) - 4));
+    if (flags) *flags = flg & 0x3C;
+    if (content_size) *content_size = cs;
+    if (header_len) *header_len = at + 1;
+    return 0;
+}
+
+int b200lz4_frame_compress_batch(b200lz4_ctx* c, const void* src, int64_t src_bytes,
+                                 const int64_t* src_off, const int32_t* src_len, int n_frames,
+                                 int block_max, int flags, int acceleration,
+                                 void* dst, int64_t dst_cap, int64_t* dst_off, int32_t* out_len)
+{
+    const int rc = frame_compress(c, src, src_bytes, src_off, src_len, n_frames, block_max, flags, acceleration, dst, dst_cap, dst_off, out_len);
+    if (c && rc) c->err = g_err;
+    return rc;
+}
+
+int b200lz4_frame_decompress_batch(b200lz4_ctx* c, const void* src, int64_t src_bytes,
+                                   const int64_t* src_off, const int32_t* src_len, int n_frames,
+                                   void* dst, const int32_t* dst_cap, const int64_t* dst_off, int32_t* out_len)
+{
+    const int rc = frame_decompress(c, src, src_bytes, src_off, src_len, n_frames, dst, dst_cap, dst_off, out_len);
+    if (c && rc) c->err = g_err;
+    return rc;
 }
 
 // ------------------------------------------------------------ legacy aliases

@@ -125,6 +125,21 @@ cudaError_t launch_compact(const CompactArgs& a, cudaStream_t stream)
     return cudaGetLastError();
 }
 
+cudaError_t launch_scan(const int32_t* len, int n, int header, int64_t* out_off, cudaStream_t stream)
+{
+    scan_kernel<<<1, kScanThreads, 0, stream>>>(len, n, header, out_off, nullptr, nullptr);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_gather(const CompactArgs& a, cudaStream_t stream)
+{
+    if (a.n_blocks <= 0) return cudaSuccess;
+    int sm_count = 0;
+    cudaError_t e = device_sm_count(&sm_count); if (e != cudaSuccess) return e;
+    gather_kernel<<<a.n_blocks < sm_count * 8 ? a.n_blocks : sm_count * 8, kGatherThreads, 0, stream>>>(a);
+    return cudaGetLastError();
+}
+
 // Loads the compaction kernels now (CUDA loads a kernel lazily at its first launch, which can wait for running kernels
 // to end -- the streamed call must never launch anything for the first time while its finders wait for input).
 cudaError_t preload_compact_kernels()

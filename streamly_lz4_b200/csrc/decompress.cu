@@ -143,6 +143,7 @@ struct Parser {
     }
 };
 
+template <bool kWindow>
 __device__ void parser_main(const DecompressArgs& a, DQueue* q, uint32_t ring_s)
 {
     uint32_t* counter = &a.scratch->work_counter[2];
@@ -172,7 +173,8 @@ __device__ void parser_main(const DecompressArgs& a, DQueue* q, uint32_t ring_s)
                 r = parse_block(P, skew, g.comp_len, g.cap, dict_len);
             }
             P.publish(kEndBlock | (b == b1 - 1 ? kStreamEnd : 0), r, 0);
-            if (r > 0) dict_len = (uint32_t)r;                         // cbits/lz4.c:2353-2355
+            if (kWindow) { if (r > 0) dict_len = min(65536u, dict_len + (uint32_t)r); }   // the last 64 KiB of the stream's output
+            else if (r > 0) dict_len = (uint32_t)r;                    // cbits/lz4.c:2353-2355
         }
     }
     P.publish(kTerminate, 0, 0);
@@ -243,7 +245,7 @@ struct Copier {
 // host sends their output home segment by segment while they are still being decoded.  Whenever a block's flushed
 // prefix crosses a segment boundary the copier counts it in seg_count[s]; the block that completes segment s for the
 // whole launch raises host_ready[s] (page-locked host memory the calling thread polls).
-template <bool kPublish, bool kMirror>
+template <bool kPublish, bool kMirror, bool kWindow>
 __device__ void copier_main(const DecompressArgs& a, DQueue* q, uint32_t in_s, uint32_t out_s)
 {
     const uint32_t lane = lane_id();
@@ -433,7 +435,11 @@ __device__ void copier_main(const DecompressArgs& a, DQueue* q, uint32_t in_s, u
             if (result >= 0 && dst) { C.template flush<kMirror>(C.op, true); __syncwarp(); }
             if (kPublish) publish(a.n_segs);           // the block is over (short, failed or complete): nothing more will come
             if (lane == 0) a.out_len[blk] = result;
-            if (result > 0) { C.dict_end = dst + result; C.dict_len = (uint32_t)result; last_out = dst; last_len = result; }   // cbits/lz4.c:2353-2355
+            if (kWindow) {                                 // the next block starts where this one ended; its dictionary is the
+                if (!(cf & kStreamEnd) && lane == 0)       // stream's last min(64 KiB, bytes so far) bytes, right below it
+                    const_cast<int64_t*>(a.dst_off)[blk + 1] = a.dst_off[blk] + (result > 0 ? result : 0);
+                if (result > 0) { C.dict_end = dst + result; C.dict_len = min(65536u, C.dict_len + (uint32_t)result); }
+            } else if (result > 0) { C.dict_end = dst + result; C.dict_len = (uint32_t)result; last_out = dst; last_len = result; }   // cbits/lz4.c:2353-2355
             if ((cf & kStreamEnd) && a.states && last_out) {   // keep the reachable tail of the last output for the next call
                 DState* st = reinterpret_cast<DState*>(a.states[stream]);
                 const uint32_t kept = last_len < 65536 ? (uint32_t)last_len : 65536u;
@@ -451,7 +457,7 @@ __device__ void copier_main(const DecompressArgs& a, DQueue* q, uint32_t in_s, u
 // Two register budgets: 16 CTAs per SM (64 registers, a few spilled bytes) when a launch has more than 12 streams per SM
 // to keep busy, 12 CTAs per SM (80 registers, no spills) when everything is resident anyway -- measured +6 % on config 2's
 // single wave, -12 % on 16 384 blocks of 64 KiB if used there.
-template <int kCtasPerSm, bool kPublish = false, bool kMirror = false>
+template <int kCtasPerSm, bool kPublish = false, bool kMirror = false, bool kWindow = false>
 __global__ void __launch_bounds__(64, kCtasPerSm)
 decompress_kernel(DecompressArgs a)
 {
@@ -466,19 +472,19 @@ decompress_kernel(DecompressArgs a)
     uint32_t in_s, out_s;       // laundered so that the compiler keeps them in registers instead of re-deriving them in the hot loops
     asm volatile("mov.u32 %0, %1;" : "=r"(in_s) : "r"(smem_u32(in_ring)));
     asm volatile("mov.u32 %0, %1;" : "=r"(out_s) : "r"(smem_u32(out_ring)));
-    if (threadIdx.x < 32) parser_main(a, &queue, in_s);
-    else copier_main<kPublish, kMirror>(a, &queue, in_s, out_s);
+    if (threadIdx.x < 32) parser_main<kWindow>(a, &queue, in_s);
+    else copier_main<kPublish, kMirror, kWindow>(a, &queue, in_s, out_s);
     release_counters(a.scratch, 2);
 }
 
 // 12 CTAs per SM while every stream gets a CTA of its own, else 16 per SM (one wave; CTAs claim further streams)
-template <bool kPublish, bool kMirror>
+template <bool kPublish, bool kMirror, bool kWindow = false>
 cudaError_t launch_narrow(const DecompressArgs& a, int sm_count, cudaStream_t stream)
 {
-    if (a.n_streams <= sm_count * 12) decompress_kernel<12, kPublish, kMirror><<<a.n_streams, 64, 0, stream>>>(a);
+    if (a.n_streams <= sm_count * 12) decompress_kernel<12, kPublish, kMirror, kWindow><<<a.n_streams, 64, 0, stream>>>(a);
     else {
         const int max_ctas = sm_count * 16;
-        decompress_kernel<16, kPublish, kMirror><<<a.n_streams < max_ctas ? a.n_streams : max_ctas, 64, 0, stream>>>(a);
+        decompress_kernel<16, kPublish, kMirror, kWindow><<<a.n_streams < max_ctas ? a.n_streams : max_ctas, 64, 0, stream>>>(a);
     }
     return cudaGetLastError();
 }
@@ -519,6 +525,14 @@ cudaError_t launch_decompress(const DecompressArgs& a, cudaStream_t stream)
     if (wide_env) wide = wide_env[0] == '1';
     if (wide && a.wide_arena) return launch_decompress_wide(b, sm_count, stream);
     return launch_narrow<false, false>(b, sm_count, stream);
+}
+
+cudaError_t launch_decompress_window(const DecompressArgs& a, cudaStream_t stream)
+{
+    int sm_count = 0;
+    cudaError_t e0 = device_sm_count(&sm_count); if (e0 != cudaSuccess) return e0;
+    if (a.n_streams <= 0) return cudaSuccess;
+    return launch_narrow<false, false, true>(a, sm_count, stream);
 }
 
 }  // namespace b200lz4

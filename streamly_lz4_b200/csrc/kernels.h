@@ -84,6 +84,63 @@ struct PerDeviceOnce {
     }
 };
 
+// ---- LZ4 frames (frame.cu) ----
+// Per-frame record of the decode walk.  fb: the frame's first block (global index, and index relative to its block-maximum
+// class), its first entry of the stream_first array, its staging and slot bytes -- written by the scan.
+struct FrameBases { long long blk, rel, str, stage, slot; };
+struct FrameRec {
+    long long content_size;     // header field, -1 if absent
+    long long stage, slot;      // staging bytes (stored blocks as literal-only LZ4 blocks), output slot bytes
+    int nblk, err, cls, flags;  // blocks (0 for a failed frame), first structural error, block maximum 64 KiB << 2 * cls, FLG
+    int window;                 // linked frame with a non-final block that may decode to less than 64 KiB
+    uint32_t ccsum;             // stored content checksum
+    FrameBases fb;
+};
+// totals of the scan: blocks[4], streams[4], window frames[4] per class, staging bytes, slot bytes
+constexpr int kFrameTotals = 14;
+
+struct FrameDecodeArgs {
+    const uint8_t* base; const int64_t* src_off; const int32_t* src_len; int n;       // the frames
+    FrameRec* rec; long long* totals;
+    // per block (fill): decoder input (frame payload, or the staged literal-only block at stage_delta from base), output slot,
+    // payload in the frame, length | stored << 31, block checksum range / expected value, frame; stream_first runs per class
+    long long stage_delta;
+    int64_t* dsrc_off; int32_t* dsrc_len; int64_t* slot_off; int64_t* raw_off; int32_t* meta;
+    int32_t* csum_len; uint32_t* csum_exp; uint32_t* csum_got; int32_t* bframe; int32_t* sf;
+    int32_t* out_len;                       // decoder results per block
+    int64_t* gout_off; int32_t* glen;       // gather: output offset (inside the content, then in the destination) and bytes
+    const int32_t* dst_cap;                 // per frame
+    int32_t* content; int32_t* cclen; uint32_t* ccsum_got; int32_t* result;
+};
+
+struct FrameEncodeArgs {
+    const uint8_t* src; const int64_t* src_off; const int32_t* src_len; int n;        // the arrays, one frame each
+    int flags, cls;
+    const int32_t* frame_first;             // blocks of frame i: frame_first[i] .. frame_first[i + 1] - 1
+    const int64_t* blk_off; const int32_t* blk_len; const int32_t* blk_frame;
+    const uint8_t* slots; const int64_t* slot_off; const int32_t* pay_len;           // compressor output (header 0)
+    int64_t* blk_at; int32_t* fsize; const int64_t* foff;                             // block offset in its frame, frame sizes, frame offsets
+    uint8_t* out;
+    int64_t* csum_off; int32_t* csum_len; const uint32_t* bsum; const uint32_t* csum_content;
+};
+
+cudaError_t launch_frame_walk(const FrameDecodeArgs& a, bool fill, cudaStream_t st);
+cudaError_t launch_frame_scan(const FrameDecodeArgs& a, cudaStream_t st);
+cudaError_t launch_frame_stage(const FrameDecodeArgs& a, int nb, cudaStream_t st);
+cudaError_t launch_frame_settle(const FrameDecodeArgs& a, cudaStream_t st);
+cudaError_t launch_frame_place(const FrameDecodeArgs& a, int nb, const int64_t* fbase, cudaStream_t st);
+cudaError_t launch_frame_verdict(const FrameDecodeArgs& a, cudaStream_t st);
+cudaError_t launch_frame_csize(const FrameEncodeArgs& a, cudaStream_t st);
+cudaError_t launch_frame_cpack(const FrameEncodeArgs& a, int nb, cudaStream_t st);
+cudaError_t launch_frame_cfinish(const FrameEncodeArgs& a, int nb, cudaStream_t st);
+// the narrow decoder in window mode (linked LZ4 frames): a stream's blocks are decoded back to back from dst_off of its
+// first block (the kernel writes the real dst_off of the others), and a block's dictionary is the stream's last
+// min(64 KiB, bytes decoded so far) bytes
+cudaError_t launch_decompress_window(const DecompressArgs& a, cudaStream_t stream);
+// the two passes of launch_compact on their own: exclusive scan of (header + len[i]) into out_off, and the gather
+cudaError_t launch_scan(const int32_t* len, int n, int header, int64_t* out_off, cudaStream_t stream);
+cudaError_t launch_gather(const CompactArgs& a, cudaStream_t stream);
+
 cudaError_t launch_compress(const CompressArgs& a, cudaStream_t stream);
 cudaError_t launch_set_flag(uint32_t* flag, uint32_t v, cudaStream_t stream);
 cudaError_t preload_compress_kernels();
