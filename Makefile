@@ -32,10 +32,11 @@ bounds: $(BOUNDS)
 $(BOUNDS): $(CU_SRCS) $(CU_HDRS)
 	$(NVCC) $(NVFLAGS) -DB200LZ4_BOUNDS_CHECK -shared -o $@ $(CU_SRCS) 2> /dev/null
 
-# development build with cycle accounting in the wide decoder (load it with B200LZ4_LIB=build/libb200lz4_stats.so)
+# development build with cycle accounting in the wide decoder and the compress finder
+# (load it with B200LZ4_LIB=build/libb200lz4_stats.so)
 stats: $(CU_SRCS) $(CU_HDRS)
 	mkdir -p build
-	$(NVCC) $(NVFLAGS) -DB200LZ4_WIDE_STATS -shared -o build/libb200lz4_stats$(SUFFIX).so $(CU_SRCS) 2> build/ptxas_stats.log || (cat build/ptxas_stats.log; false)
+	$(NVCC) $(NVFLAGS) -DB200LZ4_WIDE_STATS -DB200LZ4_FINDER_STATS -shared -o build/libb200lz4_stats$(SUFFIX).so $(CU_SRCS) 2> build/ptxas_stats.log || (cat build/ptxas_stats.log; false)
 
 clean:
 	rm -f $(LIB) $(BOUNDS) $(GEN) $(CSRC)/ptxas.log

@@ -165,17 +165,54 @@ struct BlockIn {
     const uint32_t* arrived; int seg; long long stall; bool timed_out;
 };
 
+// Finder cycle account for development builds (make stats -> build/libb200lz4_stats.so; tools/finder_stats.py): every
+// finder charges its clock64() intervals to the region it is in and counts how its sequences were found; the totals
+// are added to 64-bit counters in the scratch block's padding when the finder ends.  Compiled out of the product.
+// Regions 0-7 are cycles, 8-21 are counts; tools/finder_stats.py names them in this order.
+enum FinderStat {
+    kFsOther, kFsLoop, kFsMove, kFsScalar, kFsWindow, kFsCount, kFsFlush, kFsRegions_,
+    kFsLoopSeq = 8, kFsExitMiss, kFsExitLong, kFsExitEdge, kFsExitFull, kFsScalarProbe, kFsScalarHit, kFsWindows,
+    kFsMissThenHit0, kFsSeq, kFsRestartHit, kFsRestartMiss, kFsRestartLong, kFsLongInLoop, kFsSlots_
+};
+#ifdef B200LZ4_FINDER_STATS
+struct FinderStats {
+    unsigned long long v[kFsSlots_];
+    long long t;
+    int cur;
+    __device__ void start() { for (int i = 0; i < kFsSlots_; i++) v[i] = 0; t = clock64(); cur = kFsOther; }
+    __device__ int to(int r) { const long long now = clock64(); v[cur] += (unsigned long long)(now - t); t = now; const int p = cur; cur = r; return p; }
+};
+#define FSTAT_TO(r) out.fs.to(r)
+#define FSTAT_ENTER(r) const int fs_prev_ = out.fs.to(r)
+#define FSTAT_LEAVE() out.fs.to(fs_prev_)
+#define FSTAT_COUNT(i) (out.fs.v[i]++)
+#define FSTAT_ADD(i, n) (out.fs.v[i] += (n))
+#else
+#define FSTAT_TO(r)
+#define FSTAT_ENTER(r)
+#define FSTAT_LEAVE()
+#define FSTAT_COUNT(i)
+#define FSTAT_ADD(i, n)
+#endif
+
 // Producer side of the queue (finder warp).  The buffer being filled is always already acquired.
 struct Producer {
     Queue* q;
     uint32_t batch;     // batches pushed so far
     int fill;           // descriptors in the current buffer
     uint32_t slot_s;    // shared address of the next descriptor slot
+#ifdef B200LZ4_FINDER_STATS
+    FinderStats fs;
+#endif
 
     __device__ __forceinline__ void begin()
     {   // wait until the buffer we are about to fill has been drained, point at its first slot
         const uint32_t b = batch & 1, t = batch >> 1;
+#ifdef B200LZ4_FINDER_STATS
+        if (t) { const int p = fs.to(kFsFlush); mbar_wait(&q->empty[b], (t - 1) & 1); fs.to(p); }
+#else
         if (t) mbar_wait(&q->empty[b], (t - 1) & 1);
+#endif
         slot_s = smem_u32(&q->desc[b][0]);
         fill = 0;
     }
@@ -183,6 +220,9 @@ struct Producer {
     {
         sts128(slot_s, lit_pos, lit_len, mcode, off);     // all lanes store the same 16 bytes: no lane predicate on the hot path
         slot_s += 16;
+#ifdef B200LZ4_FINDER_STATS
+        fs.v[kFsSeq]++;
+#endif
         if (++fill == kQueueDepth) flush(block, 0);
     }
     __device__ __forceinline__ void flush(int block, int flags)
@@ -379,6 +419,7 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
         };
         auto move_window = [&](int ip) {       // (re)centre the window on ip's line
             const uintptr_t L = (base + (uintptr_t)ip) >> 7;
+            FSTAT_ENTER(kFsMove);
             if (kStreamed) wait_for((long long)((L + 3) << 7) - (long long)base);       // lines L-1 .. L+2 are touched below
             __syncwarp();
             cp_async_wait<0>();
@@ -408,6 +449,7 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
                 cur_line = L;
                 trigger = (int)(((L + 1) << 7) - base);
                 if ((uint32_t)ip + kPrefetchAhead > pf_next) l2_prefetch(ip);
+                FSTAT_LEAVE();
                 return;
             }
             if (L == cur_line + 1) {           // steady state: line L+1 has just landed
@@ -430,6 +472,7 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
             cur_line = L;
             trigger = (int)(((L + 1) << 7) - base);
             if ((uint32_t)ip + kPrefetchAhead > pf_next) l2_prefetch(ip);
+            FSTAT_LEAVE();
         };
 
         // Scalar probe at position p (every lane computes the same thing; the only 32-wide step is the
@@ -624,10 +667,19 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
         // arranged so that one sequence costs one dependent chain and one branch.  Inside the inner loop ip stays below
         // both the next ring window (no move_window) and mlimit - 31 (32-byte compares need no cap); the hash-ring and
         // byte loads of the next sequence are issued as soon as this one's length is known, ahead of the descriptor
-        // store; the queue is flushed when the loop leaves it full.  Anything else -- a miss, a match of 32+ bytes, the
-        // window edge, a full queue -- leaves the inner loop and is settled here.
+        // store; the queue is flushed when the loop leaves it full.
+        // A re-test miss at p is followed, as in the reference (cbits/lz4.c:1200, :959-1014), by probe 0 of a search
+        // run at p+1 -- step 1 whatever the acceleration -- whose catch-up (:1019) can walk back one byte at most, since
+        // anchor == p.  That probe is taken here, on the same chain: put(p-2), swap(p) (the miss), swap(p+1), then one
+        // ballot of the bytes p.. the loop already holds against cand-1..: lane 0 is the catch-up pair, lanes 1..31 the
+        // match.  A hit of 4..30 bytes becomes a one-literal sequence (none when the byte pair agrees) and the loop
+        // goes on at its end.  A match that fills its ballot (32 bytes from a re-test, 31 from the restart) gets one more
+        // ballot of the next 32 bytes from the rings when they hold both sides, and stays in the loop if it ends there.
+        // Anything else -- a miss on both, a longer match or one the rings cannot serve, the window edge, a full queue
+        // -- leaves the inner loop and is settled here.
         // Returns 0: the re-test at ip missed (ip unchanged), 1: ip reached mflimit, 2: ip is within 32 bytes of
-        // matchlimit (the caller finishes the run with retest_probe).
+        // matchlimit (the caller finishes the run with retest_probe), 3: the re-test at ip and probe 0 of the search run
+        // at ip+1 both missed (ip unchanged; the run goes on at probe 1).
         auto retest_run = [&](int& ip) -> int {
             const uint32_t gl_s = g32 + lane - S;                   // ring position of byte lane of candidate index cand: gl_s + cand
             const uint8_t* const src_s = src + lane - S;            // its global address: src_s + cand (cand >= S)
@@ -641,42 +693,100 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
                 const uint32_t ap = g32 + (uint32_t)ip;
                 uint32_t cur = S + (uint32_t)ip;
                 uint32_t h = hash_at(ap), h2 = hash_at(ap - 2), mine = ring8(ap + lane);
-                uint32_t m, ne;
+                // the probe that left the loop: at ip + lit, its catch-up (back), and when it is a match, its equal bytes so far
+                uint32_t m, ne, lit, back, known;
                 bool near, hit;
-                do {
-                    t_put(h2, cur - 2);                                                              // :1146
-                    m = t_swap(h, cur);                                                              // :1185
-                    near = (m >= S) && (m + kMaxDistance >= cur);                                    // :1187-1188
-                    // ring bytes unless the candidate is older than the ring (a far miss compares garbage: near decides)
-                    uint32_t theirs = ring8(gl_s + m);
-                    if (near && m < ring_lo) theirs = __ldg(src_s + m);
-                    ne = __ballot_sync(kFull, mine != theirs);
-                    const uint32_t L = (uint32_t)__ffs(ne) - 1u;
-                    hit = near && L - 4u < 28u;                                                      // 4 <= L < 32
-                    // The next sequence's loads.  On the iteration that leaves the loop (a miss, where L may be
-                    // ffs(0) - 1, or ip + L at the window edge) they may read ring bytes past ready_end, including the
-                    // line cp.async is still filling: on purpose -- the addresses are masked into this finder's rings,
-                    // the values are dropped, and the outer loop reloads h / h2 / mine after move_window.
-                    const uint32_t na = g32 + (uint32_t)ip + L;
-                    const uint32_t nh = hash_at(na), nh2 = hash_at(na - 2), nmine = ring8(na + lane);
-                    sts128(slot, (uint32_t)ip, 0u, L - 4, cur - m);      // after a miss: a stale slot past the fill mark
-                    if (hit) { slot += 16; ip += (int)L; cur += L; h = nh; h2 = nh2; mine = nmine; }
-                } while (hit && ip < lim && slot != slot_end);
+                for (;;) {
+                    do {
+                        t_put(h2, cur - 2);                                                          // :1146
+                        m = t_swap(h, cur);                                                          // :1185
+                        near = (m >= S) && (m + kMaxDistance >= cur);                                // :1187-1188
+                        // ring bytes unless the candidate is older than the ring (a far miss compares garbage: near decides)
+                        uint32_t theirs = ring8(gl_s + m);
+                        if (near && m < ring_lo) theirs = __ldg(src_s + m);
+                        ne = __ballot_sync(kFull, mine != theirs);
+                        const uint32_t L = (uint32_t)__ffs(ne) - 1u;
+                        hit = near && L - 4u < 28u;                                                  // 4 <= L < 32
+                        // The next sequence's loads.  On the iteration that leaves the loop (a miss, where L may be
+                        // ffs(0) - 1, or ip + L at the window edge) they may read ring bytes past ready_end, including the
+                        // line cp.async is still filling: on purpose -- the addresses are masked into this finder's rings,
+                        // the values are dropped, and the outer loop reloads h / h2 / mine after move_window.
+                        const uint32_t na = g32 + (uint32_t)ip + L;
+                        const uint32_t nh = hash_at(na), nh2 = hash_at(na - 2), nmine = ring8(na + lane);
+                        sts128(slot, (uint32_t)ip, 0u, L - 4, cur - m);      // after a miss: a stale slot past the fill mark
+                        if (hit) { slot += 16; ip += (int)L; cur += L; h = nh; h2 = nh2; mine = nmine; }
+                    } while (hit && ip < lim && slot != slot_end);
+                    if (hit) break;                                         // the window edge or a full queue
+                    lit = 0; back = 0; known = 32;
+                    if (!near || ne != 0) {
+                        // a re-test miss.  Probe 0 of the search run at ip+1 (hash and bytes are in the rings:
+                        // ip+1 < lim <= trigger); the miss left a slot free, since the loop goes on only while the queue has room
+                        if (ip + 1 >= lim) break;
+                        lit = 1; known = 31;
+                        m = t_swap(hash_at(g32 + (uint32_t)ip + 1), cur + 1);                      // :959-998
+                        near = (m >= S) && (m + kMaxDistance >= cur + 1);                            // :1001-1006
+                        // lane l: byte cand-1+l (lane 0 is the catch-up byte; none before the block start: m == S)
+                        uint32_t theirs = ring8(gl_s + m - 1);
+                        if (near && m - 1 + lane < ring_lo && m + lane > S) theirs = __ldg(src_s + m - 1);
+                        if (lane == 0 && m == S) theirs = 0x100u;
+                        const uint32_t ne1 = __ballot_sync(kFull, mine != theirs);
+                        ne = ne1 >> 1;
+                        back = (~ne1) & 1u;                                                          // :1019
+                        const uint32_t L = (uint32_t)__ffs(ne) - 1u;                                 // :1009, :1076-1095
+                        if (near && L - 4u < 27u) {                                                  // 4 <= L < 31
+                            sts128(slot, (uint32_t)ip, 1u - back, L + back - 4u, cur + 1 - m);
+                            FSTAT_COUNT(kFsRestartHit);
+                            slot += 16; ip += 1 + (int)L; cur += 1 + L;
+                            hit = true;
+                            if (!(ip < lim && slot != slot_end)) break;
+                            const uint32_t na = g32 + (uint32_t)ip;
+                            h = hash_at(na); h2 = hash_at(na - 2); mine = ring8(na + lane);
+                            continue;
+                        }
+                        if (!near || ne != 0) break;                                                 // a miss on both
+                    }
+                    // a match of 32 - lit equal bytes from ip + lit.  When its next 32 bytes and the candidate's lie in the
+                    // ring and below matchlimit, one more ballot of the same shape settles all matches shorter than 64 - lit.
+                    const uint32_t q = (uint32_t)ip + lit;
+                    if (m + known < ring_lo || (int)(q + known) + 32 > mlimit) break;
+                    const uint32_t ne2 = __ballot_sync(kFull, ring8(g32 + q + known + lane) != ring8(gl_s + m + known));
+                    if (ne2 == 0) { known += 32; break; }
+                    const uint32_t L = known + (uint32_t)__ffs(ne2) - 1u;
+                    sts128(slot, (uint32_t)ip, lit - back, L + back - 4u, cur + lit - m);
+                    FSTAT_COUNT(kFsLongInLoop);
+                    slot += 16; ip = (int)(q + L); cur = S + (uint32_t)ip;
+                    hit = true;
+                    if (!(ip < lim && slot != slot_end)) break;
+                    const uint32_t na = g32 + (uint32_t)ip;
+                    h = hash_at(na); h2 = hash_at(na - 2); mine = ring8(na + lane);
+                }
                 out.fill += (int)((slot - slot0) >> 4);
                 out.slot_s = slot;
                 anchor = ip;
+                FSTAT_ADD(kFsLoopSeq, (slot - slot0) >> 4);
                 if (!hit) {
-                    // a miss: out of reach, or fewer than 4 equal bytes (4..31 would have been a hit)      :1187-1189
-                    if (!near || ne != 0) return 0;
-                    // 32 equal bytes; cap >= 32 below lim
-                    const uint32_t cap = (uint32_t)(mlimit - ip);
-                    uint32_t L = 32u;
-                    if (cap > 32u) L += count_ahead(ip + 32, src + (m - S) + 32, cap - 32u);
-                    out.push((uint32_t)ip, 0u, L - 4, cur - m, in.block);
-                    ip += (int)L;
+                    // fewer than 4 equal bytes or out of reach (a hit would have stayed in the loop)      :1187-1189
+                    if (!near || ne != 0) {
+                        if (lit) { FSTAT_COUNT(kFsRestartMiss); return 3; }
+                        FSTAT_COUNT(kFsExitMiss);
+                        return 0;
+                    }
+                    // `known` equal bytes from ip + lit, known <= cap (both ballots stay below mlimit)
+                    FSTAT_COUNT(lit ? kFsRestartLong : kFsExitLong);
+                    FSTAT_TO(kFsCount);
+                    const int q = ip + (int)lit;
+                    const uint32_t cap = (uint32_t)(mlimit - q);
+                    uint32_t L = known;
+                    if (cap > known) L += count_ahead(q + (int)known, src + (m - S) + known, cap - known);
+                    FSTAT_TO(kFsLoop);
+                    out.push((uint32_t)ip, lit - back, L + back - 4, cur + lit - m, in.block);
+                    ip = q + (int)L;
                     anchor = ip;
                 } else if (out.fill == kQueueDepth) {
+                    FSTAT_COUNT(kFsExitFull);
                     out.flush(in.block, 0);
+                } else {
+                    FSTAT_COUNT(kFsExitEdge);
                 }
                 if (ip >= mfl) return 1;                                                             // :1143
             }
@@ -692,14 +802,16 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
         const bool ring_probes = in.accel <= 8; // the first probes of a run are (nearly) consecutive positions
         for (;;) {
             bool have = false;
+            long long jbase = 0;               // first probe of the search run still to take
             if (after_match) {
                 // ---- put(ip-2), re-test ip (cbits/lz4.c:1146, :1159-1196); ip == anchor here.
                 // Loops for as long as a match immediately follows a match.
                 int run = 2;
                 if constexpr (!kWide && !kCompact) {
-                    if (in.dict_len == 0) run = retest_run(ip);
+                    if (in.dict_len == 0) { FSTAT_TO(kFsLoop); run = retest_run(ip); FSTAT_TO(kFsOther); }
                 }
                 if (run == 1) goto tail;
+                if (run == 3) jbase = 1;       // retest_run took probe 0 at ip+1, and it missed
                 if (run == 2) while (retest_probe(ip)) {
                     out.push((uint32_t)ip, 0u, mlen - 4, dist, in.block);
                     ip += (int)mlen;
@@ -711,10 +823,13 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
             if ((uint32_t)ip + kPrefetchAhead > pf_next) l2_prefetch(ip);
             // ---- a search run starts at ip (cbits/lz4.c:956-1014)
             if (ring_probes && ip >= trigger) move_window(ip);      // dense probing: keep the rings under the first window
-            long long jbase = 0;
-            if (first_scalar) {                // probe 0 of the run on the scalar path
+            if (first_scalar && jbase == 0) {  // probe 0 of the run on the scalar path
                 if (ip + 1 > mfl) break;                                                             // :969
+                FSTAT_TO(kFsScalar);
                 have = scalar_probe(ip, false);
+                FSTAT_TO(kFsOther);
+                FSTAT_COUNT(kFsScalarProbe);
+                if (have) { FSTAT_COUNT(kFsScalarHit); if (after_match) FSTAT_COUNT(kFsMissThenHit0); }
                 jbase = 1;
             }
             if (!have) {
@@ -722,7 +837,9 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
                 int mpos = 0; uint32_t midx = 0;
                 uint32_t width = narrow ? 4u : 32u;
                 bool found = false; int hit_index = 0;
+                FSTAT_TO(kFsWindow);
                 for (;;) {
+                    FSTAT_COUNT(kFsWindows);
                     long long off; int step;
                     if (jbase == 0) { off = off0; step = (int)step0; }
                     else if (jbase == 1) { off = off1; step = (int)step1; }
@@ -792,7 +909,9 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
                     jbase += width;
                     width = 32;
                 }
+                FSTAT_TO(kFsCount);
                 if (!found) break;
+                if (after_match && hit_index == 0) FSTAT_COUNT(kFsMissThenHit0);
                 narrow = (in.accel > 16) && (hit_index < 3);
                 first_scalar = (hit_index == 0);
 
@@ -819,6 +938,7 @@ __device__ void find_block(BlockIn& in, uint32_t* table, const uint32_t data_s, 
                 mip = mpos - (int)back;
                 mlen = L + back; dist = (S + (uint32_t)mpos) - midx;
                 }
+                FSTAT_TO(kFsOther);
             }
             out.push((uint32_t)anchor, (uint32_t)(mip - anchor), mlen - 4, dist, in.block);
             ip = mip + (int)mlen;
@@ -846,6 +966,9 @@ __device__ void finder_main(const CompressArgs& a, uint32_t* table, uint32_t* ri
     uint32_t* counter = &a.scratch->work_counter[0];
     const int accel = a.accel < 1 ? 1 : (a.accel > kAccelMax ? kAccelMax : a.accel);   // :1577-1578
     Producer out{q, 0, 0, 0};
+#ifdef B200LZ4_FINDER_STATS
+    out.fs.start();
+#endif
     out.begin();
     const uint32_t data_s = smem_u32(ring), hash_s = smem_u32(hring);
     long long off0, off1; int step0, step1;
@@ -962,6 +1085,11 @@ __device__ void finder_main(const CompressArgs& a, uint32_t* table, uint32_t* ri
         }
         __syncwarp();
     }
+#ifdef B200LZ4_FINDER_STATS
+    out.fs.to(kFsOther);
+    if (lane == 0)
+        for (int i = 0; i < kFsSlots_; i++) atomicAdd(reinterpret_cast<unsigned long long*>(a.scratch->pad_) + i, out.fs.v[i]);
+#endif
     out.flush(-1, kTerminate);
 }
 
