@@ -12,7 +12,7 @@ library of LZ4 is not part of the reference tree, so what follows restates the p
         HC : (XXH32(FLG .. last descriptor byte, seed 0) >> 8) & 0xFF
     blocks: [size LE32: bit 31 set = stored uncompressed][data][XXH32(data) LE32 iff block checksum]
     end mark 0x00000000 | [XXH32(whole content) LE32 iff content checksum]
-    linked blocks (independence flag clear) may reference the previous 64 KiB of DECODED data.
+    linked blocks (independence flag clear) may reference the previous 64 KiB of DECODED data, across block boundaries.
 
 Known answers pinned in tests/test_oracle.py: descriptors 60 40 -> HC 82, 64 40 -> A7, 64 70 -> B9 (the headers the
 stock `lz4` tool writes for -B4 / -B4 --content-checksum / -B7 --content-checksum streams).
@@ -26,17 +26,49 @@ from typing import List, Optional, Sequence, Tuple
 MAGIC = 0x184D2204
 BD_SIZES = {4: 64 << 10, 5: 256 << 10, 6: 1 << 20, 7: 4 << 20}
 
+E_NOMEM, E_BLOCK, E_FRAME, E_CHECKSUM = -3, -4, -5, -6      # B200LZ4_E_* (include/b200lz4.h)
+WINDOW = 65536
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _lib = None
 
 
-def xxh32(data: bytes, seed: int = 0) -> int:
+class _DStream(ctypes.Structure):         # struct ora_dstream (lz4_oracle.c)
+    _fields_ = [("prev_out", ctypes.c_void_p), ("prev_len", ctypes.c_size_t)]
+
+
+def _load():
     global _lib
     if _lib is None:
-        _lib = ctypes.CDLL(os.path.join(_HERE, "liboracle.so"))
-        _lib.ora_xxh32.restype = ctypes.c_uint32
-        _lib.ora_xxh32.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint32]
-    return int(_lib.ora_xxh32(bytes(data), len(data), seed))
+        lib = ctypes.CDLL(os.path.join(_HERE, "liboracle.so"))
+        lib.ora_xxh32.restype = ctypes.c_uint32
+        lib.ora_xxh32.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint32]
+        lib.ora_dstream_create.restype = ctypes.POINTER(_DStream)
+        lib.ora_dstream_free.argtypes = [ctypes.POINTER(_DStream)]
+        lib.ora_decompress_continue.argtypes = [ctypes.POINTER(_DStream), ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+                                                ctypes.c_int]
+        lib.ora_decompress_continue.restype = ctypes.c_int
+        _lib = lib
+    return _lib
+
+
+def xxh32(data: bytes, seed: int = 0) -> int:
+    return int(_load().ora_xxh32(bytes(data), len(data), seed))
+
+
+def decode_block(payload: bytes, cap: int, dictionary: bytes = b"") -> Optional[bytes]:
+    """LZ4_decompress_safe_usingDict(payload, cap, dictionary) through the restatement (a decode record whose previous
+    output is `dictionary`, as dict_golden.Port sets it up): the block's output, or None when the block is rejected."""
+    lib = _load()
+    dbuf = ctypes.create_string_buffer(bytes(dictionary), len(dictionary) + 1)
+    src = ctypes.create_string_buffer(bytes(payload), len(payload) + 1)
+    dst = ctypes.create_string_buffer(cap + 1)
+    s = lib.ora_dstream_create()
+    s.contents.prev_out = ctypes.addressof(dbuf) if dictionary else None
+    s.contents.prev_len = len(dictionary)
+    r = lib.ora_decompress_continue(s, src, dst, len(payload), cap)
+    lib.ora_dstream_free(s)
+    return None if r < 0 else dst.raw[:r]
 
 
 def header(bd_code: int, independent: bool = False, block_checksum: bool = False, content_size: Optional[int] = None,
@@ -116,22 +148,99 @@ def parse(blob: bytes) -> Tuple[dict, List[Tuple[bool, bytes]], Optional[int]]:
     return d, blocks, cc
 
 
-def decode(oracle, blob: bytes) -> bytes:
-    """Stock frame decode: linked blocks see the previous 64 KiB of decoded data (here: the oracle's linked decoder, whose
-    dictionary is the previous block -- identical whenever every block but the last is at least 64 KiB, which is what
-    both writers in the tests produce)."""
-    d, blocks, cc = parse(blob)
-    name = {4: "BlockMax64KB", 5: "BlockMax256KB", 6: "BlockMax1MB", 7: "BlockMax4MB"}[d["bd_code"]]
-    framed = []
-    for stored, data in blocks:
-        if stored:                                   # a stored block as an LZ4 block made of literals only (same bytes out, keeps the chain)
-            data = literal_block(data)
-        framed.append(len(data).to_bytes(4, "little") + data)
-    out = b"".join(oracle.decompress_chunks_raw(framed, block_size=name, linked=not d["independent"]))
+def _walk(blob: bytes, dict_id_ok: bool):
+    """The frame's structure as frame_walk_kernel reads it: (descriptor, [(stored, block data, block checksum or None)],
+    content checksum or None), or the error code of the first structural fault (FRAME; CHECKSUM for the header checksum).
+    dict_id_ok: a dictionary id is read rather than refused."""
+    L = len(blob)
+    flg, bd = (blob[4], blob[5]) if L >= 6 else (0, 0)
+    if L < 7 or int.from_bytes(blob[0:4], "little") != MAGIC or (flg >> 6) != 1 or flg & 0x02 or bd & 0x8F \
+            or (flg & 0x01 and not dict_id_ok) or (bd >> 4) & 7 < 4:
+        return E_FRAME
+    at = 6 + (8 if flg & 0x08 else 0) + (4 if flg & 0x01 else 0)
+    if L <= at:
+        return E_FRAME
+    if blob[at] != (xxh32(blob[4:at]) >> 8) & 0xFF:
+        return E_CHECKSUM
+    d = {"independent": bool(flg & 0x20), "block_checksum": bool(flg & 0x10), "content_checksum": bool(flg & 0x04),
+         "content_size": int.from_bytes(blob[6:14], "little") if flg & 0x08 else None, "bd_code": (bd >> 4) & 7,
+         "block_max": BD_SIZES[(bd >> 4) & 7]}
+    at += 1
+    blocks = []
+    while True:
+        if L - at < 4:
+            return E_FRAME                                   # truncated before a block size or the end mark
+        size = int.from_bytes(blob[at:at + 4], "little"); at += 4
+        n = size & 0x7FFFFFFF
+        if n == 0:
+            break                                            # the end mark (read without its stored bit, as upstream does)
+        bc = 4 if d["block_checksum"] else 0
+        if n > d["block_max"] or L - at < n + bc:
+            return E_FRAME
+        blocks.append((bool(size >> 31), blob[at:at + n], int.from_bytes(blob[at + n:at + n + 4], "little") if bc else None))
+        at += n + bc
+    cc = None
+    if d["content_checksum"]:
+        if L - at < 4:
+            return E_FRAME
+        cc = int.from_bytes(blob[at:at + 4], "little"); at += 4
+    if at != L:
+        return E_FRAME                                       # one frame per range: nothing may follow it
+    return d, blocks, cc
+
+
+def decode_result(blob: bytes, cap: Optional[int], dictionary: bytes, dict_id_ok: bool, codec=None):
+    """(code, content): code is the content length or the first fault in stream order -- the structure, then per block its
+    checksum before its decode, then the content size, the capacity (cap; None: any) and the content checksum.
+    codec: decodes the blocks that see no earlier bytes (oracle.Oracle, or None: the restatement); a block with a window
+    goes through the restatement's dictionary decode (decode_block)."""
+    w = _walk(blob, dict_id_ok)
+    if isinstance(w, int):
+        return w, None
+    d, blocks, cc = w
+    out = bytearray()
+    for stored, data, csum in blocks:
+        if csum is not None and csum != xxh32(data):
+            return E_CHECKSUM, None
+        if stored:
+            out += data
+            continue
+        # linked blocks see the last 64 KiB of the dictionary followed by everything decoded so far (LZ4F_decompress)
+        window = dictionary[-WINDOW:] if d["independent"] else (dictionary[-WINDOW:] + bytes(out[-WINDOW:]))[-WINDOW:]
+        if window or codec is None:
+            got = decode_block(data, d["block_max"], window)
+        else:
+            try:
+                name = {4: "BlockMax64KB", 5: "BlockMax256KB", 6: "BlockMax1MB", 7: "BlockMax4MB"}[d["bd_code"]]
+                (got,) = codec.decompress_chunks_raw([len(data).to_bytes(4, "little") + data], block_size=name, linked=False)
+            except RuntimeError:
+                got = None
+        if got is None:
+            return E_BLOCK, None
+        out += got
     if d["content_size"] is not None and d["content_size"] != len(out):
-        raise ValueError("content size mismatch")
+        return E_FRAME, None
+    if cap is not None and len(out) > cap:
+        return E_NOMEM, None
     if cc is not None and cc != xxh32(out):
-        raise ValueError("content checksum mismatch")
+        return E_CHECKSUM, bytes(out)
+    return len(out), bytes(out)
+
+
+def verdict(blob: bytes, cap: int) -> int:
+    """What b200lz4_frame_decompress_batch reports for one frame given dst_cap = cap: the content length, or the code of
+    the frame's first fault (frame_walk_kernel's structural checks, then frame_settle_kernel's order)."""
+    return decode_result(blob, cap, b"", False)[0]
+
+
+def decode(oracle, blob: bytes, dictionary: bytes = b"") -> bytes:
+    """Stock frame decode (LZ4F_decompress, LZ4F_decompress_usingDict with a dictionary) over the whole range: a linked
+    block sees the last 64 KiB of the dictionary and the content decoded before it, across any number of blocks; every
+    block of an independent frame sees the dictionary alone.  `oracle` decodes the blocks that see no earlier bytes (see
+    decode_result).  Raises ValueError like a stock reader would."""
+    code, out = decode_result(blob, None, bytes(dictionary), True, oracle)
+    if code < 0:
+        raise ValueError(f"frame rejected ({code})")
     return out
 
 

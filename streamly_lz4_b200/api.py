@@ -858,18 +858,21 @@ def read_frame(chunks: Iterable, *, ctx: Optional[Context] = None, verify: bool 
                dictionary: Optional[Dictionary] = None, **kw) -> Iterator[bytes]:
     """Decode one complete LZ4 frame from an arbitrarily fragmented byte stream: header (checksum verified), blocks
     (stored blocks pass through as literal-only LZ4 blocks, so a linked chain stays intact), block checksums, end
-    mark, content size and content checksum.  Yields one array per block.
-    dictionary: the blocks are decoded as LZ4F_decompress_usingDict does (every block of an independent frame, the first
-    of a linked one).  A frame with a dictionary id is refused without one; the id itself is not checked (it names the
-    dictionary the writer used, and only the caller knows which one that is)."""
+    mark, content size and content checksum.  A linked block may reference the last 64 KiB of the content decoded before
+    it, across any number of earlier blocks (LZ4F_decompress), which frames flushed after small updates need.
+    Without a dictionary (and with verify) the frame is decoded in one b200lz4_frame_decompress_batch call and the
+    content is yielded as one array; otherwise one array per block.
+    dictionary: the blocks are decoded as LZ4F_decompress_usingDict does (every block of an independent frame starts
+    from it; a linked block sees the last 64 KiB of the dictionary followed by the content before it).  A frame with a
+    dictionary id is refused without one; the id itself is not checked (it names the dictionary the writer used, and only
+    the caller knows which one that is)."""
     ctx = ctx or (dictionary.ctx if dictionary is not None else default_context())
     data = b"".join(bytes(c) for c in chunks)
     cfg, _, info = parse_frame_header(data[:19], allow_dict_id=dictionary is not None)
-    if dictionary is not None:
-        kw["dictionary"] = dictionary
     at = info.header_len
     framed: List[bytes] = []
     check_off, check_len, check_want = [], [], []
+    bound = 0
     while True:
         if at + 4 > len(data):
             raise LZ4Error("resizeChunksD: No end mark found")
@@ -885,6 +888,7 @@ def read_frame(chunks: Iterable, *, ctx: Optional[Context] = None, verify: bool 
             check_off.append(at); check_len.append(n); check_want.append(int.from_bytes(data[at + n:at + n + 4], "little"))
             at += 4
         at += n
+        bound += n if stored else min(cfg.max_block_size, 255 * n)       # an LZ4 block makes at most 255 bytes per byte
         if stored:                                               # token, length bytes, literals: decodes to `body` itself
             m = len(body)
             if m < 15:
@@ -900,8 +904,19 @@ def read_frame(chunks: Iterable, *, ctx: Optional[Context] = None, verify: bool 
         bad = np.nonzero(got != np.array(check_want, dtype=np.uint32))[0]
         if len(bad):
             raise LZ4Error(f"frame: block checksum mismatch in block {int(bad[0])}")
+    if info.content_checksum and at + 4 > len(data):
+        raise LZ4Error("frame: input ended inside the content checksum")
+    if dictionary is None and verify:
+        yield _read_frame_device(ctx, data[:at + (4 if info.content_checksum else 0)], bound, info)
+        return
+    if dictionary is not None:
+        kw["dictionary"] = dictionary
     total, outs = 0, []
-    for a in decompress_chunks_raw(cfg, framed, ctx=ctx, **kw):
+    if cfg.independent:
+        decoded = decompress_chunks_raw(cfg, framed, ctx=ctx, **kw)
+    else:
+        decoded = _linked_blocks(ctx, cfg, framed, dictionary, kw)
+    for a in decoded:
         total += len(a)
         if info.content_checksum and verify:
             outs.append(a)
@@ -915,3 +930,36 @@ def read_frame(chunks: Iterable, *, ctx: Optional[Context] = None, verify: bool 
         buf[:len(whole)] = np.frombuffer(whole, dtype=np.uint8)
         if int(ctx.xxh32(buf[:max(len(whole), 1)], [0], [len(whole)])[0]) != want:
             raise LZ4Error("frame: content checksum mismatch")
+
+
+def _read_frame_device(ctx: Context, blob: bytes, bound: int, info: FrameInfo) -> bytes:
+    """read_frame's decode of a whole frame (already walked and its block checksums verified) in one device call"""
+    src = np.frombuffer(blob + b"\0", dtype=np.uint8).copy()
+    cap = max(1, min(bound, 0x7FFFFFFF) if info.content_size is None else min(bound, info.content_size, 0x7FFFFFFF))
+    dst = np.empty(cap, dtype=np.uint8)
+    rc, out = ctx.frame_decompress_batch(src, np.zeros(1, np.int64), np.array([len(blob)], np.int32), dst,
+                                         np.zeros(1, np.int64), np.array([cap], np.int32))
+    code = int(out[0])
+    if code == E_CHECKSUM:
+        raise LZ4Error("frame: content checksum mismatch")
+    if code == E_FRAME and info.content_size is not None:
+        raise LZ4Error(f"frame: the content size does not match the header's {info.content_size}")
+    if rc != 0 or code < 0:
+        raise LZ4Error(f"decompressChunk: frame decode failed ({code}): {ctx.last_error()}")
+    return dst[:code].tobytes()
+
+
+def _linked_blocks(ctx: Context, cfg: BlockConfig, framed: List[bytes], dictionary: Optional[Dictionary], kw) -> Iterator[bytes]:
+    """The blocks of a linked frame one at a time, each against the last 64 KiB of the dictionary and the content so far"""
+    one = BlockConfig(block_size=cfg.block_size, independent=True)
+    window = dictionary.data[-65536:] if dictionary is not None else b""
+    for f in framed:
+        d = Dictionary(ctx, window) if window else None
+        kw["dictionary"] = d
+        try:
+            (a,) = list(decompress_chunks_raw(one, [f], ctx=ctx, **kw))
+        finally:
+            if d is not None:
+                d.free()
+        window = (window + a)[-65536:]
+        yield a

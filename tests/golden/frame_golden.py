@@ -1,6 +1,8 @@
 """Golden LZ4 frames written by upstream LZ4F (the system liblz4, 1.9.x), with upstream's accept/reject verdicts.
 
-  python tests/golden/frame_golden.py [LIB]  -> tests/golden/frames/*.lz4 + tests/golden/frames/frames.json
+  python tests/golden/frame_golden.py [LIB]         -> tests/golden/frames/*.lz4 + tests/golden/frames/frames.json
+  python tests/golden/frame_golden.py window [LIB]  -> tests/golden/frames/window_checks.json: upstream's verdict and
+                                                       content digest for every hand-built case of window_cases.py
 
 Every frame's content is datagen(kind, seed)[:length]; frames.json holds, per file, the content's SHA-256, upstream's
 verdict (LZ4F_decompress over the whole range: accept = no error, frame complete, every byte consumed) and the code
@@ -282,7 +284,27 @@ def main(path: str) -> None:
     print(f"{len(records)} frames, {total} bytes")
 
 
+def window(path: str) -> None:
+    """Upstream's verdict on the hand-built window cases (the frames are rebuilt from window_cases.py, not stored)"""
+    sys.path.insert(0, HERE)
+    import window_cases
+    up = LZ4F(path)
+    checks = {}
+    for c in window_cases.cases():
+        acc, got = up.decompress(c.blob, len(c.plain) if c.plain is not None else c.block_max)
+        if c.plain is not None:
+            assert acc and got == c.plain, c.id
+        checks[c.id] = {"upstream": "accept" if acc else "reject", "sha256": hashlib.sha256(got).hexdigest() if acc else None}
+    v = up.lib.LZ4_versionNumber()
+    with open(os.path.join(OUT, "window_checks.json"), "w") as fh:
+        json.dump({"generator": "tests/golden/frame_golden.py window", "library": f"{os.path.basename(path)} "
+                   f"({v // 10000}.{v // 100 % 100}.{v % 100})", "cases": checks}, fh, indent=0)
+    print(f"{len(checks)} window cases, {sum(r['upstream'] == 'reject' for r in checks.values())} rejected")
+
+
 if __name__ == "__main__":
-    lib = sys.argv[1] if len(sys.argv) > 1 else ctypes.util.find_library("lz4")
-    assert lib, "no liblz4 found: name one, frame_golden.py /path/to/liblz4.so"
-    main(lib)
+    args = sys.argv[1:]
+    sub = args.pop(0) if args and args[0] == "window" else None
+    lib = args[0] if args else ctypes.util.find_library("lz4")
+    assert lib, "no liblz4 found: name one, frame_golden.py [window] /path/to/liblz4.so"
+    (window if sub else main)(lib)

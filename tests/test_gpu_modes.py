@@ -16,10 +16,11 @@ SUBSET = ["tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py", "tests/test_gpu_
 
 
 DECODE_SUBSET = ["tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py", "tests/test_gpu_configs.py", "tests/test_gpu_device_abi.py",
-                 "tests/test_gpu_decode_geometry.py", "-k",
+                 "tests/test_gpu_decode_geometry.py", "tests/test_gpu_frame_window.py", "-k",
                  "handbuilt or corrupted or random_round_trips or echoing or split_over or generators or edge_sizes or "
                  "empty_and_tiny or block_max or large_blocks or linked_state or malformed or fragmented or "
-                 "config3 or config4 or (device_abi and (decompress_dev or scratch_shared)) or decode_geometry"]       # config 3: 1 678 one-block streams = several streams per CTA in the wide kernel
+                 "config3 or config4 or (device_abi and (decompress_dev or scratch_shared)) or decode_geometry or "
+                 "(frame_window and not compress)"]       # config 3: 1 678 one-block streams = several streams per CTA in the wide kernel
 
 
 @pytest.mark.parametrize("env", [{"B200LZ4_DWIDE": "0"},        # every decode through the narrow kernel (parser + copier warp per stream)
@@ -49,17 +50,17 @@ def test_parity_with_forced_kernel(ctx, env):
 def test_decoder_bounds_checked_build_on_malformed_input(ctx):
     """compute-sanitizer is not available on the GPU pool, so memory safety of the decoders on hostile input is shown with
     a debug build (make bounds: -DB200LZ4_BOUNDS_CHECK) that checks every destination range against the block capacity
-    and traps on a violation: the hand-built, corrupted and malformed-block tests and the copy-path geometry cases run
-    through it, narrow and wide."""
+    and traps on a violation: the hand-built, corrupted and malformed-block tests, the copy-path geometry cases and the
+    frame window cases run through it, narrow and wide."""
     lib = os.path.join(ROOT, "streamly_lz4_b200", "libb200lz4_bounds.so")
     if not os.path.exists(lib):
         pytest.skip("libb200lz4_bounds.so not built (make bounds)")
     for wide in ("0", "1"):
         e = dict(os.environ, B200LZ4_LIB=lib, B200LZ4_DWIDE=wide)
         out = subprocess.run([sys.executable, "-m", "pytest", "-x", "-q", "-m", "gpu", "tests/test_gpu_fuzz.py", "tests/test_gpu_parity.py",
-                              "tests/test_gpu_device_abi.py", "tests/test_gpu_decode_geometry.py",
+                              "tests/test_gpu_device_abi.py", "tests/test_gpu_decode_geometry.py", "tests/test_gpu_frame_window.py",
                               "-k", "handbuilt or corrupted or malformed or edge_sizes or echoing or (device_abi and decompress_dev) or "
-                              "decode_geometry"],
+                              "decode_geometry or (frame_window and not compress)"],
                              cwd=ROOT, env=e,
                              stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
         assert out.returncode == 0, out.stdout[-3000:]
